@@ -8,6 +8,7 @@ every rank verifies its own 2^20 triples (independent units, no data-path collec
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            # engine arm
   python bench.py --impl reference [--gpus N] [--steps K] ...    # the reference's CPU algorithm (oracle port)
+  python bench.py --dump-outputs DIR ...                         # also write the last timed step's verdicts to DIR
 """
 import argparse
 import json
@@ -15,6 +16,8 @@ import os
 import sys
 import time
 
+# the benchmark may run from a read-only tree: no bytecode caches are written next to the sources
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -42,7 +45,14 @@ def parse():
     ap.add_argument('--keygen-log2n', type=int, default=20, help='configs[2]: log2 of seeds, whole job (split over the GPUs)')
     ap.add_argument('--adaptor-log2n', type=int, default=18, help='configs[4]: log2 of instances, whole job')
     ap.add_argument('--cpu-bklm-log2n', type=int, default=8, help='CPU baseline: largest BKLM aggregate actually run')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='engine arm: write the verdicts of the last timed step as DIR/verdict.npy (float32; '
+                         'verdict_rank<r>.npy per rank when several run), so that two builds can be compared output '
+                         'for output on the same seeded inputs')
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != 'engine':
+        ap.error('--dump-outputs writes what the engine arm computes')
+    return a
 
 
 def workload_name(a):
@@ -202,6 +212,20 @@ def build_inputs(a, rank, torch, np):
     ch_off = np.arange(n + 1, dtype=np.int64) * ch.shape[1]
     return seeds.reshape(-1), seed_off, ch, ch_off
 
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays, world, np):
+    """Writes every array of `arrays` (name -> array) as <dirname>/<name>.npy in float32.  All ranks together write at
+    most DUMP_BYTES: a larger output is replaced by a fixed sample, its elements at indices drawn by a generator seeded
+    with 0 (the same indices on every run with the same arguments)."""
+    os.makedirs(dirname, exist_ok=True)
+    cap = DUMP_BYTES // 4 // (world * len(arrays))
+    for name, arr in arrays.items():
+        if arr.size > cap:
+            arr = arr.reshape(-1)[np.sort(np.random.default_rng(0).choice(arr.size, cap, replace=False))]
+        np.save(os.path.join(dirname, name + '.npy'), arr.astype(np.float32))
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -722,6 +746,8 @@ def engine_arm(a):
     eng.profile(False)
     total_ms = float(ms.item())
     value = world * n * a.steps / (total_ms * 1e-3)
+    if a.dump_outputs:          # before the packed leg below reuses `verdict`
+        dump_outputs(a.dump_outputs, {'verdict' if world == 1 else f'verdict_rank{rank}': verdict.cpu().numpy()}, world, np)
 
     # ---- end to end: the same call with pinned HOST buffers (H2D of every input + D2H of the verdicts inside)
     h_sig = torch.empty(sig.shape, dtype=torch.int16, pin_memory=True)
