@@ -189,6 +189,34 @@ int lcb_bklm_aggverify_partial(lcb_ctx* ctx, const lcb_scheme* sch, const uint16
 int lcb_bklm_aggverify_finish(lcb_ctx* ctx, const int32_t* partial_sum, const int16_t* ag_sig, int64_t total,
                               int ag_cap, int avf_bd, int avf_wt, uint8_t* verdict);
 
+/* ---- Batches of independent aggregates: many small aggregates (the reference caps one at ag_cap = 2 signatures) in one
+ * call instead of a handful of launches, copies and synchronisations per aggregate.  Whole aggregates only: a group is
+ * never split across calls (the shard entry points above do that).  Group g covers sorted items
+ * [agg_off[g], agg_off[g+1]); offset arrays have n_agg + 1 entries.  Host-resident offset arrays must start at 0 and
+ * never decrease (LCB_ERR_INVALID otherwise); device-resident ones are trusted.  The call reads agg_off[n_agg] and
+ * agmsg_off[n_agg] on the host (a device array costs one small copy and a synchronisation).  At most 2^30 signatures
+ * and 2^30 aggregates per call; n_agg == 0 returns LCB_OK.
+ * The shipped geometry (d = 256, q < 2^16) with ag_wt = ag_bd = 1 runs segmented kernels over the whole batch; generic
+ * contexts and non-monomial coefficients loop over the groups through the single-aggregate kernels: correct, not fast. */
+
+/* aggregate (bklm_one_time_agg_sigs.py:92-96) for n_agg independent aggregates in one call.
+ * Aggregate g covers the SORTED signatures [agg_off[g], agg_off[g+1]) of sig_sorted int16[agg_off[n_agg]][l][d];
+ * its coefficients are H2P(ag_salt + str(j) || agmsg_g) for j = 0 .. count_g - 1 (the index restarts in every
+ * aggregate), agmsg_g = agmsg[agmsg_off[g] .. agmsg_off[g+1]).  ag_sig int16[n_agg][l][d].
+ * Every aggregate must hold >= 1 signature (LCB_ERR_INVALID otherwise); at most 2^30 signatures per call. */
+int lcb_bklm_aggregate_batch(lcb_ctx* ctx, const lcb_scheme* sch, const int64_t* agg_off, int64_t n_agg,
+                             const int16_t* sig_sorted, const uint8_t* agmsg, const int64_t* agmsg_off,
+                             int16_t* ag_sig);
+
+/* aggregate_verify (:99-116) for n_agg aggregates.  vk_ntt_sorted uint16[total][2][d], chmsg_sorted ragged over the
+ * same total items, ag_sig int16[n_agg][l][d], verdict uint8[n_agg].  verdict[g] is exactly what
+ * lcb_bklm_aggverify_partial(first = 0, count_g) + lcb_bklm_aggverify_finish(total = count_g) give for that group;
+ * an empty group, or one above ag_cap, gets verdict 0 (not an error). */
+int lcb_bklm_aggregate_verify_batch(lcb_ctx* ctx, const lcb_scheme* sch, const int64_t* agg_off, int64_t n_agg,
+                                    const uint16_t* vk_ntt_sorted, const uint8_t* chmsg_sorted,
+                                    const int64_t* chmsg_off, const uint8_t* agmsg, const int64_t* agmsg_off,
+                                    const int16_t* ag_sig, int ag_cap, int avf_bd, int avf_wt, uint8_t* verdict);
+
 /* adaptor make_one_wit / witgen (adaptor_sigs.py:80-101,140-151):
  *   wit_coef int16[n][l][d], st_ntt uint16[n][d], st_coef int16[n][d]; any may be NULL. */
 int lcb_adaptor_witgen_batch(lcb_ctx* ctx, const lcb_scheme* sch, const uint8_t* seeds, const int64_t* seed_off,
@@ -238,7 +266,8 @@ int lcb_mctx_bklm_aggregate_verify(lcb_mctx* m, const lcb_scheme* sch, const uin
 int64_t lcb_launch_count(const lcb_ctx* ctx);
 /* Optional per-kernel timing with CUDA events on the ctx stream (what bench.py's roofline reads).
  * kernel names: sampler shake256 ntt_fwd ntt_inv poly_mul matvec sign verify vec_addsub agg_coefs
- * agg_partial agg_finish aggv_partial aggv_finish.  lcb_profile_read synchronises the stream. */
+ * agg_partial agg_finish aggv_partial aggv_finish pack unpack, and for the batch calls group_ids agg_coefs_seg
+ * agg_partial_seg aggv_partial_seg aggv_residues aggv_limits.  lcb_profile_read synchronises the stream. */
 int lcb_profile_enable(lcb_ctx* ctx, int on);
 int lcb_profile_reset(lcb_ctx* ctx);
 int lcb_profile_read(lcb_ctx* ctx, const char* kernel, double* total_ms, int64_t* launches);

@@ -74,6 +74,9 @@ PROTOTYPES = {
     'lcb_bklm_aggverify_partial': (c_int, [c_void_p, POINTER(LcbScheme), _P, _P, _P, _P, _P, c_int64, c_int64,
                                            c_int64, _P]),
     'lcb_bklm_aggverify_finish': (c_int, [c_void_p, _P, _P, c_int64, c_int, c_int, c_int, _P]),
+    'lcb_bklm_aggregate_batch': (c_int, [c_void_p, POINTER(LcbScheme), _P, c_int64, _P, _P, _P, _P]),
+    'lcb_bklm_aggregate_verify_batch': (c_int, [c_void_p, POINTER(LcbScheme), _P, c_int64, _P, _P, _P, _P, _P, _P, c_int,
+                                                c_int, c_int, _P]),
     'lcb_adaptor_witgen_batch': (c_int, [c_void_p, POINTER(LcbScheme), _P, _P, c_int64, _P, _P, _P]),
     'lcb_vec_add_batch': (c_int, [c_void_p, _P, _P, c_int64, _P]),
     'lcb_vec_sub_batch': (c_int, [c_void_p, _P, _P, c_int64, _P]),

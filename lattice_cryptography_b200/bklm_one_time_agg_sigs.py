@@ -6,6 +6,8 @@ Drop-in: make_setup_parameters, prepare_make_agg_coefs, prepare_hash2polyinput, 
 Sharded: aggregate_shard / aggregate_finish, aggregate_verify_shard / aggregate_verify_finish -
          each rank (GPU) handles a contiguous range of the SORTED list and the int32 partial sums
          are added across ranks (one NCCL reduce; see lattice_cryptography_b200.distributed).
+Batched: aggregate_batch, aggregate_verify_batch - many independent aggregates (the reference caps one at
+         ag_cap = 2 signatures) in one engine call; element g equals aggregate / aggregate_verify of group g.
 
 Sorting by str(otvk) and building the hash-input strings stay on the host: they depend on CPython
 object identity (SURVEY.md section 0.4).  The shipped parameters have ag_wt = ag_bd = 1, i.e. every
@@ -206,3 +208,93 @@ def aggregate_verify(pp: PublicParameters, otvks: List[OneTimeVerificationKey], 
     vk_sorted = np.ascontiguousarray(np.stack([np.stack([k[0].ntt, k[1].ntt]) for k in srt_keys]))
     partial = aggregate_verify_shard(pp, vk_sorted, challenge_messages(srt_keys, srt_msgs), agmsg, 0)
     return aggregate_verify_finish(pp, partial, np.ascontiguousarray(ag_sig.coef), len(otvks))
+
+
+# ------------------------------------------------------------------------------- batched drop-in API
+def _commit_batch(pp: PublicParameters, agmsgs: List[str]) -> List[str]:
+    """commit_aggregation_message of every message, with two hash calls in all: every leaf of every message, then
+    every root."""
+    eng, _ = _ctx(pp)
+    raws = [m.encode() for m in agmsgs]
+    lens = [len(r) for r in raws]
+    base = np.concatenate([[0], np.cumsum(lens, dtype=np.int64)]).astype(np.int64)
+    cuts = [np.arange(base[g], base[g + 1], TREE_LEAF_BYTES, dtype=np.int64) for g in range(len(raws))]
+    nleaf = [len(c) for c in cuts]
+    leaves = np.zeros((0, 32), dtype=np.uint8)
+    if sum(nleaf):
+        blob = np.frombuffer(b''.join(raws), dtype=np.uint8)
+        off = np.concatenate(cuts + [base[-1:]]).astype(np.int64)
+        leaves = eng.shake256((np.ascontiguousarray(blob), off), 32)
+    first = np.concatenate([[0], np.cumsum(nleaf)]).astype(np.int64)
+    tops = [TREE_DOMAIN + lens[g].to_bytes(8, 'little') + leaves[first[g]:first[g + 1]].tobytes() for g in range(len(raws))]
+    if not tops:
+        return []
+    return [bytes(r).hex() for r in eng.shake256(tops, 32)]
+
+
+def _batch_messages(pp: PublicParameters, agmsgs: List[str]) -> List[str]:
+    return _commit_batch(pp, agmsgs) if pp.get('ag_mode', 'reference') == 'tree' else agmsgs
+
+
+def _check_messages(otvks, msgs) -> None:
+    """The argument checks of prepare_make_agg_coefs, without its sort."""
+    if len(otvks) != len(msgs):
+        raise ValueError("Cannot prepare_make_agg_coefs without two input vectors of equal length.")
+    elif not all(is_bitstring(msg) for msg in msgs):
+        raise ValueError("Input messages must be bitstrings.")
+
+
+def aggregate_batch(pp: PublicParameters, otvks: List[List[OneTimeVerificationKey]], msgs: List[List[Message]],
+                    sigs: List[List[Signature]]) -> List[Signature]:
+    """[aggregate(pp, otvks[g], msgs[g], sigs[g]) for every g] in one engine call (same errors, raised for the first
+    group that has one).  Sorting and the aggregation message stay on the host, once per group."""
+    if not len(otvks) == len(msgs) == len(sigs):
+        raise ValueError('aggregate_batch needs one list of keys, messages and signatures per aggregate')
+    sp = pp['scheme_parameters']
+    rows, agmsgs, counts = [], [], []
+    for keys_g, msgs_g, sigs_g in zip(otvks, msgs, sigs):
+        srt_keys, srt_msgs, srt_sigs = prepare_aggregate(otvks=keys_g, msgs=msgs_g, sigs=sigs_g)
+        _check_messages(keys_g, msgs_g)
+        if not srt_sigs:
+            raise ValueError('need at least one array to stack')      # what aggregate() raises for an empty group
+        rows.extend(s.coef for s in srt_sigs)
+        agmsgs.append(str(list(zip(srt_keys, srt_msgs))))
+        counts.append(len(srt_sigs))
+    if not counts:
+        return []
+    eng, sch = _ctx(pp)
+    agg_off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
+    out = eng.aggregate_batch(sch, agg_off, np.ascontiguousarray(np.stack(rows)), _batch_messages(pp, agmsgs))
+    return [PolynomialVector(sp.lp, const_time_flag=False, _coef=out[g]) for g in range(len(counts))]
+
+
+def aggregate_verify_batch(pp: PublicParameters, otvks: List[List[OneTimeVerificationKey]], msgs: List[List[Message]],
+                           ag_sigs: List[Signature]) -> List[bool]:
+    """[aggregate_verify(pp, otvks[g], msgs[g], ag_sigs[g]) for every g]: the host-side early False (length mismatch,
+    over capacity, ill-formed aggregate) per group, then every remaining group in one engine call."""
+    if not len(otvks) == len(msgs) == len(ag_sigs):
+        raise ValueError('aggregate_verify_batch needs one list of keys and messages and one aggregate per group')
+    lp = pp['scheme_parameters'].lp
+    verdicts = [False] * len(otvks)
+    live, vks, chmsgs, agmsgs, counts, ags = [], [], [], [], [], []
+    for g, (keys_g, msgs_g, ag_g) in enumerate(zip(otvks, msgs, ag_sigs)):
+        if len(keys_g) < 1 or len(keys_g) > pp['ag_cap'] or len(keys_g) != len(msgs_g):
+            continue
+        if not well_formed(lp, ag_g):
+            continue
+        srt_keys, srt_msgs = prepare_make_agg_coefs(otvks=keys_g, msgs=msgs_g)
+        vks.extend(np.stack([k[0].ntt, k[1].ntt]) for k in srt_keys)
+        chmsgs.extend(challenge_messages(srt_keys, srt_msgs))
+        agmsgs.append(str(list(zip(srt_keys, srt_msgs))))
+        counts.append(len(srt_keys))
+        ags.append(ag_g.coef)
+        live.append(g)
+    if not live:
+        return verdicts
+    eng, sch = _ctx(pp)
+    agg_off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
+    got = eng.aggregate_verify_batch(sch, agg_off, np.ascontiguousarray(np.stack(vks)), chmsgs, _batch_messages(pp, agmsgs),
+                                     np.ascontiguousarray(np.stack(ags)), pp['ag_cap'], pp['avf_bd'], pp['avf_wt'])
+    for g, v in zip(live, got):
+        verdicts[g] = bool(v)
+    return verdicts

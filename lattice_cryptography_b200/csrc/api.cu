@@ -4,6 +4,7 @@
 #include <cstdio>
 #include <cstring>
 #include <new>
+#include <algorithm>
 #include <cstdlib>
 #include <string>
 #include <vector>
@@ -78,10 +79,14 @@ int fail_cuda(lcb_ctx* c, cudaError_t e, const char* what) {
 constexpr int64_t kPipeChunk = 1 << 17;
 
 enum KernelId { K_SAMPLER = 0, K_SHAKE, K_NTT_FWD, K_NTT_INV, K_POLY_MUL, K_MATVEC, K_SIGN, K_VERIFY, K_ADDSUB,
-                K_AGG_COEFS, K_AGG_PARTIAL, K_AGG_FINISH, K_AGGV_PARTIAL, K_AGGV_FINISH, K_PACK, K_UNPACK, K_COUNT };
+                K_AGG_COEFS, K_AGG_PARTIAL, K_AGG_FINISH, K_AGGV_PARTIAL, K_AGGV_FINISH, K_PACK, K_UNPACK, K_GROUP_IDS,
+                K_AGG_COEFS_SEG, K_AGG_PARTIAL_SEG, K_AGGV_PARTIAL_SEG, K_AGGV_RESIDUES, K_AGGV_LIMITS, K_COUNT };
 const char* const kKernelNames[K_COUNT] = {"sampler", "shake256", "ntt_fwd", "ntt_inv", "poly_mul", "matvec", "sign",
                                            "verify", "vec_addsub", "agg_coefs", "agg_partial", "agg_finish",
-                                           "aggv_partial", "aggv_finish", "pack", "unpack"};
+                                           "aggv_partial", "aggv_finish", "pack", "unpack", "group_ids",
+                                           "agg_coefs_seg", "agg_partial_seg", "aggv_partial_seg", "aggv_residues",
+                                           "aggv_limits"};
+static_assert(K_COUNT <= 24, "grow lcb_ctx::prof_ms / prof_n");
 
 // Launch wrapper: counts the launch and, when profiling is on, brackets it with CUDA events on the
 // ctx stream (resolved lazily in lcb_profile_read).
@@ -417,6 +422,60 @@ int run_agg_coefs(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* d_agmsg, int
         c->launches += 1;                                  // the pre-split kernel
     }
     CK(c, timed(c, K_AGG_COEFS, [&] { return launch_agg_coefs(a, c->ring.num_sms, c->stream); }));
+    return LCB_OK;
+}
+
+
+// ---- batches of aggregates ------------------------------------------------------------------------------------
+// What the host needs of the offset arrays of a batch call: the item and message totals, and for the per-group
+// fallback every entry.  Host-resident arrays are checked (start at 0, never decrease; strictly increase when every
+// group must hold a signature); device-resident ones are trusted, as every device offset array of this ABI, and only
+// copied back as far as needed (one 8-byte read and a stream synchronisation for the totals).
+struct GroupOffsets {
+    int64_t items = 0, msg_bytes = 0;
+    std::vector<int64_t> agg, msg;     // filled when `all`
+};
+
+int read_offsets(lcb_ctx* c, const int64_t* off, int64_t n, bool strict, bool all, int64_t* last, std::vector<int64_t>& out,
+                 const char* what) {
+    if (on_device(off)) {
+        if (all) {
+            out.resize((size_t)n + 1);
+            CK(c, cudaMemcpyAsync(out.data(), off, out.size() * sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
+        } else {
+            CK(c, cudaMemcpyAsync(last, off + n, sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
+        }
+        CK(c, cudaStreamSynchronize(c->stream));
+        if (all) *last = out[(size_t)n];
+        return LCB_OK;
+    }
+    if (off[0] != 0) return fail(c, LCB_ERR_INVALID, std::string(what) + " must start at 0");
+    for (int64_t i = 0; i < n; ++i)
+        if (off[i + 1] < off[i] || (strict && off[i + 1] == off[i]))
+            return fail(c, LCB_ERR_INVALID, std::string(what) + (strict ? " must increase (every aggregate needs a signature)"
+                                                                         : " must not decrease"));
+    if (all) out.assign(off, off + n + 1);
+    *last = off[n];
+    return LCB_OK;
+}
+
+int group_offsets(lcb_ctx* c, const int64_t* agg_off, const int64_t* agmsg_off, int64_t n_agg, bool nonempty, bool all,
+                  GroupOffsets& g) {
+    int st = read_offsets(c, agg_off, n_agg, nonempty, all, &g.items, g.agg, "agg_off");
+    if (st == LCB_OK) st = read_offsets(c, agmsg_off, n_agg, false, all, &g.msg_bytes, g.msg, "agmsg_off");
+    if (st != LCB_OK) return st;
+    if (g.items < 0 || g.items > ((int64_t)1 << 30)) return fail(c, LCB_ERR_INVALID, "at most 2^30 signatures per batch call");
+    return LCB_OK;
+}
+
+// The aggregation-coefficient sampler arguments of the segmented kernel (ag_wt = ag_bd = 1)
+int seg_coef_args(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* d_msg, int64_t items, int16_t* d_pairs, SamplerArgs& a) {
+    int st = fill_sampler(c, a, salt_of(sch->ag_salt).c_str(), nullptr, sch->ag_bd, sch->ag_wt, 1);
+    if (st != LCB_OK) return fail(c, st, "bad aggregation parameters");
+    if (a.salt_len + 20 > 32) return fail(c, LCB_ERR_INVALID, "ag_salt longer than 12 bytes");
+    a.msgs = d_msg;
+    a.n = items;
+    a.out_pairs = d_pairs;
     return LCB_OK;
 }
 
@@ -1360,6 +1419,183 @@ int lcb_bklm_aggverify_finish(lcb_ctx* c, const int32_t* partial_sum, const int1
         return c->generic ? g_launch_aggv_finish(c->gen, d_partial, d_sig, total, ag_cap, avf_bd, avf_wt, d_verdict, c->stream)
                           : launch_aggv_finish(c->ring, d_partial, d_sig, total, ag_cap, avf_bd, avf_wt, d_verdict, c->stream);
     }));
+    CK(c, sg.finish());
+    return LCB_OK;
+}
+
+int lcb_bklm_aggregate_batch(lcb_ctx* c, const lcb_scheme* sch, const int64_t* agg_off, int64_t n_agg,
+                             const int16_t* sig_sorted, const uint8_t* agmsg, const int64_t* agmsg_off, int16_t* ag_sig) {
+    LCB_RANGE();
+    if (!c || !sch || !agg_off || !agmsg_off || n_agg < 0 || (n_agg > 0 && (!sig_sorted || !agmsg || !ag_sig)))
+        return LCB_ERR_INVALID;
+    if (sch->ag_wt < 1 || sch->ag_wt > c->d || sch->ag_bd < 1) return fail(c, LCB_ERR_INVALID, "bad aggregation parameters");
+    if (n_agg > ((int64_t)1 << 30)) return fail(c, LCB_ERR_INVALID, "more than 2^30 aggregates in one call");
+    if (n_agg == 0) return LCB_OK;
+    CK(c, cudaSetDevice(c->device));
+    const bool fast = !c->generic && sch->ag_wt == 1 && sch->ag_bd == 1;
+    GroupOffsets go;
+    int st = group_offsets(c, agg_off, agmsg_off, n_agg, true, !fast, go);
+    if (st != LCB_OK) return st;
+    const int l = c->l;
+    const size_t D_ = (size_t)c->d * ew(c);
+    const size_t pair_len = (size_t)sch->ag_wt * 2 * ew(c);
+    Staging sg(c);
+    const int16_t* d_sig;
+    const uint8_t* d_msg;
+    const int64_t *d_aoff, *d_moff;
+    int16_t* d_out;
+    int32_t* d_part;
+    CK(c, sg.in(&d_sig, sig_sorted, (size_t)go.items * l * D_));
+    CK(c, sg.in(&d_msg, agmsg, (size_t)go.msg_bytes));
+    CK(c, sg.in(&d_aoff, agg_off, (size_t)n_agg + 1));
+    CK(c, sg.in(&d_moff, agmsg_off, (size_t)n_agg + 1));
+    CK(c, sg.out(&d_out, ag_sig, (size_t)n_agg * l * D_));
+    CK(c, sg.alloc((void**)&d_part, (size_t)n_agg * l * D_ * sizeof(int32_t)));
+    CK(c, cudaMemsetAsync(d_part, 0, (size_t)n_agg * l * D_ * sizeof(int32_t), c->stream));
+    if (fast) {
+        int32_t* d_gid;
+        int16_t* d_pairs;
+        CK(c, sg.alloc((void**)&d_gid, (size_t)go.items * sizeof(int32_t)));
+        CK(c, sg.alloc((void**)&d_pairs, (size_t)go.items * pair_len * sizeof(int16_t)));
+        SamplerArgs a{};
+        st = seg_coef_args(c, sch, d_msg, go.items, d_pairs, a);
+        if (st != LCB_OK) return st;
+        CK(c, timed(c, K_GROUP_IDS, [&] { return launch_group_ids(d_aoff, n_agg, go.items, d_gid, c->ring.num_sms, c->stream); }));
+        CK(c, timed(c, K_AGG_COEFS_SEG, [&] { return launch_agg_coefs_seg(a, d_gid, d_aoff, d_moff, n_agg, c->stream); }));
+        CK(c, timed(c, K_AGG_PARTIAL_SEG, [&] {
+            return launch_agg_partial_seg(c->ring, d_sig, d_pairs, d_gid, go.items, n_agg, d_part, c->stream);
+        }));
+        CK(c, timed(c, K_AGG_FINISH, [&] { return launch_agg_finish_n(c->ring, d_part, n_agg * l * D, d_out, c->stream); }));
+    } else {
+        // generic geometry or non-monomial coefficients: the single-aggregate kernels, group by group (correct, not fast)
+        const bool monomial = sch->ag_wt == 1 && sch->ag_bd == 1;
+        int64_t most = 0;
+        for (int64_t g = 0; g < n_agg; ++g) most = std::max(most, go.agg[(size_t)g + 1] - go.agg[(size_t)g]);
+        int16_t* d_pairs;
+        CK(c, sg.alloc((void**)&d_pairs, (size_t)most * pair_len * sizeof(int16_t)));
+        for (int64_t g = 0; g < n_agg; ++g) {
+            const int64_t first = go.agg[(size_t)g], count = go.agg[(size_t)g + 1] - first;
+            const int16_t* sig_g = d_sig + (size_t)first * l * D_;
+            int32_t* part_g = d_part + (size_t)g * l * D_;
+            if (count > 0) {
+                st = run_agg_coefs(c, sch, d_msg + go.msg[(size_t)g], go.msg[(size_t)g + 1] - go.msg[(size_t)g], 0, count, d_pairs);
+                if (st != LCB_OK) return st;
+                CK(c, timed(c, K_AGG_PARTIAL, [&] {
+                    if (!monomial) return g_launch_agg_partial_poly(c->gen, sig_g, d_pairs, sch->ag_wt, count, part_g, c->stream);
+                    return g_launch_agg_partial(c->gen, sig_g, d_pairs, count, part_g, c->stream);
+                }));
+            }
+            CK(c, timed(c, K_AGG_FINISH, [&] {
+                return c->generic ? g_launch_agg_finish(c->gen, part_g, d_out + (size_t)g * l * D_, c->stream)
+                                  : launch_agg_finish(c->ring, part_g, d_out + (size_t)g * l * D_, c->stream);
+            }));
+        }
+    }
+    CK(c, sg.finish());
+    return LCB_OK;
+}
+
+int lcb_bklm_aggregate_verify_batch(lcb_ctx* c, const lcb_scheme* sch, const int64_t* agg_off, int64_t n_agg,
+                                    const uint16_t* vk_ntt_sorted, const uint8_t* chmsg_sorted, const int64_t* chmsg_off,
+                                    const uint8_t* agmsg, const int64_t* agmsg_off, const int16_t* ag_sig, int ag_cap,
+                                    int avf_bd, int avf_wt, uint8_t* verdict) {
+    LCB_RANGE();
+    if (!c || !sch || !agg_off || !agmsg_off || !chmsg_off || n_agg < 0 || (n_agg > 0 && (!agmsg || !ag_sig || !verdict)))
+        return LCB_ERR_INVALID;
+    if (sch->ag_wt < 1 || sch->ag_wt > c->d || sch->ag_bd < 1) return fail(c, LCB_ERR_INVALID, "bad aggregation parameters");
+    if (!c->has_key_ch) return fail(c, LCB_ERR_NO_KEY_CH, "lcb_bklm_aggregate_verify_batch before lcb_set_key_ch");
+    if (n_agg > ((int64_t)1 << 30)) return fail(c, LCB_ERR_INVALID, "more than 2^30 aggregates in one call");
+    if (n_agg == 0) return LCB_OK;
+    CK(c, cudaSetDevice(c->device));
+    const bool fast = !c->generic && sch->ag_wt == 1 && sch->ag_bd == 1;
+    GroupOffsets go;
+    int st = group_offsets(c, agg_off, agmsg_off, n_agg, false, !fast, go);
+    if (st != LCB_OK) return st;
+    if (go.items > 0 && (!vk_ntt_sorted || !chmsg_sorted)) return LCB_ERR_INVALID;
+    int64_t ch_bytes = 0;
+    std::vector<int64_t> unused;
+    if (go.items > 0 && !on_device(chmsg_off)) {
+        st = read_offsets(c, chmsg_off, go.items, false, false, &ch_bytes, unused, "chmsg_off");
+        if (st != LCB_OK) return st;
+    }
+    if (go.items > 0) CK(c, last_offset(c, chmsg_sorted, chmsg_off, go.items, &ch_bytes));
+    const int l = c->l;
+    const size_t D_ = (size_t)c->d * ew(c);
+    const size_t pair_len = (size_t)sch->ag_wt * 2 * ew(c);
+    Staging sg(c);
+    const uint16_t* d_vk;
+    const uint8_t *d_chmsg, *d_msg;
+    const int64_t *d_choff, *d_aoff, *d_moff;
+    const int16_t* d_ag;
+    uint8_t* d_verdict;
+    int16_t* d_ch;
+    int32_t* d_part;
+    CK(c, sg.in(&d_vk, vk_ntt_sorted, (size_t)go.items * 2 * D_));
+    CK(c, sg.in(&d_chmsg, chmsg_sorted, (size_t)ch_bytes));
+    CK(c, sg.in(&d_choff, chmsg_off, (size_t)go.items + 1));
+    CK(c, sg.in(&d_msg, agmsg, (size_t)go.msg_bytes));
+    CK(c, sg.in(&d_aoff, agg_off, (size_t)n_agg + 1));
+    CK(c, sg.in(&d_moff, agmsg_off, (size_t)n_agg + 1));
+    CK(c, sg.in(&d_ag, ag_sig, (size_t)n_agg * l * D_));
+    CK(c, sg.out(&d_verdict, verdict, (size_t)n_agg));
+    CK(c, sg.alloc((void**)&d_ch, (size_t)go.items * sch->ch_wt * 2 * ew(c) * sizeof(int16_t)));
+    CK(c, sg.alloc((void**)&d_part, (size_t)n_agg * D_ * sizeof(int32_t)));
+    CK(c, cudaMemsetAsync(d_part, 0, (size_t)n_agg * D_ * sizeof(int32_t), c->stream));
+    if (go.items > 0) {           // the challenges of every item of every group: one sampler launch
+        st = run_challenge(c, sch, d_chmsg, d_choff, go.items, d_ch);
+        if (st != LCB_OK) return st;
+    }
+    if (fast) {
+        int32_t* d_gid;
+        int16_t* d_pairs;
+        uint16_t* d_rhs;
+        CK(c, sg.alloc((void**)&d_gid, (size_t)go.items * sizeof(int32_t)));
+        CK(c, sg.alloc((void**)&d_pairs, (size_t)go.items * pair_len * sizeof(int16_t)));
+        CK(c, sg.alloc((void**)&d_rhs, (size_t)n_agg * D * sizeof(uint16_t)));
+        SamplerArgs a{};
+        st = seg_coef_args(c, sch, d_msg, go.items, d_pairs, a);
+        if (st != LCB_OK) return st;
+        CK(c, timed(c, K_GROUP_IDS, [&] { return launch_group_ids(d_aoff, n_agg, go.items, d_gid, c->ring.num_sms, c->stream); }));
+        CK(c, timed(c, K_AGG_COEFS_SEG, [&] { return launch_agg_coefs_seg(a, d_gid, d_aoff, d_moff, n_agg, c->stream); }));
+        CK(c, timed(c, K_AGGV_PARTIAL_SEG, [&] {
+            return launch_aggv_partial_seg(c->ring, d_vk, d_ch, sch->ch_wt, d_pairs, d_gid, go.items, n_agg, d_part, c->stream);
+        }));
+        CK(c, timed(c, K_AGGV_RESIDUES, [&] { return launch_aggv_residues(c->ring, d_part, n_agg * D, d_rhs, c->stream); }));
+        // bounds and key_ch * ag_sig == rhs: the witness-verify form of k_verify.  Every int16 passes a bound of 32768, as
+        // it passes any larger one in k_aggv_finish.
+        CK(c, timed(c, K_VERIFY, [&] {
+            return launch_verify(c->ring, d_ag, nullptr, nullptr, 0, d_rhs, nullptr, n_agg, std::min(avf_bd, 32768), avf_wt,
+                                 d_verdict, c->stream);
+        }));
+        CK(c, timed(c, K_AGGV_LIMITS, [&] { return launch_aggv_limits(c->ring, d_aoff, n_agg, d_ag, ag_cap, d_verdict, c->stream); }));
+    } else {
+        // generic geometry or non-monomial coefficients: the single-aggregate kernels, group by group (correct, not fast)
+        const bool monomial = sch->ag_wt == 1 && sch->ag_bd == 1;
+        int64_t most = 0;
+        for (int64_t g = 0; g < n_agg; ++g) most = std::max(most, go.agg[(size_t)g + 1] - go.agg[(size_t)g]);
+        int16_t* d_pairs;
+        CK(c, sg.alloc((void**)&d_pairs, (size_t)most * pair_len * sizeof(int16_t)));
+        for (int64_t g = 0; g < n_agg; ++g) {
+            const int64_t first = go.agg[(size_t)g], count = go.agg[(size_t)g + 1] - first;
+            int32_t* part_g = d_part + (size_t)g * D_;
+            const int16_t* ag_g = d_ag + (size_t)g * l * D_;
+            if (count > 0) {
+                const uint16_t* vk_g = d_vk + (size_t)first * 2 * D_;
+                const int16_t* ch_g = d_ch + (size_t)first * sch->ch_wt * 2 * ew(c);
+                st = run_agg_coefs(c, sch, d_msg + go.msg[(size_t)g], go.msg[(size_t)g + 1] - go.msg[(size_t)g], 0, count, d_pairs);
+                if (st != LCB_OK) return st;
+                CK(c, timed(c, K_AGGV_PARTIAL, [&] {
+                    if (!monomial)
+                        return g_launch_aggv_partial_poly(c->gen, vk_g, ch_g, sch->ch_wt, d_pairs, sch->ag_wt, count, part_g, c->stream);
+                    return g_launch_aggv_partial(c->gen, vk_g, ch_g, sch->ch_wt, d_pairs, count, part_g, c->stream);
+                }));
+            }
+            CK(c, timed(c, K_AGGV_FINISH, [&] {
+                return c->generic ? g_launch_aggv_finish(c->gen, part_g, ag_g, count, ag_cap, avf_bd, avf_wt, d_verdict + g, c->stream)
+                                  : launch_aggv_finish(c->ring, part_g, ag_g, count, ag_cap, avf_bd, avf_wt, d_verdict + g, c->stream);
+            }));
+        }
+    }
     CK(c, sg.finish());
     return LCB_OK;
 }

@@ -71,6 +71,11 @@ cudaError_t launch_agg_coefs(const SamplerArgs& a, int num_sms, cudaStream_t st)
 bool agg_coefs_two_lane(int64_t n, int num_sms);
 inline int64_t agg_il_stride(int64_t msg_len) { return msg_len / 8 + 1; }
 inline size_t agg_il_bytes(int64_t msg_len) { return (size_t)8 * (size_t)agg_il_stride(msg_len) * sizeof(uint2); }
+// batches of independent aggregates (lcb_bklm_aggregate_batch): gid[i] = group of sorted item i, built once per call
+// and shared by the segmented kernels; the coefficient of item i is H2P(salt || str(i - agg_off[g]) || message g)
+cudaError_t launch_group_ids(const int64_t* agg_off, int64_t n_agg, int64_t total, int32_t* gid, int num_sms, cudaStream_t st);
+cudaError_t launch_agg_coefs_seg(const SamplerArgs& a, const int32_t* gid, const int64_t* agg_off, const int64_t* msg_off,
+                                 int64_t n_agg, cudaStream_t st);
 
 // ---- generic degree / modulus (ring_generic.cu) -------------------------------------------------------------
 struct GenRing {
@@ -154,6 +159,18 @@ cudaError_t launch_aggv_partial(const RingCtx& c, const uint16_t* vk_ntt, const 
                                 const int16_t* ag_pairs, int64_t count, int32_t* partial, cudaStream_t st);
 cudaError_t launch_aggv_finish(const RingCtx& c, const int32_t* partial, const int16_t* ag_sig, int64_t total,
                                int ag_cap, int avf_bd, int avf_wt, uint8_t* verdict, cudaStream_t st);
+// batches of aggregates (items sorted by group, gid from launch_group_ids): partial int32[n_agg][l][256] /
+// int32[n_agg][256], zeroed by the caller; k_agg_finish over nelem elements; residues of the verify partials in [0, q);
+// the lower limits k_verify does not check (1 <= count_g <= ag_cap, ag_sig != 0), ANDed into verdict
+cudaError_t launch_agg_partial_seg(const RingCtx& c, const int16_t* sigs, const int16_t* ag_pairs, const int32_t* gid,
+                                   int64_t total, int64_t n_agg, int32_t* partial, cudaStream_t st);
+cudaError_t launch_agg_finish_n(const RingCtx& c, const int32_t* partial, int64_t nelem, int16_t* ag_sig, cudaStream_t st);
+cudaError_t launch_aggv_partial_seg(const RingCtx& c, const uint16_t* vk_ntt, const int16_t* ch_pairs, int ch_wt,
+                                    const int16_t* ag_pairs, const int32_t* gid, int64_t total, int64_t n_agg,
+                                    int32_t* partial, cudaStream_t st);
+cudaError_t launch_aggv_residues(const RingCtx& c, const int32_t* partial, int64_t nelem, uint16_t* out, cudaStream_t st);
+cudaError_t launch_aggv_limits(const RingCtx& c, const int64_t* agg_off, int64_t n_agg, const int16_t* ag_sig, int64_t ag_cap,
+                               uint8_t* verdict, cudaStream_t st);
 
 // wire format (wire.cu): `bits`-bit little-endian packing of (x + bias) mod 2^16, 32*bits bytes per polynomial
 cudaError_t launch_pack(const RingCtx& c, const void* in, int64_t npoly, int bits, int bias, uint8_t* out,

@@ -6,6 +6,7 @@
 //   bounds; key_ch*sig == vk0*c+vk1[+st] lm_one_time_sigs.py:173-191, adaptor_sigs.py:198-266 -> k_verify
 //   sum(sig ** ag)                      bklm_one_time_agg_sigs.py:96                       -> k_agg_partial
 //   sum((vk0*c+vk1)*ag); key_ch*ag_sig == . bklm_one_time_agg_sigs.py:99-116               -> k_aggv_*
+//   the same for many aggregates per call                                                  -> k_agg*_partial_seg
 //   presig + wit, sig - presig          adaptor_sigs.py:221,225                            -> k_vec_addsub
 //
 // Work mapping: one polynomial vector (one signature / key half / instance) per HALF-WARP; a lane
@@ -880,6 +881,270 @@ __global__ void __launch_bounds__(RBS, 4) k_aggv_partial(ModQ m, StageConstF scf
     for (int i = threadIdx.x; i < D; i += blockDim.x) atomicAdd(&partial[i], (int32_t)(red[i] % m.q));
 }
 
+// ------------------------------------------------------------------------------------------------
+// Batches of independent aggregates (lcb_bklm_aggregate_batch / lcb_bklm_aggregate_verify_batch).  The sorted items of
+// all groups lie back to back; gid[i] is the group of item i.  Each warp (half-warp) owns ONE CONTIGUOUS range of
+// items, accumulates while consecutive items belong to the same group and flushes the sum into that group's slice of
+// `partial` with atomicAdd when the group changes and at the end of its range.  A group is thus flushed at most once
+// per warp (half-warp) whose range it touches, and each flush adds a value reduced mod q (|v| < q < 2^16): with at
+// most SEG_MAX_WARPS such ranges per polynomial, |partial| < 2^14 * 2^16 = 2^30 and int32 cannot overflow.
+constexpr int SEG_MAX_WARPS = 1 << 14;
+// rows accumulated between in-register reductions of k_agg_partial_seg: 2^15 rows of |x| <= 2^15 stay below 2^30
+constexpr int SEG_REDUCE_ROWS = 1 << 15;
+
+// Aggregate: partial[g][i][p] += s * sig[t][i][(p - k) mod 256] * (p < k ? -1 : 1) over the items t of group g.
+// grid = (chunks, l) as k_agg_partial, but warp w of polynomial i walks rows [w R, (w + 1) R) in order.  Rows are
+// parked as E = [~row | row] exactly as in k_agg_partial; the wrapped reads (~v = -v - 1 instead of -v) are repaired
+// per group: lane 0 counts s per rotation k in the warp's own histogram, and a flush adds
+// corr[p] = sum over k > p of hist[k] (a warp suffix scan of the 256 counts) before it clears the histogram.
+// Three resident blocks (79 registers); at four the 64-register cap spills 48 bytes.
+__global__ void __launch_bounds__(32 * AGG_WARPS, 3) k_agg_partial_seg(ModQ m, int l, const int16_t* __restrict__ sigs,
+                                                                   const int16_t* __restrict__ ag_pairs,
+                                                                   const int32_t* __restrict__ gid, int64_t total,
+                                                                   int64_t n_agg, int64_t per_warp,
+                                                                   int32_t* __restrict__ partial) {
+    __shared__ __align__(16) int32_t hist[AGG_WARPS][D];
+    __shared__ __align__(16) int16_t rows[AGG_WARPS][AGG_DEPTH][2 * D];
+    const int poly = blockIdx.y;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    int32_t* hw = hist[warp];
+#pragma unroll
+    for (int jj = 0; jj < 8; ++jj) hw[lane + 32 * jj] = 0;
+    const int64_t t_begin = ((int64_t)blockIdx.x * AGG_WARPS + warp) * per_warp;
+    const int64_t t_end = min(t_begin + per_warp, total);
+    int left = t_begin < t_end ? (int)(t_end - t_begin) : 0;
+    const uint32_t* app = reinterpret_cast<const uint32_t*>(ag_pairs) + t_begin;
+    const int32_t* gp = gid + t_begin;
+    const unsigned char* rowp = reinterpret_cast<const unsigned char*>(sigs + (t_begin * l + poly) * D) + 16 * lane;
+    const int64_t rstep = (int64_t)l * (D * 2);
+    int32_t acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    uint4 v[AGG_DEPTH];
+    uint32_t pr[AGG_DEPTH];
+    int grp[AGG_DEPTH];
+    auto fetch = [&]() {                         // the next min(left, AGG_DEPTH) rows; missing rows are never folded
+#pragma unroll
+        for (int j = 0; j < AGG_DEPTH; ++j)
+            if (j < left) {
+                v[j] = __ldg(reinterpret_cast<const uint4*>(rowp + j * rstep));
+                pr[j] = __ldg(app + j);
+                grp[j] = __ldg(gp + j);
+            }
+        LCB_CHECK(left <= 0 || (app - reinterpret_cast<const uint32_t*>(ag_pairs)) + min(left, AGG_DEPTH) <= total);
+        rowp += AGG_DEPTH * rstep;
+        app += AGG_DEPTH;
+        gp += AGG_DEPTH;
+    };
+    int cur_g = -1, since = 0;
+    auto flush = [&]() {
+        __syncwarp();
+        // corr[p] = sum_{k > p} hist[k]: lane owns counts 8 lane .. 8 lane + 7, suffix sums inside, then across lanes
+        int4 h0 = *reinterpret_cast<const int4*>(hw + 8 * lane), h1 = *reinterpret_cast<const int4*>(hw + 8 * lane + 4);
+        int hv[8] = {h0.x, h0.y, h0.z, h0.w, h1.x, h1.y, h1.z, h1.w};
+        int sfx[8];
+        sfx[7] = 0;
+#pragma unroll
+        for (int i = 6; i >= 0; --i) sfx[i] = sfx[i + 1] + hv[i + 1];
+        const int own = sfx[0] + hv[0];
+        int above = own;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int y = __shfl_down_sync(0xFFFFFFFFu, above, o);
+            if (lane + o < 32) above += y;
+        }
+        above -= own;
+        __syncwarp();
+        *reinterpret_cast<int4*>(hw + 8 * lane) = make_int4(sfx[0] + above, sfx[1] + above, sfx[2] + above, sfx[3] + above);
+        *reinterpret_cast<int4*>(hw + 8 * lane + 4) = make_int4(sfx[4] + above, sfx[5] + above, sfx[6] + above, sfx[7] + above);
+        __syncwarp();
+        LCB_CHECK(cur_g >= 0 && cur_g < n_agg);
+        int32_t* out = partial + ((int64_t)cur_g * l + poly) * D;
+#pragma unroll
+        for (int jj = 0; jj < 8; ++jj) {
+            // |acc| < q + 2^30 and |corr| <= 2^30 before the reduction of corr: no int32 overflow
+            const int32_t r = (acc[jj] + hw[lane + 32 * jj] % (int)m.q) % (int)m.q;
+            atomicAdd(out + lane + 32 * jj, r);
+            acc[jj] = 0;
+        }
+        __syncwarp();
+#pragma unroll
+        for (int jj = 0; jj < 8; ++jj) hw[lane + 32 * jj] = 0;
+        __syncwarp();
+        since = 0;
+    };
+    if (left > 0) fetch();
+    const unsigned rows_s = (unsigned)__cvta_generic_to_shared(rows[warp][0]);
+    while (left > 0) {
+        const int nrow = min(left, AGG_DEPTH);
+        uint32_t cur[AGG_DEPTH];
+        int cg[AGG_DEPTH];
+        __syncwarp();
+#pragma unroll
+        for (int j = 0; j < AGG_DEPTH; ++j) {
+            uint4* e = reinterpret_cast<uint4*>(rows[warp][j]);
+            e[lane] = make_uint4(~v[j].x, ~v[j].y, ~v[j].z, ~v[j].w);
+            e[32 + lane] = v[j];
+            cur[j] = pr[j];
+            cg[j] = grp[j];
+        }
+        __syncwarp();
+        left -= AGG_DEPTH;
+        if (left > 0) fetch();                   // next rows in flight while this batch is folded
+#pragma unroll
+        for (int j = 0; j < AGG_DEPTH; ++j) {
+            if (j < nrow) {                      // warp-uniform
+                if (cg[j] != cur_g) {
+                    if (cur_g >= 0) flush();
+                    cur_g = cg[j];
+                } else if (since == SEG_REDUCE_ROWS) {
+#pragma unroll
+                    for (int jj = 0; jj < 8; ++jj) acc[jj] %= (int)m.q;
+                    since = 0;
+                }
+                const int k = (int)(cur[j] & 0xFF);
+                const int sg = (int)(int16_t)(cur[j] >> 16);
+                const unsigned a = rows_s + (unsigned)(j * 4 * D) + 2u * (unsigned)(D - k + lane);
+#pragma unroll
+                for (int jj = 0; jj < 8; ++jj) {
+                    int x;
+                    asm volatile("ld.shared.s16 %0, [%1];" : "=r"(x) : "r"(a + 64u * jj));
+                    acc[jj] += sg * x;
+                }
+                if (lane == 0) hw[k] += sg;
+                ++since;
+            }
+        }
+    }
+    if (cur_g >= 0) flush();
+}
+
+// Aggregate-verify right-hand sides of many groups: the per-item math of k_aggv_partial (one half-warp per item,
+// FP32-assisted challenge transform, lazy 64-bit accumulation), but half-warp h walks items [h R, (h + 1) R) in order
+// and flushes per group.  Every half-warp runs the same number of trips (items past its range are dead, as the clamped
+// tail of k_aggv_partial) because the transform synchronises the whole warp.  A trip adds t * w < 2^18 * 2^16 to the
+// accumulator; reduce64 takes sums below 2^54, so a range holds at most 2^20 items (the launcher sizes the grid so).
+__global__ void __launch_bounds__(RBS, 4) k_aggv_partial_seg(ModQ m, StageConstF scf, const NttTables* __restrict__ tab,
+                                                             const uint16_t* __restrict__ vk_ntt,
+                                                             const int16_t* __restrict__ ch_pairs, int ch_wt,
+                                                             const int16_t* __restrict__ ag_pairs,
+                                                             const int32_t* __restrict__ gid, int64_t total,
+                                                             int64_t n_agg, int64_t per_hw, int32_t* __restrict__ partial) {
+    __shared__ __align__(16) uint32_t xbuf[(RBS / 32) * XWARP];
+    __shared__ __align__(16) uint4 twtab[LANES * TW_ROW];
+    __shared__ uint32_t pw[512];
+    for (int i = threadIdx.x; i < 512; i += blockDim.x) pw[i] = tab->pw[i];
+    fill_tw_shared(twtab, tab);
+    const HalfWarp h = half_warp(xbuf);
+    const LaneTwFShared twf{twtab + h.lane * TW_ROW};
+    uint32_t odd[EPT];
+#pragma unroll
+    for (int k = 0; k < EPT; ++k) odd[k] = 2 * (__brev((uint32_t)(16 * h.lane + k)) >> 24) + 1;
+    uint64_t acc[EPT];
+#pragma unroll
+    for (int k = 0; k < EPT; ++k) acc[k] = 0;
+    const uint32_t* ap = reinterpret_cast<const uint32_t*>(ag_pairs);
+    const uint32_t* cp = reinterpret_cast<const uint32_t*>(ch_pairs);
+    const int64_t t_begin = ((int64_t)blockIdx.x * HWB + h.slot) * per_hw;
+    const int64_t t_end = min(t_begin + per_hw, total);
+    auto item_of = [&](int64_t t) { return t < t_end ? t : (t_begin < total ? t_begin : total - 1); };
+    uint32_t n_c0 = 0, n_c1 = 0, n_pr = 0;
+    int n_g = 0;
+    auto prefetch = [&](int64_t t) {
+        const int64_t it = item_of(t);
+        LCB_CHECK(it >= 0 && it < total);
+        const uint32_t* q = cp + it * ch_wt;
+        n_c0 = h.lane < ch_wt ? __ldg(q + h.lane) : 0xFFFF0000u;            // index 0, coefficient -1: never written
+        n_c1 = h.lane + LANES < ch_wt ? __ldg(q + h.lane + LANES) : 0xFFFF0000u;
+        n_pr = __ldg(ap + it);
+        n_g = __ldg(gid + it);
+    };
+    int cur_g = -1;
+    auto flush = [&]() {
+        LCB_CHECK(cur_g >= 0 && cur_g < n_agg);
+#pragma unroll
+        for (int k = 0; k < EPT; ++k) {
+            atomicAdd(&partial[(int64_t)cur_g * D + 16 * h.lane + k], (int32_t)reduce64(acc[k], m));
+            acc[k] = 0;
+        }
+    };
+    prefetch(t_begin);
+    for (int64_t t = t_begin; t < t_begin + per_hw; ++t) {
+        const bool live = t < t_end;
+        const int64_t item = item_of(t);
+        const uint32_t c0 = n_c0, c1 = n_c1, pr = n_pr;
+        const int g = n_g;
+        const uint4* vkp = reinterpret_cast<const uint4*>(vk_ntt + item * 2 * D + 16 * h.lane);
+        const uint4 va = __ldg(vkp), vb = __ldg(vkp + 1), vc = __ldg(vkp + D / 8), vd = __ldg(vkp + D / 8 + 1);
+        if (t + 1 < t_begin + per_hw) prefetch(t + 1);
+        uint32_t c[EPT];
+        {
+            int cx[EPT];
+#pragma unroll
+            for (int j = 0; j < EPT; ++j) h.xb[XROW * j + h.lane] = 0;
+            __syncwarp();
+            if (h.lane < ch_wt) h.xb[XROW * ((c0 & 0xFFu) >> 4) + (c0 & 15u)] = (uint32_t)(int)(int16_t)(c0 >> 16);
+            if (h.lane + LANES < ch_wt) h.xb[XROW * ((c1 & 0xFFu) >> 4) + (c1 & 15u)] = (uint32_t)(int)(int16_t)(c1 >> 16);
+            for (int e = h.lane + 2 * LANES; e < ch_wt; e += LANES) {
+                const uint32_t w = __ldg(cp + item * ch_wt + e);
+                h.xb[XROW * ((w & 0xFFu) >> 4) + (w & 15u)] = (uint32_t)(int)(int16_t)(w >> 16);
+            }
+            __syncwarp();
+#pragma unroll
+            for (int j = 0; j < EPT; ++j) cx[j] = (int)h.xb[XROW * j + h.lane];
+            __syncwarp();
+            ntt_fwd_256_fp(cx, c, m, scf, twf, h.xb, h.lane);
+        }
+        if (live && g != cur_g) {                // half-warp-uniform
+            if (cur_g >= 0) flush();
+            cur_g = g;
+        }
+        const uint32_t wl[8] = {va.x, va.y, va.z, va.w, vb.x, vb.y, vb.z, vb.w};
+        const uint32_t wr[8] = {vc.x, vc.y, vc.z, vc.w, vd.x, vd.y, vd.z, vd.w};
+        const uint32_t kk = pr & 0xFF;
+        const uint32_t negoff = (int16_t)(pr >> 16) < 0 ? 256u : 0u;
+#pragma unroll
+        for (int k = 0; k < EPT; ++k) {
+            const uint32_t vl = (k & 1) ? wl[k >> 1] >> 16 : wl[k >> 1] & 0xFFFFu;
+            const uint32_t vr = (k & 1) ? wr[k >> 1] >> 16 : wr[k >> 1] & 0xFFFFu;
+            uint32_t ck = barrett_lazy(c[k] - FP_BIAS, m);                 // < 2q
+            ck = min(ck, ck - m.q);                                       // < q: the product below stays under 2^32
+            const uint32_t tt = barrett_lazy(ck * vl, m) + vr;            // < 2q + 2^16
+            const uint32_t w = live ? pw[(odd[k] * kk + negoff) & 511] : 0u;
+            acc[k] += (uint64_t)tt * w;
+        }
+    }
+    if (cur_g >= 0) flush();
+}
+
+// partial int32[n][256] -> residues uint16 in [0, q): the right-hand sides k_verify compares key_ch * ag_sig with
+__global__ void k_aggv_residues(ModQ m, const int32_t* __restrict__ partial, int64_t nelem, uint16_t* __restrict__ out) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nelem; i += (int64_t)gridDim.x * blockDim.x) {
+        int v = partial[i] % (int)m.q;
+        out[i] = (uint16_t)(v < 0 ? v + (int)m.q : v);
+    }
+}
+
+// The lower limits k_verify does not test: 1 <= count_g <= ag_cap and ag_sig[g] != 0 (max |coefficient| >= 1, i.e. also
+// weight >= 1).  One thread per group; the zero test stops at the first non-zero 16 bytes, so an honest aggregate costs
+// one sector and the aggregate signatures are not read a second time.
+__global__ void k_aggv_limits(const int64_t* __restrict__ agg_off, int64_t n_agg, const int16_t* __restrict__ ag_sig,
+                              int64_t words16, int64_t ag_cap, uint8_t* __restrict__ verdict) {
+    for (int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; g < n_agg; g += (int64_t)gridDim.x * blockDim.x) {
+        if (!verdict[g]) continue;
+        const int64_t cnt = __ldg(agg_off + g + 1) - __ldg(agg_off + g);
+        bool ok = cnt >= 1 && cnt <= ag_cap;
+        if (ok) {
+            const uint4* p = reinterpret_cast<const uint4*>(ag_sig) + g * words16;
+            bool nz = false;
+            for (int64_t w = 0; w < words16 && !nz; ++w) {
+                const uint4 x = __ldg(p + w);
+                nz = (x.x | x.y | x.z | x.w) != 0;
+            }
+            ok = nz;
+        }
+        if (!ok) verdict[g] = 0;
+    }
+}
+
 // bounds on ag_sig (with lower limits), key_ch * ag_sig == partial sum; one half-warp
 __global__ void __launch_bounds__(32) k_aggv_finish(ModQ m, StageConst sc, const NttTables* __restrict__ tab,
                                                     const uint32_t* __restrict__ a_hat, int l,
@@ -1079,6 +1344,59 @@ cudaError_t launch_aggv_finish(const RingCtx& c, const int32_t* partial, const i
                                int ag_cap, int avf_bd, int avf_wt, uint8_t* verdict, cudaStream_t st) {
     k_aggv_finish<<<1, 32, 0, st>>>(c.m, c.sc, c.tab, c.a_hat, c.l, partial, ag_sig, total, ag_cap, avf_bd, avf_wt,
                                     verdict);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_agg_finish_n(const RingCtx& c, const int32_t* partial, int64_t nelem, int16_t* ag_sig, cudaStream_t st) {
+    // k_agg_finish indexes with int: chunks of 2^30 elements
+    for (int64_t first = 0; first < nelem; first += (int64_t)1 << 30) {
+        const int n = (int)min(nelem - first, (int64_t)1 << 30);
+        k_agg_finish<<<(n + 255) / 256, 256, 0, st>>>(c.m, partial + first, n, ag_sig + first);
+        cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
+
+cudaError_t launch_agg_partial_seg(const RingCtx& c, const int16_t* sigs, const int16_t* ag_pairs, const int32_t* gid,
+                                   int64_t total, int64_t n_agg, int32_t* partial, cudaStream_t st) {
+    if (total <= 0) return cudaSuccess;
+    int64_t cap = (int64_t)c.num_sms * resident_blocks(k_agg_partial_seg, 32 * AGG_WARPS, 0) / c.l;
+    cap = max((int64_t)1, min(cap, (int64_t)SEG_MAX_WARPS / AGG_WARPS));
+    const int64_t need = (total + AGG_WARPS * AGG_DEPTH - 1) / (AGG_WARPS * AGG_DEPTH);
+    const int64_t chunks = min(need, cap);
+    const int64_t per_warp = (total + chunks * AGG_WARPS - 1) / (chunks * AGG_WARPS);
+    dim3 grid((unsigned)chunks, (unsigned)c.l);
+    k_agg_partial_seg<<<grid, 32 * AGG_WARPS, 0, st>>>(c.m, c.l, sigs, ag_pairs, gid, total, n_agg, per_warp, partial);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_aggv_partial_seg(const RingCtx& c, const uint16_t* vk_ntt, const int16_t* ch_pairs, int ch_wt,
+                                    const int16_t* ag_pairs, const int32_t* gid, int64_t total, int64_t n_agg,
+                                    int32_t* partial, cudaStream_t st) {
+    if (total <= 0) return cudaSuccess;
+    int64_t blocks = (int64_t)persistent_grid(total, HWB, c.num_sms, resident_blocks(k_aggv_partial_seg, RBS, 0));
+    blocks = min(blocks, (int64_t)SEG_MAX_WARPS / HWB);
+    const int64_t per_hw = (total + blocks * HWB - 1) / (blocks * HWB);
+    if (per_hw > ((int64_t)1 << 20)) return cudaErrorInvalidValue;      // reduce64 bound (see the kernel)
+    k_aggv_partial_seg<<<(unsigned)blocks, RBS, 0, st>>>(c.m, c.scf, c.tab, vk_ntt, ch_pairs, ch_wt, ag_pairs, gid, total,
+                                                         n_agg, per_hw, partial);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_aggv_residues(const RingCtx& c, const int32_t* partial, int64_t nelem, uint16_t* out, cudaStream_t st) {
+    if (nelem <= 0) return cudaSuccess;
+    const int64_t need = (nelem + 255) / 256;
+    k_aggv_residues<<<(unsigned)min(need, (int64_t)c.num_sms * 16), 256, 0, st>>>(c.m, partial, nelem, out);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_aggv_limits(const RingCtx& c, const int64_t* agg_off, int64_t n_agg, const int16_t* ag_sig, int64_t ag_cap,
+                               uint8_t* verdict, cudaStream_t st) {
+    if (n_agg <= 0) return cudaSuccess;
+    const int64_t need = (n_agg + 255) / 256;
+    k_aggv_limits<<<(unsigned)min(need, (int64_t)c.num_sms * 16), 256, 0, st>>>(agg_off, n_agg, ag_sig, (int64_t)c.l * D / 8,
+                                                                                ag_cap, verdict);
     return cudaGetLastError();
 }
 

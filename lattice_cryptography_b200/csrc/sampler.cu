@@ -402,6 +402,123 @@ __global__ void __launch_bounds__(ABS) k_agg_coefs(SamplerArgs a) {
     reinterpret_cast<uint32_t*>(a.out_pairs)[inst] = k | ((uint32_t)(uint16_t)(int16_t)sgn << 16);
 }
 
+// One sponge of the derivation: SHAKE256(salt || decimal(index) || msg[0 .. msg_len)) -> packed (k, +-1) pair.
+// The body of k_agg_coefs with the index, message and length as arguments (k_agg_coefs keeps its own copy: calling this
+// from it reorders its prologue, and that kernel stays as measured).  `edge` is the block's [RATE_WORDS][ABS] staging.
+__device__ __forceinline__ uint32_t agg_coef_pair(const SamplerArgs& a, uint64_t index, const uint8_t* msg, int64_t msg_len,
+                                                  uint32_t* edge) {
+    // salt' = ag_salt || decimal(index), at most 27 bytes, kept in eight registers as words
+    uint32_t sw[8];
+    const uint32_t* salt_w = reinterpret_cast<const uint32_t*>(a.salt);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) sw[i] = i < (SALT_BYTES / 4) ? salt_w[i] : 0;
+    int ndig = 1;
+    for (uint64_t v = index; v >= 10; v /= 10) ++ndig;
+    const int slen = a.salt_len + ndig;
+    {
+        uint64_t v = index;
+        for (int dpos = slen - 1; dpos >= a.salt_len; --dpos, v /= 10) {
+            const uint32_t ch = (uint32_t)('0' + (v % 10));
+#pragma unroll
+            for (int i = 0; i < 8; ++i)
+                if ((dpos >> 2) == i) sw[i] |= ch << (8 * (dpos & 3));
+        }
+    }
+    const int64_t tot = (int64_t)slen + msg_len;
+    const int64_t nblocks = tot / 136 + 1;
+    const int64_t last = nblocks * 136 - 1;
+    auto salt_byte = [&](int p) -> uint32_t {
+        uint32_t w = 0;
+#pragma unroll
+        for (int i = 0; i < 8; ++i)
+            if ((p >> 2) == i) w = sw[i];
+        return (w >> (8 * (p & 3))) & 0xFFu;
+    };
+    auto word_at = [&](int64_t k) -> uint32_t {
+        const int64_t p = 4 * k;
+        if (p >= slen && p + 4 <= tot) return load_u32_unaligned(msg + (p - slen));
+        uint32_t v = 0;
+#pragma unroll
+        for (int b = 0; b < 4; ++b) {
+            const int64_t q = p + b;
+            uint32_t byte = q < slen ? salt_byte((int)q) : (q < tot ? (uint32_t)__ldg(msg + (q - slen)) : (q == tot ? 0x1Fu : 0u));
+            if (q == last) byte ^= 0x80u;
+            v |= byte << (8 * b);
+        }
+        return v;
+    };
+    KeccakState s;
+#pragma unroll
+    for (int i = 0; i < 25; ++i) { s.lo[i] = 0; s.hi[i] = 0; }
+    for (int64_t blk = 0; blk < nblocks; ++blk) {
+        const int64_t k0 = blk * RATE_WORDS;
+        // interior blocks: every word is a plain unaligned message word
+        const bool interior = 4 * k0 >= slen && 4 * (k0 + RATE_WORDS) <= tot;
+        if (interior) {
+            const uint8_t* p = msg + (4 * k0 - slen);
+            const uintptr_t addr = reinterpret_cast<uintptr_t>(p);
+            const uint32_t* w = reinterpret_cast<const uint32_t*>(addr & ~(uintptr_t)3);
+            const unsigned sh = (unsigned)(addr & 3) * 8;
+#ifdef LCB_CHECKED
+            {   // the 34 or 35 aligned words of this block lie inside the (word-rounded) message
+                const uintptr_t lo_ok = reinterpret_cast<uintptr_t>(msg) & ~(uintptr_t)3;
+                const uintptr_t hi_ok = (reinterpret_cast<uintptr_t>(msg) + (uintptr_t)msg_len + 3) & ~(uintptr_t)3;
+                LCB_CHECK(reinterpret_cast<uintptr_t>(w) >= lo_ok && reinterpret_cast<uintptr_t>(w + 34 + (sh ? 1 : 0)) <= hi_ok);
+            }
+#endif
+            uint32_t prev = __ldg(w);
+#pragma unroll
+            for (int i = 0; i < 17; ++i) {
+                const uint32_t m1 = __ldg(w + 2 * i + 1);
+                const uint32_t m2 = (i < 16 || sh) ? __ldg(w + 2 * i + 2) : 0u;
+                s.lo[i] ^= __funnelshift_r(prev, m1, sh);
+                s.hi[i] ^= __funnelshift_r(m1, m2, sh);
+                prev = m2;
+            }
+        } else {
+            // first / last blocks (salt, tail, padding): assemble word by word through shared memory
+            for (int w2 = 0; w2 < RATE_WORDS; ++w2) edge[w2 * ABS + threadIdx.x] = word_at(k0 + w2);
+#pragma unroll
+            for (int i = 0; i < 17; ++i) {
+                s.lo[i] ^= edge[(2 * i) * ABS + threadIdx.x];
+                s.hi[i] ^= edge[(2 * i + 1) * ABS + threadIdx.x];
+            }
+        }
+        keccak_f1600(s, c_keccak_rc);
+    }
+    const uint32_t k = s.lo[0] & 0xFFu;                 // first digest byte: the 8 index bits
+    const int sgn = (s.lo[0] >> 15) & 1u ? 1 : -1;      // top bit of the second byte: the sign bit
+    return k | ((uint32_t)(uint16_t)(int16_t)sgn << 16);
+}
+
+
+// Many independent aggregates in one launch (lcb_bklm_aggregate_batch): stream i is local index j = i - agg_off[g] of
+// group g = gid[i] and hashes ag_salt || str(j) || msg[msg_off[g] .. msg_off[g+1]).  One thread per sponge, as
+// k_agg_coefs: the groups of the batch calls are short (the reference caps an aggregate at two signatures).
+__global__ void __launch_bounds__(ABS) k_agg_coefs_seg(SamplerArgs a, const int32_t* __restrict__ gid,
+                                                       const int64_t* __restrict__ agg_off, const int64_t* __restrict__ msg_off,
+                                                       int64_t n_agg) {
+    __shared__ uint32_t edge[RATE_WORDS * ABS];
+    const int64_t inst = (int64_t)blockIdx.x * ABS + threadIdx.x;
+    if (inst >= a.n) return;
+    const int g = __ldg(gid + inst);
+    LCB_CHECK(g >= 0 && g < n_agg);
+    const int64_t j = inst - __ldg(agg_off + g);
+    const int64_t m0 = __ldg(msg_off + g), m1 = __ldg(msg_off + g + 1);
+    LCB_CHECK(j >= 0 && m0 <= m1);
+    reinterpret_cast<uint32_t*>(a.out_pairs)[inst] = agg_coef_pair(a, (uint64_t)j, a.msgs + m0, m1 - m0, edge);
+}
+
+// gid[i] = group of sorted item i for i in [agg_off[g], agg_off[g+1]): one warp per group, lanes over its items
+__global__ void __launch_bounds__(256) k_group_ids(const int64_t* __restrict__ agg_off, int64_t n_agg, int64_t total,
+                                                   int32_t* __restrict__ gid) {
+    const int lane = threadIdx.x & 31;
+    for (int64_t g = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; g < n_agg; g += ((int64_t)gridDim.x * blockDim.x) >> 5) {
+        const int64_t a0 = __ldg(agg_off + g), a1 = __ldg(agg_off + g + 1);
+        LCB_CHECK(a0 >= 0 && a0 <= a1 && a1 <= total);
+        for (int64_t i = a0 + lane; i < a1; i += 32) gid[i] = (int32_t)g;
+    }
+}
 
 // ------------------------------------------------------------------------------------------------
 // The same derivation with TWO lanes per sponge (keccak_f1600_half, lcb_device.cuh), for launches that would
@@ -683,6 +800,20 @@ cudaError_t launch_agg_coefs(const SamplerArgs& a, int num_sms, cudaStream_t st)
     }
     int64_t blocks = (a.n + ABS - 1) / ABS;
     k_agg_coefs<<<(unsigned)blocks, ABS, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_group_ids(const int64_t* agg_off, int64_t n_agg, int64_t total, int32_t* gid, int num_sms, cudaStream_t st) {
+    if (n_agg <= 0 || total <= 0) return cudaSuccess;
+    const int64_t need = (n_agg + 7) / 8;                    // 8 warps (groups) per block
+    k_group_ids<<<(unsigned)(need < 16 * num_sms ? need : 16 * num_sms), 256, 0, st>>>(agg_off, n_agg, total, gid);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_agg_coefs_seg(const SamplerArgs& a, const int32_t* gid, const int64_t* agg_off, const int64_t* msg_off,
+                                 int64_t n_agg, cudaStream_t st) {
+    if (a.n <= 0) return cudaSuccess;
+    k_agg_coefs_seg<<<(unsigned)((a.n + ABS - 1) / ABS), ABS, 0, st>>>(a, gid, agg_off, msg_off, n_agg);
     return cudaGetLastError();
 }
 

@@ -390,6 +390,47 @@ class Engine(object):
                                                      avf_bd, avf_wt, _addr(verdict)))
         return bool(verdict[0])
 
+    # many independent aggregates per call (include/lcb200.h, lcb_bklm_aggregate_batch): group g covers the sorted rows
+    # agg_off[g] .. agg_off[g+1] and hashes agmsgs[g]
+    @staticmethod
+    def _groups(agg_off, total: int) -> int:
+        _want(agg_off, 'agg_off', np.int64, (None,))
+        if int(agg_off.shape[0]) < 1:
+            raise ValueError('agg_off needs n_agg + 1 entries')
+        if isinstance(agg_off, np.ndarray) and int(agg_off[-1]) != total:
+            raise ValueError(f'agg_off must end at the number of sorted items ({total}), not {int(agg_off[-1])}')
+        return int(agg_off.shape[0]) - 1
+
+    def aggregate_batch(self, sch: LcbScheme, agg_off, sig_sorted, agmsgs, device: bool = False):
+        """-> int16[n_agg, l, d]: aggregate g of the sorted signatures agg_off[g] .. agg_off[g+1] under agmsgs[g]."""
+        total = int(sig_sorted.shape[0]) if hasattr(sig_sorted, 'shape') and len(sig_sorted.shape) else 0
+        _want(sig_sorted, 'sig_sorted', self.ct, (total, self.l, self.d))
+        n_agg = self._groups(agg_off, total)
+        mblob, moff = self._rag(agmsgs)
+        if self._count(moff) != n_agg:
+            raise ValueError(f'{self._count(moff)} aggregation messages for {n_agg} aggregates')
+        out = self._out((n_agg, self.l, self.d), self.ct, device)
+        self._ck(self._lib.lcb_bklm_aggregate_batch(self._ctx, byref(sch), _addr(agg_off), n_agg, _addr(sig_sorted),
+                                                    _addr(mblob), _addr(moff), _addr(out)))
+        return out
+
+    def aggregate_verify_batch(self, sch: LcbScheme, agg_off, vk_ntt_sorted, chmsgs_sorted, agmsgs, ag_sig, ag_cap: int,
+                               avf_bd: int, avf_wt: int, device: bool = False):
+        """-> uint8[n_agg]: verdict g = aggregate_verify of group g (0 for an empty group or one above ag_cap)."""
+        cblob, coff = self._rag(chmsgs_sorted)
+        total = self._count(coff)
+        _want(vk_ntt_sorted, 'vk_ntt_sorted', self.nt, (total, 2, self.d))
+        n_agg = self._groups(agg_off, total)
+        _want(ag_sig, 'ag_sig', self.ct, (n_agg, self.l, self.d))
+        mblob, moff = self._rag(agmsgs)
+        if self._count(moff) != n_agg:
+            raise ValueError(f'{self._count(moff)} aggregation messages for {n_agg} aggregates')
+        verdict = self._out((n_agg,), np.uint8, device)
+        self._ck(self._lib.lcb_bklm_aggregate_verify_batch(self._ctx, byref(sch), _addr(agg_off), n_agg, _addr(vk_ntt_sorted),
+                                                           _addr(cblob), _addr(coff), _addr(mblob), _addr(moff),
+                                                           _addr(ag_sig), ag_cap, avf_bd, avf_wt, _addr(verdict)))
+        return verdict
+
     # ------------------------------------------------------------------ adaptor signatures
     def witgen(self, sch: LcbScheme, seeds, want_wit: bool = True, want_st_ntt: bool = True,
                want_st_coef: bool = True, device: bool = False):
