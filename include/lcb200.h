@@ -217,6 +217,29 @@ int lcb_bklm_aggregate_verify_batch(lcb_ctx* ctx, const lcb_scheme* sch, const i
                                     const int64_t* chmsg_off, const uint8_t* agmsg, const int64_t* agmsg_off,
                                     const int16_t* ag_sig, int ag_cap, int avf_bd, int avf_wt, uint8_t* verdict);
 
+/* The same two calls on the packed wire format (d = 256, q < 2^16 only; LCB_ERR_INVALID with "the packed wire format is
+ * defined for d == 256, q < 2^16 contexts only" otherwise).  An aggregate is packed like a signature, in
+ * ceil(log2(2 avf_bd + 1)) bits with bias avf_bd (12 bits at secpar 128, 14 at 256).  Results are exactly those of
+ * lcb_unpack_batch -> the unpacked batch call -> lcb_pack_batch, for any bytes in the packed buffers.  bits 1..16,
+ * biases 0..32767, packed buffers 4-byte aligned (LCB_ERR_INVALID otherwise); the other checks and limits are those of
+ * the unpacked calls.  Monomial coefficients with the shipped widths (signatures 11 / 13, keys 14 / 16, aggregates 12 / 14
+ * bits) and 16-byte aligned rows are read and written by the kernels directly; anything else is unpacked into scratch
+ * first.
+ * aggregate (bklm_one_time_agg_sigs.py:92-96): sig_packed uint8[agg_off[n_agg]][l][32*sig_bits] (bias sig_bias) ->
+ * ag_packed uint8[n_agg][l][32*ag_bits] (bias ag_bias) and in_range (nullable) uint8[n_agg][l], as lcb_pack_batch sets it. */
+int lcb_bklm_aggregate_packed_batch(lcb_ctx* ctx, const lcb_scheme* sch, const int64_t* agg_off, int64_t n_agg,
+                                    const uint8_t* sig_packed, int sig_bits, int sig_bias,
+                                    const uint8_t* agmsg, const int64_t* agmsg_off,
+                                    int ag_bits, int ag_bias, uint8_t* ag_packed, uint8_t* in_range);
+/* aggregate_verify (:99-116) from packed keys uint8[total][2][32*vk_bits] (bias 0) and packed aggregates
+ * uint8[n_agg][l][32*ag_bits] (bias ag_bias); verdict uint8[n_agg]. */
+int lcb_bklm_aggregate_verify_packed_batch(lcb_ctx* ctx, const lcb_scheme* sch, const int64_t* agg_off, int64_t n_agg,
+                                           const uint8_t* vk_packed, int vk_bits,
+                                           const uint8_t* chmsg_sorted, const int64_t* chmsg_off,
+                                           const uint8_t* agmsg, const int64_t* agmsg_off,
+                                           const uint8_t* ag_packed, int ag_bits, int ag_bias,
+                                           int ag_cap, int avf_bd, int avf_wt, uint8_t* verdict);
+
 /* adaptor make_one_wit / witgen (adaptor_sigs.py:80-101,140-151):
  *   wit_coef int16[n][l][d], st_ntt uint16[n][d], st_coef int16[n][d]; any may be NULL. */
 int lcb_adaptor_witgen_batch(lcb_ctx* ctx, const lcb_scheme* sch, const uint8_t* seeds, const int64_t* seed_off,
@@ -267,7 +290,8 @@ int64_t lcb_launch_count(const lcb_ctx* ctx);
 /* Optional per-kernel timing with CUDA events on the ctx stream (what bench.py's roofline reads).
  * kernel names: sampler shake256 ntt_fwd ntt_inv poly_mul matvec sign verify vec_addsub agg_coefs
  * agg_partial agg_finish aggv_partial aggv_finish pack unpack, and for the batch calls group_ids agg_coefs_seg
- * agg_partial_seg aggv_partial_seg aggv_residues aggv_limits.  lcb_profile_read synchronises the stream. */
+ * agg_partial_seg aggv_partial_seg aggv_residues aggv_limits, and agg_finish_pack for packed aggregates.
+ * lcb_profile_read synchronises the stream. */
 int lcb_profile_enable(lcb_ctx* ctx, int on);
 int lcb_profile_reset(lcb_ctx* ctx);
 int lcb_profile_read(lcb_ctx* ctx, const char* kernel, double* total_ms, int64_t* launches);

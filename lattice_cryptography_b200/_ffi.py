@@ -77,6 +77,10 @@ PROTOTYPES = {
     'lcb_bklm_aggregate_batch': (c_int, [c_void_p, POINTER(LcbScheme), _P, c_int64, _P, _P, _P, _P]),
     'lcb_bklm_aggregate_verify_batch': (c_int, [c_void_p, POINTER(LcbScheme), _P, c_int64, _P, _P, _P, _P, _P, _P, c_int,
                                                 c_int, c_int, _P]),
+    'lcb_bklm_aggregate_packed_batch': (c_int, [c_void_p, POINTER(LcbScheme), _P, c_int64, _P, c_int, c_int, _P, _P, c_int,
+                                                c_int, _P, _P]),
+    'lcb_bklm_aggregate_verify_packed_batch': (c_int, [c_void_p, POINTER(LcbScheme), _P, c_int64, _P, c_int, _P, _P, _P, _P,
+                                                       _P, c_int, c_int, c_int, c_int, c_int, _P]),
     'lcb_adaptor_witgen_batch': (c_int, [c_void_p, POINTER(LcbScheme), _P, _P, c_int64, _P, _P, _P]),
     'lcb_vec_add_batch': (c_int, [c_void_p, _P, _P, c_int64, _P]),
     'lcb_vec_sub_batch': (c_int, [c_void_p, _P, _P, c_int64, _P]),

@@ -80,12 +80,13 @@ constexpr int64_t kPipeChunk = 1 << 17;
 
 enum KernelId { K_SAMPLER = 0, K_SHAKE, K_NTT_FWD, K_NTT_INV, K_POLY_MUL, K_MATVEC, K_SIGN, K_VERIFY, K_ADDSUB,
                 K_AGG_COEFS, K_AGG_PARTIAL, K_AGG_FINISH, K_AGGV_PARTIAL, K_AGGV_FINISH, K_PACK, K_UNPACK, K_GROUP_IDS,
-                K_AGG_COEFS_SEG, K_AGG_PARTIAL_SEG, K_AGGV_PARTIAL_SEG, K_AGGV_RESIDUES, K_AGGV_LIMITS, K_COUNT };
+                K_AGG_COEFS_SEG, K_AGG_PARTIAL_SEG, K_AGGV_PARTIAL_SEG, K_AGGV_RESIDUES, K_AGGV_LIMITS, K_AGG_FINISH_PACK,
+                K_COUNT };
 const char* const kKernelNames[K_COUNT] = {"sampler", "shake256", "ntt_fwd", "ntt_inv", "poly_mul", "matvec", "sign",
                                            "verify", "vec_addsub", "agg_coefs", "agg_partial", "agg_finish",
                                            "aggv_partial", "aggv_finish", "pack", "unpack", "group_ids",
                                            "agg_coefs_seg", "agg_partial_seg", "aggv_partial_seg", "aggv_residues",
-                                           "aggv_limits"};
+                                           "aggv_limits", "agg_finish_pack"};
 static_assert(K_COUNT <= 24, "grow lcb_ctx::prof_ms / prof_n");
 
 // Launch wrapper: counts the launch and, when profiling is on, brackets it with CUDA events on the
@@ -478,6 +479,163 @@ int seg_coef_args(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* d_msg, int64
     a.out_pairs = d_pairs;
     return LCB_OK;
 }
+
+// The body of lcb_bklm_aggregate_batch over device buffers (go from group_offsets with all = !fast).  On the fast route
+// (d = 256, monomial coefficients) the signatures may also be packed rows (sig_bits 11 / 13, bias sig_bias) and the
+// aggregates may be written packed (ag_bits 1..16, bias ag_bias, in_range nullable); 0 bits = int16 arrays.
+int aggregate_batch_dev(lcb_ctx* c, const lcb_scheme* sch, Staging& sg, const GroupOffsets& go, int64_t n_agg,
+                        const void* d_sig, int sig_bits, int sig_bias, const uint8_t* d_msg, const int64_t* d_aoff,
+                        const int64_t* d_moff, void* d_out, int ag_bits, int ag_bias, uint8_t* d_range) {
+    const bool fast = !c->generic && sch->ag_wt == 1 && sch->ag_bd == 1;
+    if (!fast && (sig_bits || ag_bits)) return fail(c, LCB_ERR_INVALID, "packed aggregation needs monomial coefficients");
+    const int l = c->l;
+    const size_t D_ = (size_t)c->d * ew(c);
+    const size_t pair_len = (size_t)sch->ag_wt * 2 * ew(c);
+    int32_t* d_part;
+    CK(c, sg.alloc((void**)&d_part, (size_t)n_agg * l * D_ * sizeof(int32_t)));
+    CK(c, cudaMemsetAsync(d_part, 0, (size_t)n_agg * l * D_ * sizeof(int32_t), c->stream));
+    if (fast) {
+        int32_t* d_gid;
+        int16_t* d_pairs;
+        CK(c, sg.alloc((void**)&d_gid, (size_t)go.items * sizeof(int32_t)));
+        CK(c, sg.alloc((void**)&d_pairs, (size_t)go.items * pair_len * sizeof(int16_t)));
+        SamplerArgs a{};
+        int st = seg_coef_args(c, sch, d_msg, go.items, d_pairs, a);
+        if (st != LCB_OK) return st;
+        CK(c, timed(c, K_GROUP_IDS, [&] { return launch_group_ids(d_aoff, n_agg, go.items, d_gid, c->ring.num_sms, c->stream); }));
+        CK(c, timed(c, K_AGG_COEFS_SEG, [&] { return launch_agg_coefs_seg(a, d_gid, d_aoff, d_moff, n_agg, c->stream); }));
+        CK(c, timed(c, K_AGG_PARTIAL_SEG, [&] {
+            return launch_agg_partial_seg(c->ring, d_sig, sig_bits, sig_bias, d_pairs, d_gid, go.items, n_agg, d_part, c->stream);
+        }));
+        if (ag_bits) {
+            CK(c, timed(c, K_AGG_FINISH_PACK, [&] {
+                return launch_agg_finish_pack(c->ring, d_part, n_agg * l, ag_bits, ag_bias, static_cast<uint8_t*>(d_out), d_range,
+                                              c->stream);
+            }));
+        } else {
+            CK(c, timed(c, K_AGG_FINISH, [&] {
+                return launch_agg_finish_n(c->ring, d_part, n_agg * l * D, static_cast<int16_t*>(d_out), c->stream);
+            }));
+        }
+        return LCB_OK;
+    }
+    // generic geometry or non-monomial coefficients: the single-aggregate kernels, group by group (correct, not fast)
+    const bool monomial = sch->ag_wt == 1 && sch->ag_bd == 1;
+    const int16_t* sig = static_cast<const int16_t*>(d_sig);
+    int16_t* out = static_cast<int16_t*>(d_out);
+    int64_t most = 0;
+    for (int64_t g = 0; g < n_agg; ++g) most = std::max(most, go.agg[(size_t)g + 1] - go.agg[(size_t)g]);
+    int16_t* d_pairs;
+    CK(c, sg.alloc((void**)&d_pairs, (size_t)most * pair_len * sizeof(int16_t)));
+    for (int64_t g = 0; g < n_agg; ++g) {
+        const int64_t first = go.agg[(size_t)g], count = go.agg[(size_t)g + 1] - first;
+        const int16_t* sig_g = sig + (size_t)first * l * D_;
+        int32_t* part_g = d_part + (size_t)g * l * D_;
+        if (count > 0) {
+            int st = run_agg_coefs(c, sch, d_msg + go.msg[(size_t)g], go.msg[(size_t)g + 1] - go.msg[(size_t)g], 0, count, d_pairs);
+            if (st != LCB_OK) return st;
+            CK(c, timed(c, K_AGG_PARTIAL, [&] {
+                if (!monomial) return g_launch_agg_partial_poly(c->gen, sig_g, d_pairs, sch->ag_wt, count, part_g, c->stream);
+                return g_launch_agg_partial(c->gen, sig_g, d_pairs, count, part_g, c->stream);
+            }));
+        }
+        CK(c, timed(c, K_AGG_FINISH, [&] {
+            return c->generic ? g_launch_agg_finish(c->gen, part_g, out + (size_t)g * l * D_, c->stream)
+                              : launch_agg_finish(c->ring, part_g, out + (size_t)g * l * D_, c->stream);
+        }));
+    }
+    return LCB_OK;
+}
+
+// The body of lcb_bklm_aggregate_verify_batch over device buffers.  On the fast route the keys may also be 14-bit packed
+// rows (vk_bits 14; 0 = uint16 slots, which the 16-bit packing is byte for byte) and the aggregates 12- / 14-bit packed
+// rows with bias ag_bias (ag_bits 0 = int16).
+int aggregate_verify_batch_dev(lcb_ctx* c, const lcb_scheme* sch, Staging& sg, const GroupOffsets& go, int64_t n_agg,
+                               const void* d_vk, int vk_bits, const uint8_t* d_chmsg, const int64_t* d_choff,
+                               const uint8_t* d_msg, const int64_t* d_aoff, const int64_t* d_moff, const void* d_ag, int ag_bits,
+                               int ag_bias, int ag_cap, int avf_bd, int avf_wt, uint8_t* d_verdict) {
+    const bool fast = !c->generic && sch->ag_wt == 1 && sch->ag_bd == 1;
+    if (!fast && (vk_bits || ag_bits)) return fail(c, LCB_ERR_INVALID, "packed aggregate verification needs monomial coefficients");
+    const int l = c->l;
+    const size_t D_ = (size_t)c->d * ew(c);
+    const size_t pair_len = (size_t)sch->ag_wt * 2 * ew(c);
+    int16_t* d_ch;
+    int32_t* d_part;
+    CK(c, sg.alloc((void**)&d_ch, (size_t)go.items * sch->ch_wt * 2 * ew(c) * sizeof(int16_t)));
+    CK(c, sg.alloc((void**)&d_part, (size_t)n_agg * D_ * sizeof(int32_t)));
+    CK(c, cudaMemsetAsync(d_part, 0, (size_t)n_agg * D_ * sizeof(int32_t), c->stream));
+    int st;
+    if (go.items > 0) {           // the challenges of every item of every group: one sampler launch
+        st = run_challenge(c, sch, d_chmsg, d_choff, go.items, d_ch);
+        if (st != LCB_OK) return st;
+    }
+    if (fast) {
+        int32_t* d_gid;
+        int16_t* d_pairs;
+        uint16_t* d_rhs;
+        CK(c, sg.alloc((void**)&d_gid, (size_t)go.items * sizeof(int32_t)));
+        CK(c, sg.alloc((void**)&d_pairs, (size_t)go.items * pair_len * sizeof(int16_t)));
+        CK(c, sg.alloc((void**)&d_rhs, (size_t)n_agg * D * sizeof(uint16_t)));
+        SamplerArgs a{};
+        st = seg_coef_args(c, sch, d_msg, go.items, d_pairs, a);
+        if (st != LCB_OK) return st;
+        CK(c, timed(c, K_GROUP_IDS, [&] { return launch_group_ids(d_aoff, n_agg, go.items, d_gid, c->ring.num_sms, c->stream); }));
+        CK(c, timed(c, K_AGG_COEFS_SEG, [&] { return launch_agg_coefs_seg(a, d_gid, d_aoff, d_moff, n_agg, c->stream); }));
+        CK(c, timed(c, K_AGGV_PARTIAL_SEG, [&] {
+            return launch_aggv_partial_seg(c->ring, d_vk, vk_bits, d_ch, sch->ch_wt, d_pairs, d_gid, go.items, n_agg, d_part,
+                                           c->stream);
+        }));
+        CK(c, timed(c, K_AGGV_RESIDUES, [&] { return launch_aggv_residues(c->ring, d_part, n_agg * D, d_rhs, c->stream); }));
+        // bounds and key_ch * ag_sig == rhs: the witness-verify form of k_verify.  Every int16 passes a bound of 32768, as
+        // it passes any larger one in k_aggv_finish.
+        CK(c, timed(c, K_VERIFY, [&] {
+            if (ag_bits)
+                return launch_verify_rhs_packed(c->ring, static_cast<const uint8_t*>(d_ag), ag_bits, ag_bias, d_rhs, n_agg,
+                                                std::min(avf_bd, 32768), avf_wt, d_verdict, c->stream);
+            return launch_verify(c->ring, static_cast<const int16_t*>(d_ag), nullptr, nullptr, 0, d_rhs, nullptr, n_agg,
+                                 std::min(avf_bd, 32768), avf_wt, d_verdict, c->stream);
+        }));
+        CK(c, timed(c, K_AGGV_LIMITS, [&] {
+            if (ag_bits)
+                return launch_aggv_limits_packed(c->ring, d_aoff, n_agg, static_cast<const uint8_t*>(d_ag), ag_bits, ag_bias, ag_cap,
+                                                 d_verdict, c->stream);
+            return launch_aggv_limits(c->ring, d_aoff, n_agg, static_cast<const int16_t*>(d_ag), ag_cap, d_verdict, c->stream);
+        }));
+        return LCB_OK;
+    }
+    // generic geometry or non-monomial coefficients: the single-aggregate kernels, group by group (correct, not fast)
+    const bool monomial = sch->ag_wt == 1 && sch->ag_bd == 1;
+    const uint16_t* vk = static_cast<const uint16_t*>(d_vk);
+    const int16_t* ag = static_cast<const int16_t*>(d_ag);
+    int64_t most = 0;
+    for (int64_t g = 0; g < n_agg; ++g) most = std::max(most, go.agg[(size_t)g + 1] - go.agg[(size_t)g]);
+    int16_t* d_pairs;
+    CK(c, sg.alloc((void**)&d_pairs, (size_t)most * pair_len * sizeof(int16_t)));
+    for (int64_t g = 0; g < n_agg; ++g) {
+        const int64_t first = go.agg[(size_t)g], count = go.agg[(size_t)g + 1] - first;
+        int32_t* part_g = d_part + (size_t)g * D_;
+        const int16_t* ag_g = ag + (size_t)g * l * D_;
+        if (count > 0) {
+            const uint16_t* vk_g = vk + (size_t)first * 2 * D_;
+            const int16_t* ch_g = d_ch + (size_t)first * sch->ch_wt * 2 * ew(c);
+            st = run_agg_coefs(c, sch, d_msg + go.msg[(size_t)g], go.msg[(size_t)g + 1] - go.msg[(size_t)g], 0, count, d_pairs);
+            if (st != LCB_OK) return st;
+            CK(c, timed(c, K_AGGV_PARTIAL, [&] {
+                if (!monomial)
+                    return g_launch_aggv_partial_poly(c->gen, vk_g, ch_g, sch->ch_wt, d_pairs, sch->ag_wt, count, part_g, c->stream);
+                return g_launch_aggv_partial(c->gen, vk_g, ch_g, sch->ch_wt, d_pairs, count, part_g, c->stream);
+            }));
+        }
+        CK(c, timed(c, K_AGGV_FINISH, [&] {
+            return c->generic ? g_launch_aggv_finish(c->gen, part_g, ag_g, count, ag_cap, avf_bd, avf_wt, d_verdict + g, c->stream)
+                              : launch_aggv_finish(c->ring, part_g, ag_g, count, ag_cap, avf_bd, avf_wt, d_verdict + g, c->stream);
+        }));
+    }
+    return LCB_OK;
+}
+
+// Packed-buffer arguments shared by the packed aggregate calls: widths 1..16, biases 0..32767 (lcb_lm_verify_packed_batch)
+bool wire_args_ok(int bits, int bias) { return bits >= 1 && bits <= 16 && bias >= 0 && bias <= 32767; }
 
 }  // namespace
 
@@ -1438,59 +1596,18 @@ int lcb_bklm_aggregate_batch(lcb_ctx* c, const lcb_scheme* sch, const int64_t* a
     if (st != LCB_OK) return st;
     const int l = c->l;
     const size_t D_ = (size_t)c->d * ew(c);
-    const size_t pair_len = (size_t)sch->ag_wt * 2 * ew(c);
     Staging sg(c);
     const int16_t* d_sig;
     const uint8_t* d_msg;
     const int64_t *d_aoff, *d_moff;
     int16_t* d_out;
-    int32_t* d_part;
     CK(c, sg.in(&d_sig, sig_sorted, (size_t)go.items * l * D_));
     CK(c, sg.in(&d_msg, agmsg, (size_t)go.msg_bytes));
     CK(c, sg.in(&d_aoff, agg_off, (size_t)n_agg + 1));
     CK(c, sg.in(&d_moff, agmsg_off, (size_t)n_agg + 1));
     CK(c, sg.out(&d_out, ag_sig, (size_t)n_agg * l * D_));
-    CK(c, sg.alloc((void**)&d_part, (size_t)n_agg * l * D_ * sizeof(int32_t)));
-    CK(c, cudaMemsetAsync(d_part, 0, (size_t)n_agg * l * D_ * sizeof(int32_t), c->stream));
-    if (fast) {
-        int32_t* d_gid;
-        int16_t* d_pairs;
-        CK(c, sg.alloc((void**)&d_gid, (size_t)go.items * sizeof(int32_t)));
-        CK(c, sg.alloc((void**)&d_pairs, (size_t)go.items * pair_len * sizeof(int16_t)));
-        SamplerArgs a{};
-        st = seg_coef_args(c, sch, d_msg, go.items, d_pairs, a);
-        if (st != LCB_OK) return st;
-        CK(c, timed(c, K_GROUP_IDS, [&] { return launch_group_ids(d_aoff, n_agg, go.items, d_gid, c->ring.num_sms, c->stream); }));
-        CK(c, timed(c, K_AGG_COEFS_SEG, [&] { return launch_agg_coefs_seg(a, d_gid, d_aoff, d_moff, n_agg, c->stream); }));
-        CK(c, timed(c, K_AGG_PARTIAL_SEG, [&] {
-            return launch_agg_partial_seg(c->ring, d_sig, d_pairs, d_gid, go.items, n_agg, d_part, c->stream);
-        }));
-        CK(c, timed(c, K_AGG_FINISH, [&] { return launch_agg_finish_n(c->ring, d_part, n_agg * l * D, d_out, c->stream); }));
-    } else {
-        // generic geometry or non-monomial coefficients: the single-aggregate kernels, group by group (correct, not fast)
-        const bool monomial = sch->ag_wt == 1 && sch->ag_bd == 1;
-        int64_t most = 0;
-        for (int64_t g = 0; g < n_agg; ++g) most = std::max(most, go.agg[(size_t)g + 1] - go.agg[(size_t)g]);
-        int16_t* d_pairs;
-        CK(c, sg.alloc((void**)&d_pairs, (size_t)most * pair_len * sizeof(int16_t)));
-        for (int64_t g = 0; g < n_agg; ++g) {
-            const int64_t first = go.agg[(size_t)g], count = go.agg[(size_t)g + 1] - first;
-            const int16_t* sig_g = d_sig + (size_t)first * l * D_;
-            int32_t* part_g = d_part + (size_t)g * l * D_;
-            if (count > 0) {
-                st = run_agg_coefs(c, sch, d_msg + go.msg[(size_t)g], go.msg[(size_t)g + 1] - go.msg[(size_t)g], 0, count, d_pairs);
-                if (st != LCB_OK) return st;
-                CK(c, timed(c, K_AGG_PARTIAL, [&] {
-                    if (!monomial) return g_launch_agg_partial_poly(c->gen, sig_g, d_pairs, sch->ag_wt, count, part_g, c->stream);
-                    return g_launch_agg_partial(c->gen, sig_g, d_pairs, count, part_g, c->stream);
-                }));
-            }
-            CK(c, timed(c, K_AGG_FINISH, [&] {
-                return c->generic ? g_launch_agg_finish(c->gen, part_g, d_out + (size_t)g * l * D_, c->stream)
-                                  : launch_agg_finish(c->ring, part_g, d_out + (size_t)g * l * D_, c->stream);
-            }));
-        }
-    }
+    st = aggregate_batch_dev(c, sch, sg, go, n_agg, d_sig, 0, 0, d_msg, d_aoff, d_moff, d_out, 0, 0, nullptr);
+    if (st != LCB_OK) return st;
     CK(c, sg.finish());
     return LCB_OK;
 }
@@ -1521,15 +1638,12 @@ int lcb_bklm_aggregate_verify_batch(lcb_ctx* c, const lcb_scheme* sch, const int
     if (go.items > 0) CK(c, last_offset(c, chmsg_sorted, chmsg_off, go.items, &ch_bytes));
     const int l = c->l;
     const size_t D_ = (size_t)c->d * ew(c);
-    const size_t pair_len = (size_t)sch->ag_wt * 2 * ew(c);
     Staging sg(c);
     const uint16_t* d_vk;
     const uint8_t *d_chmsg, *d_msg;
     const int64_t *d_choff, *d_aoff, *d_moff;
     const int16_t* d_ag;
     uint8_t* d_verdict;
-    int16_t* d_ch;
-    int32_t* d_part;
     CK(c, sg.in(&d_vk, vk_ntt_sorted, (size_t)go.items * 2 * D_));
     CK(c, sg.in(&d_chmsg, chmsg_sorted, (size_t)ch_bytes));
     CK(c, sg.in(&d_choff, chmsg_off, (size_t)go.items + 1));
@@ -1538,64 +1652,129 @@ int lcb_bklm_aggregate_verify_batch(lcb_ctx* c, const lcb_scheme* sch, const int
     CK(c, sg.in(&d_moff, agmsg_off, (size_t)n_agg + 1));
     CK(c, sg.in(&d_ag, ag_sig, (size_t)n_agg * l * D_));
     CK(c, sg.out(&d_verdict, verdict, (size_t)n_agg));
-    CK(c, sg.alloc((void**)&d_ch, (size_t)go.items * sch->ch_wt * 2 * ew(c) * sizeof(int16_t)));
-    CK(c, sg.alloc((void**)&d_part, (size_t)n_agg * D_ * sizeof(int32_t)));
-    CK(c, cudaMemsetAsync(d_part, 0, (size_t)n_agg * D_ * sizeof(int32_t), c->stream));
-    if (go.items > 0) {           // the challenges of every item of every group: one sampler launch
-        st = run_challenge(c, sch, d_chmsg, d_choff, go.items, d_ch);
-        if (st != LCB_OK) return st;
-    }
-    if (fast) {
-        int32_t* d_gid;
-        int16_t* d_pairs;
-        uint16_t* d_rhs;
-        CK(c, sg.alloc((void**)&d_gid, (size_t)go.items * sizeof(int32_t)));
-        CK(c, sg.alloc((void**)&d_pairs, (size_t)go.items * pair_len * sizeof(int16_t)));
-        CK(c, sg.alloc((void**)&d_rhs, (size_t)n_agg * D * sizeof(uint16_t)));
-        SamplerArgs a{};
-        st = seg_coef_args(c, sch, d_msg, go.items, d_pairs, a);
-        if (st != LCB_OK) return st;
-        CK(c, timed(c, K_GROUP_IDS, [&] { return launch_group_ids(d_aoff, n_agg, go.items, d_gid, c->ring.num_sms, c->stream); }));
-        CK(c, timed(c, K_AGG_COEFS_SEG, [&] { return launch_agg_coefs_seg(a, d_gid, d_aoff, d_moff, n_agg, c->stream); }));
-        CK(c, timed(c, K_AGGV_PARTIAL_SEG, [&] {
-            return launch_aggv_partial_seg(c->ring, d_vk, d_ch, sch->ch_wt, d_pairs, d_gid, go.items, n_agg, d_part, c->stream);
-        }));
-        CK(c, timed(c, K_AGGV_RESIDUES, [&] { return launch_aggv_residues(c->ring, d_part, n_agg * D, d_rhs, c->stream); }));
-        // bounds and key_ch * ag_sig == rhs: the witness-verify form of k_verify.  Every int16 passes a bound of 32768, as
-        // it passes any larger one in k_aggv_finish.
-        CK(c, timed(c, K_VERIFY, [&] {
-            return launch_verify(c->ring, d_ag, nullptr, nullptr, 0, d_rhs, nullptr, n_agg, std::min(avf_bd, 32768), avf_wt,
-                                 d_verdict, c->stream);
-        }));
-        CK(c, timed(c, K_AGGV_LIMITS, [&] { return launch_aggv_limits(c->ring, d_aoff, n_agg, d_ag, ag_cap, d_verdict, c->stream); }));
+    st = aggregate_verify_batch_dev(c, sch, sg, go, n_agg, d_vk, 0, d_chmsg, d_choff, d_msg, d_aoff, d_moff, d_ag, 0, 0, ag_cap,
+                                    avf_bd, avf_wt, d_verdict);
+    if (st != LCB_OK) return st;
+    CK(c, sg.finish());
+    return LCB_OK;
+}
+
+// lcb_bklm_aggregate_batch on packed signatures, writing packed aggregates.  Fused route (monomial coefficients, 11- or
+// 13-bit signatures, 16-byte aligned signature rows): k_agg_partial_seg expands the packed rows itself and
+// k_agg_finish_pack writes the packed aggregates.  Anything else is unpacked into scratch first, aggregated by the code
+// of lcb_bklm_aggregate_batch and packed by k_pack.
+int lcb_bklm_aggregate_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const int64_t* agg_off, int64_t n_agg,
+                                    const uint8_t* sig_packed, int sig_bits, int sig_bias, const uint8_t* agmsg,
+                                    const int64_t* agmsg_off, int ag_bits, int ag_bias, uint8_t* ag_packed, uint8_t* in_range) {
+    LCB_RANGE();
+    if (!c || !sch || !agg_off || !agmsg_off || n_agg < 0 || (n_agg > 0 && (!sig_packed || !agmsg || !ag_packed)) ||
+        !wire_args_ok(sig_bits, sig_bias) || !wire_args_ok(ag_bits, ag_bias))
+        return LCB_ERR_INVALID;
+    if (c->generic) return fail(c, LCB_ERR_INVALID, "the packed wire format is defined for d == 256, q < 2^16 contexts only");
+    if (sch->ag_wt < 1 || sch->ag_wt > c->d || sch->ag_bd < 1) return fail(c, LCB_ERR_INVALID, "bad aggregation parameters");
+    if (n_agg > ((int64_t)1 << 30)) return fail(c, LCB_ERR_INVALID, "more than 2^30 aggregates in one call");
+    if (n_agg == 0) return LCB_OK;
+    CK(c, cudaSetDevice(c->device));
+    const bool monomial = sch->ag_wt == 1 && sch->ag_bd == 1;
+    GroupOffsets go;
+    int st = group_offsets(c, agg_off, agmsg_off, n_agg, true, !monomial, go);
+    if (st != LCB_OK) return st;
+    const int l = c->l;
+    Staging sg(c);
+    const uint8_t *d_sigp, *d_msg;
+    const int64_t *d_aoff, *d_moff;
+    uint8_t *d_agp, *d_range;
+    CK(c, sg.in(&d_sigp, sig_packed, (size_t)go.items * l * 32 * sig_bits));
+    CK(c, sg.in(&d_msg, agmsg, (size_t)go.msg_bytes));
+    CK(c, sg.in(&d_aoff, agg_off, (size_t)n_agg + 1));
+    CK(c, sg.in(&d_moff, agmsg_off, (size_t)n_agg + 1));
+    CK(c, sg.out(&d_agp, ag_packed, (size_t)n_agg * l * 32 * ag_bits));
+    CK(c, sg.out(&d_range, in_range, (size_t)n_agg * l));
+    if ((reinterpret_cast<uintptr_t>(d_sigp) | reinterpret_cast<uintptr_t>(d_agp)) & 3u)
+        return fail(c, LCB_ERR_INVALID, "packed buffers must be 4-byte aligned");
+    // the fused route reads signature rows with 16-byte loads: a caller-owned device buffer that is only 4-byte aligned
+    // takes the unpack-first route
+    if (monomial && (sig_bits == 11 || sig_bits == 13) && (reinterpret_cast<uintptr_t>(d_sigp) & 15u) == 0) {
+        st = aggregate_batch_dev(c, sch, sg, go, n_agg, d_sigp, sig_bits, sig_bias, d_msg, d_aoff, d_moff, d_agp, ag_bits,
+                                 ag_bias, d_range);
     } else {
-        // generic geometry or non-monomial coefficients: the single-aggregate kernels, group by group (correct, not fast)
-        const bool monomial = sch->ag_wt == 1 && sch->ag_bd == 1;
-        int64_t most = 0;
-        for (int64_t g = 0; g < n_agg; ++g) most = std::max(most, go.agg[(size_t)g + 1] - go.agg[(size_t)g]);
-        int16_t* d_pairs;
-        CK(c, sg.alloc((void**)&d_pairs, (size_t)most * pair_len * sizeof(int16_t)));
-        for (int64_t g = 0; g < n_agg; ++g) {
-            const int64_t first = go.agg[(size_t)g], count = go.agg[(size_t)g + 1] - first;
-            int32_t* part_g = d_part + (size_t)g * D_;
-            const int16_t* ag_g = d_ag + (size_t)g * l * D_;
-            if (count > 0) {
-                const uint16_t* vk_g = d_vk + (size_t)first * 2 * D_;
-                const int16_t* ch_g = d_ch + (size_t)first * sch->ch_wt * 2 * ew(c);
-                st = run_agg_coefs(c, sch, d_msg + go.msg[(size_t)g], go.msg[(size_t)g + 1] - go.msg[(size_t)g], 0, count, d_pairs);
-                if (st != LCB_OK) return st;
-                CK(c, timed(c, K_AGGV_PARTIAL, [&] {
-                    if (!monomial)
-                        return g_launch_aggv_partial_poly(c->gen, vk_g, ch_g, sch->ch_wt, d_pairs, sch->ag_wt, count, part_g, c->stream);
-                    return g_launch_aggv_partial(c->gen, vk_g, ch_g, sch->ch_wt, d_pairs, count, part_g, c->stream);
-                }));
-            }
-            CK(c, timed(c, K_AGGV_FINISH, [&] {
-                return c->generic ? g_launch_aggv_finish(c->gen, part_g, ag_g, count, ag_cap, avf_bd, avf_wt, d_verdict + g, c->stream)
-                                  : launch_aggv_finish(c->ring, part_g, ag_g, count, ag_cap, avf_bd, avf_wt, d_verdict + g, c->stream);
-            }));
-        }
+        int16_t *d_sig, *d_ag;
+        CK(c, sg.alloc((void**)&d_sig, (size_t)go.items * l * D * sizeof(int16_t)));
+        CK(c, sg.alloc((void**)&d_ag, (size_t)n_agg * l * D * sizeof(int16_t)));
+        CK(c, timed(c, K_UNPACK, [&] { return launch_unpack(c->ring, d_sigp, go.items * l, sig_bits, sig_bias, d_sig, c->stream); }));
+        st = aggregate_batch_dev(c, sch, sg, go, n_agg, d_sig, 0, 0, d_msg, d_aoff, d_moff, d_ag, 0, 0, nullptr);
+        if (st == LCB_OK)
+            CK(c, timed(c, K_PACK, [&] { return launch_pack(c->ring, d_ag, n_agg * l, ag_bits, ag_bias, d_agp, d_range, c->stream); }));
     }
+    if (st != LCB_OK) return st;
+    CK(c, sg.finish());
+    return LCB_OK;
+}
+
+// lcb_bklm_aggregate_verify_batch on packed keys and aggregates.  Fused route (monomial coefficients, 14- or 16-bit keys,
+// 12- or 14-bit aggregates, 16-byte aligned aggregate rows and 16-bit key rows): k_aggv_partial_seg reads the packed
+// keys, k_verify (witness form) and k_aggv_limits_packed the packed aggregates.  Anything else is unpacked into scratch
+// first and verified by the code of lcb_bklm_aggregate_verify_batch.
+int lcb_bklm_aggregate_verify_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const int64_t* agg_off, int64_t n_agg,
+                                           const uint8_t* vk_packed, int vk_bits, const uint8_t* chmsg_sorted,
+                                           const int64_t* chmsg_off, const uint8_t* agmsg, const int64_t* agmsg_off,
+                                           const uint8_t* ag_packed, int ag_bits, int ag_bias, int ag_cap, int avf_bd,
+                                           int avf_wt, uint8_t* verdict) {
+    LCB_RANGE();
+    if (!c || !sch || !agg_off || !agmsg_off || !chmsg_off || n_agg < 0 || (n_agg > 0 && (!agmsg || !ag_packed || !verdict)) ||
+        !wire_args_ok(vk_bits, 0) || !wire_args_ok(ag_bits, ag_bias))
+        return LCB_ERR_INVALID;
+    if (c->generic) return fail(c, LCB_ERR_INVALID, "the packed wire format is defined for d == 256, q < 2^16 contexts only");
+    if (sch->ag_wt < 1 || sch->ag_wt > c->d || sch->ag_bd < 1) return fail(c, LCB_ERR_INVALID, "bad aggregation parameters");
+    if (!c->has_key_ch) return fail(c, LCB_ERR_NO_KEY_CH, "lcb_bklm_aggregate_verify_packed_batch before lcb_set_key_ch");
+    if (n_agg > ((int64_t)1 << 30)) return fail(c, LCB_ERR_INVALID, "more than 2^30 aggregates in one call");
+    if (n_agg == 0) return LCB_OK;
+    CK(c, cudaSetDevice(c->device));
+    const bool monomial = sch->ag_wt == 1 && sch->ag_bd == 1;
+    GroupOffsets go;
+    int st = group_offsets(c, agg_off, agmsg_off, n_agg, false, !monomial, go);
+    if (st != LCB_OK) return st;
+    if (go.items > 0 && (!vk_packed || !chmsg_sorted)) return LCB_ERR_INVALID;
+    int64_t ch_bytes = 0;
+    std::vector<int64_t> unused;
+    if (go.items > 0 && !on_device(chmsg_off)) {
+        st = read_offsets(c, chmsg_off, go.items, false, false, &ch_bytes, unused, "chmsg_off");
+        if (st != LCB_OK) return st;
+    }
+    if (go.items > 0) CK(c, last_offset(c, chmsg_sorted, chmsg_off, go.items, &ch_bytes));
+    const int l = c->l;
+    Staging sg(c);
+    const uint8_t *d_vkp, *d_chmsg, *d_msg, *d_agp;
+    const int64_t *d_choff, *d_aoff, *d_moff;
+    uint8_t* d_verdict;
+    CK(c, sg.in(&d_vkp, vk_packed, (size_t)go.items * 2 * 32 * vk_bits));
+    CK(c, sg.in(&d_chmsg, chmsg_sorted, (size_t)ch_bytes));
+    CK(c, sg.in(&d_choff, chmsg_off, (size_t)go.items + 1));
+    CK(c, sg.in(&d_msg, agmsg, (size_t)go.msg_bytes));
+    CK(c, sg.in(&d_aoff, agg_off, (size_t)n_agg + 1));
+    CK(c, sg.in(&d_moff, agmsg_off, (size_t)n_agg + 1));
+    CK(c, sg.in(&d_agp, ag_packed, (size_t)n_agg * l * 32 * ag_bits));
+    CK(c, sg.out(&d_verdict, verdict, (size_t)n_agg));
+    if ((reinterpret_cast<uintptr_t>(d_vkp) | reinterpret_cast<uintptr_t>(d_agp)) & 3u)
+        return fail(c, LCB_ERR_INVALID, "packed buffers must be 4-byte aligned");
+    // the fused route stages aggregate rows with 16-byte cp.async and reads 16-bit key rows with 128-bit loads: a
+    // caller-owned device buffer that is only 4-byte aligned takes the unpack-first route
+    const bool aligned16 = (reinterpret_cast<uintptr_t>(d_agp) & 15u) == 0 &&
+                           (vk_bits == 14 || (reinterpret_cast<uintptr_t>(d_vkp) & 15u) == 0);
+    if (monomial && aligned16 && (vk_bits == 14 || vk_bits == 16) && (ag_bits == 12 || ag_bits == 14)) {
+        st = aggregate_verify_batch_dev(c, sch, sg, go, n_agg, d_vkp, vk_bits == 14 ? 14 : 0, d_chmsg, d_choff, d_msg, d_aoff,
+                                        d_moff, d_agp, ag_bits, ag_bias, ag_cap, avf_bd, avf_wt, d_verdict);
+    } else {
+        uint16_t* d_vk;
+        int16_t* d_ag;
+        CK(c, sg.alloc((void**)&d_vk, (size_t)go.items * 2 * D * sizeof(uint16_t)));
+        CK(c, sg.alloc((void**)&d_ag, (size_t)n_agg * l * D * sizeof(int16_t)));
+        CK(c, timed(c, K_UNPACK, [&] { return launch_unpack(c->ring, d_vkp, go.items * 2, vk_bits, 0, d_vk, c->stream); }));
+        CK(c, timed(c, K_UNPACK, [&] { return launch_unpack(c->ring, d_agp, n_agg * l, ag_bits, ag_bias, d_ag, c->stream); }));
+        st = aggregate_verify_batch_dev(c, sch, sg, go, n_agg, d_vk, 0, d_chmsg, d_choff, d_msg, d_aoff, d_moff, d_ag, 0, 0, ag_cap,
+                                        avf_bd, avf_wt, d_verdict);
+    }
+    if (st != LCB_OK) return st;
     CK(c, sg.finish());
     return LCB_OK;
 }

@@ -161,21 +161,30 @@ cudaError_t launch_aggv_finish(const RingCtx& c, const int32_t* partial, const i
                                int ag_cap, int avf_bd, int avf_wt, uint8_t* verdict, cudaStream_t st);
 // batches of aggregates (items sorted by group, gid from launch_group_ids): partial int32[n_agg][l][256] /
 // int32[n_agg][256], zeroed by the caller; k_agg_finish over nelem elements; residues of the verify partials in [0, q);
-// the lower limits k_verify does not check (1 <= count_g <= ag_cap, ag_sig != 0), ANDed into verdict
-cudaError_t launch_agg_partial_seg(const RingCtx& c, const int16_t* sigs, const int16_t* ag_pairs, const int32_t* gid,
-                                   int64_t total, int64_t n_agg, int32_t* partial, cudaStream_t st);
+// the lower limits k_verify does not check (1 <= count_g <= ag_cap, ag_sig != 0), ANDed into verdict.
+// Packed inputs (wire format): signatures sig_bits = 11 / 13 (0 = int16), keys vk_bits = 14 (0 = uint16, which is also
+// the 16-bit packing), aggregates 12 / 14 bits in the witness-verify form of k_verify; cudaErrorNotSupported otherwise
+cudaError_t launch_agg_partial_seg(const RingCtx& c, const void* sigs, int sig_bits, int sig_bias, const int16_t* ag_pairs,
+                                   const int32_t* gid, int64_t total, int64_t n_agg, int32_t* partial, cudaStream_t st);
 cudaError_t launch_agg_finish_n(const RingCtx& c, const int32_t* partial, int64_t nelem, int16_t* ag_sig, cudaStream_t st);
-cudaError_t launch_aggv_partial_seg(const RingCtx& c, const uint16_t* vk_ntt, const int16_t* ch_pairs, int ch_wt,
+cudaError_t launch_aggv_partial_seg(const RingCtx& c, const void* vk_ntt, int vk_bits, const int16_t* ch_pairs, int ch_wt,
                                     const int16_t* ag_pairs, const int32_t* gid, int64_t total, int64_t n_agg,
                                     int32_t* partial, cudaStream_t st);
 cudaError_t launch_aggv_residues(const RingCtx& c, const int32_t* partial, int64_t nelem, uint16_t* out, cudaStream_t st);
 cudaError_t launch_aggv_limits(const RingCtx& c, const int64_t* agg_off, int64_t n_agg, const int16_t* ag_sig, int64_t ag_cap,
                                uint8_t* verdict, cudaStream_t st);
+cudaError_t launch_aggv_limits_packed(const RingCtx& c, const int64_t* agg_off, int64_t n_agg, const uint8_t* ag_packed, int bits,
+                                      int bias, int64_t ag_cap, uint8_t* verdict, cudaStream_t st);
+cudaError_t launch_verify_rhs_packed(const RingCtx& c, const uint8_t* vec_packed, int bits, int bias, const uint16_t* rhs_only,
+                                     int64_t n, int bd, int wt, uint8_t* verdict, cudaStream_t st);
 
 // wire format (wire.cu): `bits`-bit little-endian packing of (x + bias) mod 2^16, 32*bits bytes per polynomial
 cudaError_t launch_pack(const RingCtx& c, const void* in, int64_t npoly, int bits, int bias, uint8_t* out,
                         uint8_t* in_range, cudaStream_t st);
 cudaError_t launch_unpack(const RingCtx& c, const uint8_t* in, int64_t npoly, int bits, int bias, void* out,
                           cudaStream_t st);
+// k_agg_finish + k_pack in one pass: BKLM partial sums int32[npoly][256] -> packed aggregates and in_range flags
+cudaError_t launch_agg_finish_pack(const RingCtx& c, const int32_t* partial, int64_t npoly, int bits, int bias, uint8_t* out,
+                                   uint8_t* in_range, cudaStream_t st);
 
 }  // namespace lcb

@@ -898,11 +898,16 @@ constexpr int SEG_REDUCE_ROWS = 1 << 15;
 // per group: lane 0 counts s per rotation k in the warp's own histogram, and a flush adds
 // corr[p] = sum over k > p of hist[k] (a warp suffix scan of the 256 counts) before it clears the histogram.
 // Three resident blocks (79 registers); at four the 64-register cap spills 48 bytes.
+// SIG_BITS = 0: int16 signatures.  SIG_BITS = 11 / 13: rows of the packed wire format (wire.cu; bias sig_bias), 22 / 26
+// of the 32 lanes fetch 16 bytes of a row; at parking time the raw row goes to the lower half of its E buffer and every
+// lane decodes its 8 values from there, so the fold below sees exactly the int16 row k_unpack would have made.
+template <int SIG_BITS>
 __global__ void __launch_bounds__(32 * AGG_WARPS, 3) k_agg_partial_seg(ModQ m, int l, const int16_t* __restrict__ sigs,
                                                                    const int16_t* __restrict__ ag_pairs,
                                                                    const int32_t* __restrict__ gid, int64_t total,
                                                                    int64_t n_agg, int64_t per_warp,
-                                                                   int32_t* __restrict__ partial) {
+                                                                   int32_t* __restrict__ partial, int sig_bias) {
+    constexpr int ROW_BYTES = SIG_BITS ? 32 * SIG_BITS : D * 2;
     __shared__ __align__(16) int32_t hist[AGG_WARPS][D];
     __shared__ __align__(16) int16_t rows[AGG_WARPS][AGG_DEPTH][2 * D];
     const int poly = blockIdx.y;
@@ -915,8 +920,8 @@ __global__ void __launch_bounds__(32 * AGG_WARPS, 3) k_agg_partial_seg(ModQ m, i
     int left = t_begin < t_end ? (int)(t_end - t_begin) : 0;
     const uint32_t* app = reinterpret_cast<const uint32_t*>(ag_pairs) + t_begin;
     const int32_t* gp = gid + t_begin;
-    const unsigned char* rowp = reinterpret_cast<const unsigned char*>(sigs + (t_begin * l + poly) * D) + 16 * lane;
-    const int64_t rstep = (int64_t)l * (D * 2);
+    const unsigned char* rowp = reinterpret_cast<const unsigned char*>(sigs) + (t_begin * l + poly) * ROW_BYTES + 16 * lane;
+    const int64_t rstep = (int64_t)l * ROW_BYTES;
     int32_t acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     uint4 v[AGG_DEPTH];
     uint32_t pr[AGG_DEPTH];
@@ -925,7 +930,8 @@ __global__ void __launch_bounds__(32 * AGG_WARPS, 3) k_agg_partial_seg(ModQ m, i
 #pragma unroll
         for (int j = 0; j < AGG_DEPTH; ++j)
             if (j < left) {
-                v[j] = __ldg(reinterpret_cast<const uint4*>(rowp + j * rstep));
+                if (SIG_BITS == 0 || 16 * lane < ROW_BYTES)
+                    v[j] = __ldg(reinterpret_cast<const uint4*>(rowp + j * rstep));
                 pr[j] = __ldg(app + j);
                 grp[j] = __ldg(gp + j);
             }
@@ -978,6 +984,29 @@ __global__ void __launch_bounds__(32 * AGG_WARPS, 3) k_agg_partial_seg(ModQ m, i
         uint32_t cur[AGG_DEPTH];
         int cg[AGG_DEPTH];
         __syncwarp();
+        if constexpr (SIG_BITS != 0) {
+            // value 8 lane + i sits at bit (8 lane + i) * SIG_BITS of the row; the word after the last one read lies
+            // inside the 1 KB E buffer and only contributes bits the mask drops
+#pragma unroll
+            for (int j = 0; j < AGG_DEPTH; ++j)
+                if (16 * lane < ROW_BYTES) reinterpret_cast<uint4*>(rows[warp][j])[lane] = v[j];
+            __syncwarp();
+#pragma unroll
+            for (int j = 0; j < AGG_DEPTH; ++j) {
+                const uint32_t* rw = reinterpret_cast<const uint32_t*>(rows[warp][j]);
+                uint32_t w[4];
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                    const int pos = (8 * lane + i) * SIG_BITS;
+                    const uint32_t f = __funnelshift_r(rw[pos >> 5], rw[(pos >> 5) + 1], pos & 31) & ((1u << SIG_BITS) - 1);
+                    const uint32_t x = (f - (uint32_t)sig_bias) & 0xFFFFu;
+                    if (i & 1) w[i >> 1] |= x << 16;
+                    else w[i >> 1] = x;
+                }
+                v[j] = make_uint4(w[0], w[1], w[2], w[3]);
+            }
+            __syncwarp();
+        }
 #pragma unroll
         for (int j = 0; j < AGG_DEPTH; ++j) {
             uint4* e = reinterpret_cast<uint4*>(rows[warp][j]);
@@ -1022,6 +1051,9 @@ __global__ void __launch_bounds__(32 * AGG_WARPS, 3) k_agg_partial_seg(ModQ m, i
 // and flushes per group.  Every half-warp runs the same number of trips (items past its range are dead, as the clamped
 // tail of k_aggv_partial) because the transform synchronises the whole warp.  A trip adds t * w < 2^18 * 2^16 to the
 // accumulator; reduce64 takes sums below 2^54, so a range holds at most 2^20 items (the launcher sizes the grid so).
+// VK_BITS = 0: uint16 key slots (also the 16-bit wire format, whose bytes are that array); VK_BITS = 14: keys in the
+// 14-bit wire format, 7 words per lane and key half, expanded as k_verify<..., 14> does.
+template <int VK_BITS>
 __global__ void __launch_bounds__(RBS, 4) k_aggv_partial_seg(ModQ m, StageConstF scf, const NttTables* __restrict__ tab,
                                                              const uint16_t* __restrict__ vk_ntt,
                                                              const int16_t* __restrict__ ch_pairs, int ch_wt,
@@ -1072,8 +1104,18 @@ __global__ void __launch_bounds__(RBS, 4) k_aggv_partial_seg(ModQ m, StageConstF
         const int64_t item = item_of(t);
         const uint32_t c0 = n_c0, c1 = n_c1, pr = n_pr;
         const int g = n_g;
-        const uint4* vkp = reinterpret_cast<const uint4*>(vk_ntt + item * 2 * D + 16 * h.lane);
-        const uint4 va = __ldg(vkp), vb = __ldg(vkp + 1), vc = __ldg(vkp + D / 8), vd = __ldg(vkp + D / 8 + 1);
+        uint4 va, vb, vc, vd;
+        if constexpr (VK_BITS == 14) {
+            LCB_CHECK(item >= 0 && item < total);
+            const uint32_t* vkp = reinterpret_cast<const uint32_t*>(vk_ntt) + item * (2 * 112) + 7 * h.lane;
+            va = make_uint4(__ldg(vkp), __ldg(vkp + 1), __ldg(vkp + 2), __ldg(vkp + 3));
+            vb = make_uint4(__ldg(vkp + 4), __ldg(vkp + 5), __ldg(vkp + 6), 0u);
+            vc = make_uint4(__ldg(vkp + 112), __ldg(vkp + 113), __ldg(vkp + 114), __ldg(vkp + 115));
+            vd = make_uint4(__ldg(vkp + 116), __ldg(vkp + 117), __ldg(vkp + 118), 0u);
+        } else {
+            const uint4* vkp = reinterpret_cast<const uint4*>(vk_ntt + item * 2 * D + 16 * h.lane);
+            va = __ldg(vkp), vb = __ldg(vkp + 1), vc = __ldg(vkp + D / 8), vd = __ldg(vkp + D / 8 + 1);
+        }
         if (t + 1 < t_begin + per_hw) prefetch(t + 1);
         uint32_t c[EPT];
         {
@@ -1103,8 +1145,14 @@ __global__ void __launch_bounds__(RBS, 4) k_aggv_partial_seg(ModQ m, StageConstF
         const uint32_t negoff = (int16_t)(pr >> 16) < 0 ? 256u : 0u;
 #pragma unroll
         for (int k = 0; k < EPT; ++k) {
-            const uint32_t vl = (k & 1) ? wl[k >> 1] >> 16 : wl[k >> 1] & 0xFFFFu;
-            const uint32_t vr = (k & 1) ? wr[k >> 1] >> 16 : wr[k >> 1] & 0xFFFFu;
+            uint32_t vl, vr;
+            if constexpr (VK_BITS == 14) {
+                vl = __funnelshift_r(wl[(14 * k) >> 5], wl[((14 * k) >> 5) + 1], (14 * k) & 31) & 0x3FFFu;
+                vr = __funnelshift_r(wr[(14 * k) >> 5], wr[((14 * k) >> 5) + 1], (14 * k) & 31) & 0x3FFFu;
+            } else {
+                vl = (k & 1) ? wl[k >> 1] >> 16 : wl[k >> 1] & 0xFFFFu;
+                vr = (k & 1) ? wr[k >> 1] >> 16 : wr[k >> 1] & 0xFFFFu;
+            }
             uint32_t ck = barrett_lazy(c[k] - FP_BIAS, m);                 // < 2q
             ck = min(ck, ck - m.q);                                       // < q: the product below stays under 2^32
             const uint32_t tt = barrett_lazy(ck * vl, m) + vr;            // < 2q + 2^16
@@ -1138,6 +1186,31 @@ __global__ void k_aggv_limits(const int64_t* __restrict__ agg_off, int64_t n_agg
             for (int64_t w = 0; w < words16 && !nz; ++w) {
                 const uint4 x = __ldg(p + w);
                 nz = (x.x | x.y | x.z | x.w) != 0;
+            }
+            ok = nz;
+        }
+        if (!ok) verdict[g] = 0;
+    }
+}
+
+// The same on packed aggregates (wire.cu layout, `bits` bits per coefficient, bias `bias`): a coefficient is non-zero
+// exactly where its field differs from the bias.  The test stops at the first such field.
+__global__ void k_aggv_limits_packed(const int64_t* __restrict__ agg_off, int64_t n_agg, const uint32_t* __restrict__ ag_packed,
+                                     int64_t fields, int bits, uint32_t bias, int64_t ag_cap, uint8_t* __restrict__ verdict) {
+    const int64_t words = fields * bits / 32;          // fields = l * 256: whole words
+    const uint32_t mask = (1u << bits) - 1;
+    for (int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; g < n_agg; g += (int64_t)gridDim.x * blockDim.x) {
+        if (!verdict[g]) continue;
+        const int64_t cnt = __ldg(agg_off + g + 1) - __ldg(agg_off + g);
+        bool ok = cnt >= 1 && cnt <= ag_cap;
+        if (ok) {
+            const uint32_t* p = ag_packed + g * words;
+            bool nz = false;
+            for (int64_t i = 0; i < fields && !nz; ++i) {
+                const int64_t pos = i * bits, w = pos >> 5;
+                LCB_CHECK(w < words);
+                const uint32_t hi = w + 1 < words ? __ldg(p + w + 1) : 0u;
+                nz = (__funnelshift_r(__ldg(p + w), hi, (unsigned)pos & 31u) & mask) != bias;
             }
             ok = nz;
         }
@@ -1304,6 +1377,18 @@ cudaError_t launch_verify_packed(const RingCtx& c, const uint8_t* sig_packed, in
     return cudaErrorNotSupported;
 }
 
+// Witness-verify form on packed rows of BKLM aggregates: the two widths of the shipped parameter sets (12 / 14 bits);
+// the decoder of k_verify is the one of the signature widths, and at even widths every value starts in the same
+// half-word phase.
+cudaError_t launch_verify_rhs_packed(const RingCtx& c, const uint8_t* vec_packed, int bits, int bias, const uint16_t* rhs_only,
+                                     int64_t n, int bd, int wt, uint8_t* verdict, cudaStream_t st) {
+    if (bits == 12)
+        return launch_verify_t<12, 0>(c, vec_packed, nullptr, nullptr, 0, rhs_only, nullptr, n, bd, wt, bias, verdict, st);
+    if (bits == 14)
+        return launch_verify_t<14, 0>(c, vec_packed, nullptr, nullptr, 0, rhs_only, nullptr, n, bd, wt, bias, verdict, st);
+    return cudaErrorNotSupported;
+}
+
 cudaError_t launch_vec_addsub(const RingCtx& c, const int16_t* a, const int16_t* b, int64_t nelem, int sub,
                               int16_t* out, cudaStream_t st) {
     if (nelem <= 0) return cudaSuccess;
@@ -1358,29 +1443,34 @@ cudaError_t launch_agg_finish_n(const RingCtx& c, const int32_t* partial, int64_
     return cudaSuccess;
 }
 
-cudaError_t launch_agg_partial_seg(const RingCtx& c, const int16_t* sigs, const int16_t* ag_pairs, const int32_t* gid,
-                                   int64_t total, int64_t n_agg, int32_t* partial, cudaStream_t st) {
+cudaError_t launch_agg_partial_seg(const RingCtx& c, const void* sigs, int sig_bits, int sig_bias, const int16_t* ag_pairs,
+                                   const int32_t* gid, int64_t total, int64_t n_agg, int32_t* partial, cudaStream_t st) {
     if (total <= 0) return cudaSuccess;
-    int64_t cap = (int64_t)c.num_sms * resident_blocks(k_agg_partial_seg, 32 * AGG_WARPS, 0) / c.l;
+    if (sig_bits != 0 && sig_bits != 11 && sig_bits != 13) return cudaErrorNotSupported;
+    auto kern = sig_bits == 11 ? k_agg_partial_seg<11> : sig_bits == 13 ? k_agg_partial_seg<13> : k_agg_partial_seg<0>;
+    int64_t cap = (int64_t)c.num_sms * resident_blocks(kern, 32 * AGG_WARPS, 0) / c.l;
     cap = max((int64_t)1, min(cap, (int64_t)SEG_MAX_WARPS / AGG_WARPS));
     const int64_t need = (total + AGG_WARPS * AGG_DEPTH - 1) / (AGG_WARPS * AGG_DEPTH);
     const int64_t chunks = min(need, cap);
     const int64_t per_warp = (total + chunks * AGG_WARPS - 1) / (chunks * AGG_WARPS);
     dim3 grid((unsigned)chunks, (unsigned)c.l);
-    k_agg_partial_seg<<<grid, 32 * AGG_WARPS, 0, st>>>(c.m, c.l, sigs, ag_pairs, gid, total, n_agg, per_warp, partial);
+    kern<<<grid, 32 * AGG_WARPS, 0, st>>>(c.m, c.l, static_cast<const int16_t*>(sigs), ag_pairs, gid, total, n_agg, per_warp,
+                                          partial, sig_bias);
     return cudaGetLastError();
 }
 
-cudaError_t launch_aggv_partial_seg(const RingCtx& c, const uint16_t* vk_ntt, const int16_t* ch_pairs, int ch_wt,
+cudaError_t launch_aggv_partial_seg(const RingCtx& c, const void* vk_ntt, int vk_bits, const int16_t* ch_pairs, int ch_wt,
                                     const int16_t* ag_pairs, const int32_t* gid, int64_t total, int64_t n_agg,
                                     int32_t* partial, cudaStream_t st) {
     if (total <= 0) return cudaSuccess;
-    int64_t blocks = (int64_t)persistent_grid(total, HWB, c.num_sms, resident_blocks(k_aggv_partial_seg, RBS, 0));
+    if (vk_bits != 0 && vk_bits != 14) return cudaErrorNotSupported;
+    auto kern = vk_bits == 14 ? k_aggv_partial_seg<14> : k_aggv_partial_seg<0>;
+    int64_t blocks = (int64_t)persistent_grid(total, HWB, c.num_sms, resident_blocks(kern, RBS, 0));
     blocks = min(blocks, (int64_t)SEG_MAX_WARPS / HWB);
     const int64_t per_hw = (total + blocks * HWB - 1) / (blocks * HWB);
     if (per_hw > ((int64_t)1 << 20)) return cudaErrorInvalidValue;      // reduce64 bound (see the kernel)
-    k_aggv_partial_seg<<<(unsigned)blocks, RBS, 0, st>>>(c.m, c.scf, c.tab, vk_ntt, ch_pairs, ch_wt, ag_pairs, gid, total,
-                                                         n_agg, per_hw, partial);
+    kern<<<(unsigned)blocks, RBS, 0, st>>>(c.m, c.scf, c.tab, static_cast<const uint16_t*>(vk_ntt), ch_pairs, ch_wt, ag_pairs,
+                                           gid, total, n_agg, per_hw, partial);
     return cudaGetLastError();
 }
 
@@ -1397,6 +1487,17 @@ cudaError_t launch_aggv_limits(const RingCtx& c, const int64_t* agg_off, int64_t
     const int64_t need = (n_agg + 255) / 256;
     k_aggv_limits<<<(unsigned)min(need, (int64_t)c.num_sms * 16), 256, 0, st>>>(agg_off, n_agg, ag_sig, (int64_t)c.l * D / 8,
                                                                                 ag_cap, verdict);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_aggv_limits_packed(const RingCtx& c, const int64_t* agg_off, int64_t n_agg, const uint8_t* ag_packed, int bits,
+                                      int bias, int64_t ag_cap, uint8_t* verdict, cudaStream_t st) {
+    if (n_agg <= 0) return cudaSuccess;
+    if (bits < 1 || bits > 16) return cudaErrorInvalidValue;
+    const int64_t need = (n_agg + 255) / 256;
+    k_aggv_limits_packed<<<(unsigned)min(need, (int64_t)c.num_sms * 16), 256, 0, st>>>(
+        agg_off, n_agg, reinterpret_cast<const uint32_t*>(ag_packed), (int64_t)c.l * D, bits, (uint32_t)bias & 0xFFFFu, ag_cap,
+        verdict);
     return cudaGetLastError();
 }
 

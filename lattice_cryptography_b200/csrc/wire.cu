@@ -54,6 +54,55 @@ __global__ void __launch_bounds__(WBS) k_pack(const uint16_t* __restrict__ in, i
     }
 }
 
+// The 8 values of a lane (value 8 lane + i of the polynomial, already biased, < 2^16) as `bits` whole bytes at byte
+// lane*bits of the warp's row; false if one of them needs more than `bits` bits
+__device__ __forceinline__ bool pack_lane(uint8_t* rowb, int lane, int bits, const uint32_t (&v)[8]) {
+    const uint32_t limit = 1u << bits;
+    uint64_t acc = 0;
+    int fill = 0, nb = 0;
+    bool ok = true;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+        ok = ok && v[i] < limit;
+        acc |= (uint64_t)(v[i] & (limit - 1)) << fill;
+        fill += bits;
+        while (fill >= 8) {
+            rowb[lane * bits + nb++] = (uint8_t)acc;
+            acc >>= 8;
+            fill -= 8;
+        }
+    }
+    return ok;
+}
+
+// BKLM aggregates straight into the wire format: k_agg_finish followed by k_pack, without the int16 aggregates making a
+// round trip through HBM.  partial int32[npoly][256] (|x| < 2^30) -> x mod q by Barrett reduction of x + off (off: a
+// multiple of q >= 2^30) -> centred -> (x + bias) mod 2^16 in `bits` bits, in_range[p] as k_pack sets it.
+__global__ void __launch_bounds__(WBS) k_agg_finish_pack(ModQ m, uint32_t off, const int32_t* __restrict__ partial,
+                                                         int64_t npoly, int bits, uint32_t bias, uint32_t* __restrict__ out,
+                                                         uint8_t* __restrict__ in_range) {
+    __shared__ uint32_t rows[WARPS][ROW_WORDS];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    uint32_t* row = rows[warp];
+    uint8_t* rowb = reinterpret_cast<uint8_t*>(row);
+    const int words = 8 * bits;
+    for (int64_t p = (int64_t)blockIdx.x * WARPS + warp; p < npoly; p += (int64_t)gridDim.x * WARPS) {
+        const int4* src = reinterpret_cast<const int4*>(partial + p * D) + 2 * lane;
+        const int4 a = __ldg(src), b = __ldg(src + 1);
+        const int x[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+        uint32_t v[8];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) v[i] = ((uint32_t)center(barrett_full((uint32_t)x[i] + off, m), m) + bias) & 0xFFFFu;
+        bool ok = pack_lane(rowb, lane, bits, v);
+        ok = __all_sync(0xFFFFFFFFu, ok);
+        __syncwarp();
+        uint32_t* o = out + p * words;
+        for (int k = lane; k < words; k += 32) o[k] = row[k];
+        if (in_range && lane == 0) in_range[p] = ok ? 1 : 0;
+        __syncwarp();
+    }
+}
+
 __global__ void __launch_bounds__(WBS) k_unpack(const uint32_t* __restrict__ in, int64_t npoly, int bits, uint32_t bias,
                                                 uint16_t* __restrict__ out) {
     __shared__ uint32_t rows[WARPS][ROW_WORDS];
@@ -95,6 +144,16 @@ cudaError_t launch_pack(const RingCtx& c, const void* in, int64_t npoly, int bit
     k_pack<<<wire_grid(npoly, c.num_sms), WBS, 0, st>>>(static_cast<const uint16_t*>(in), npoly, bits,
                                                          (uint32_t)bias & 0xFFFFu, reinterpret_cast<uint32_t*>(out),
                                                          in_range);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_agg_finish_pack(const RingCtx& c, const int32_t* partial, int64_t npoly, int bits, int bias, uint8_t* out,
+                                   uint8_t* in_range, cudaStream_t st) {
+    if (npoly <= 0) return cudaSuccess;
+    if (bits < 1 || bits > 16) return cudaErrorInvalidValue;
+    const uint32_t off = ((1u << 30) / c.m.q + 1) * c.m.q;
+    k_agg_finish_pack<<<wire_grid(npoly, c.num_sms), WBS, 0, st>>>(c.m, off, partial, npoly, bits, (uint32_t)bias & 0xFFFFu,
+                                                                    reinterpret_cast<uint32_t*>(out), in_range);
     return cudaGetLastError();
 }
 

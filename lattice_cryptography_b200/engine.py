@@ -431,6 +431,41 @@ class Engine(object):
                                                            _addr(ag_sig), ag_cap, avf_bd, avf_wt, _addr(verdict)))
         return verdict
 
+    def aggregate_packed_batch(self, sch: LcbScheme, agg_off, sig_packed, sig_bits: int, sig_bias: int, agmsgs,
+                               ag_bits: int, ag_bias: int, device: bool = False, want_range: bool = False):
+        """aggregate_batch on the packed wire format: sig_packed uint8[total, l, 32*sig_bits] -> ag_packed
+        uint8[n_agg, l, 32*ag_bits] (and in_range uint8[n_agg, l] when want_range), exactly pack(aggregate_batch(unpack))."""
+        total = int(sig_packed.shape[0]) if hasattr(sig_packed, 'shape') and len(sig_packed.shape) else 0
+        _want(sig_packed, 'sig_packed', np.uint8, (total, self.l, self.d * sig_bits // 8))
+        n_agg = self._groups(agg_off, total)
+        mblob, moff = self._rag(agmsgs)
+        if self._count(moff) != n_agg:
+            raise ValueError(f'{self._count(moff)} aggregation messages for {n_agg} aggregates')
+        out = self._out((n_agg, self.l, self.d * ag_bits // 8), np.uint8, device)
+        ok = self._out((n_agg, self.l), np.uint8, device) if want_range else None
+        self._ck(self._lib.lcb_bklm_aggregate_packed_batch(self._ctx, byref(sch), _addr(agg_off), n_agg, _addr(sig_packed),
+                                                           sig_bits, sig_bias, _addr(mblob), _addr(moff), ag_bits, ag_bias,
+                                                           _addr(out), _addr(ok)))
+        return (out, ok) if want_range else out
+
+    def aggregate_verify_packed_batch(self, sch: LcbScheme, agg_off, vk_packed, vk_bits: int, chmsgs_sorted, agmsgs,
+                                      ag_packed, ag_bits: int, ag_bias: int, ag_cap: int, avf_bd: int, avf_wt: int,
+                                      device: bool = False):
+        """aggregate_verify_batch from packed keys uint8[total, 2, 32*vk_bits] and aggregates uint8[n_agg, l, 32*ag_bits]."""
+        cblob, coff = self._rag(chmsgs_sorted)
+        total = self._count(coff)
+        _want(vk_packed, 'vk_packed', np.uint8, (total, 2, self.d * vk_bits // 8))
+        n_agg = self._groups(agg_off, total)
+        _want(ag_packed, 'ag_packed', np.uint8, (n_agg, self.l, self.d * ag_bits // 8))
+        mblob, moff = self._rag(agmsgs)
+        if self._count(moff) != n_agg:
+            raise ValueError(f'{self._count(moff)} aggregation messages for {n_agg} aggregates')
+        verdict = self._out((n_agg,), np.uint8, device)
+        self._ck(self._lib.lcb_bklm_aggregate_verify_packed_batch(
+            self._ctx, byref(sch), _addr(agg_off), n_agg, _addr(vk_packed), vk_bits, _addr(cblob), _addr(coff), _addr(mblob),
+            _addr(moff), _addr(ag_packed), ag_bits, ag_bias, ag_cap, avf_bd, avf_wt, _addr(verdict)))
+        return verdict
+
     # ------------------------------------------------------------------ adaptor signatures
     def witgen(self, sch: LcbScheme, seeds, want_wit: bool = True, want_st_ntt: bool = True,
                want_st_coef: bool = True, device: bool = False):

@@ -9,6 +9,11 @@ module is therefore OPT-IN and does not change what the drop-in API computes:
   13 at 256) instead of 16 - 4,576 / 9,568 bytes per signature instead of 6,656 / 11,776;
 * `pack_keys` / `unpack_keys`: NTT-form verification keys in `key_bits(pp)` bits (14 / 16);
 * `verify_batch_packed`: `lm_one_time_sigs.verify_batch` straight from the packed records;
+* `aggregate_batch_packed` / `aggregate_verify_batch_packed`: the batched BKLM calls of `bklm_one_time_agg_sigs`
+  (many independent aggregates, sorted signatures / keys of group g at agg_off[g] .. agg_off[g+1]) from packed
+  signatures and keys, with packed aggregates.  An aggregate is encoded as a signature with the aggregate bound:
+  `pack_signatures(pp, ag, bound_key='avf_bd')`, `sig_bits(pp, 'avf_bd')` bits (12 at secpar 128, 14 at 256), bias
+  `avf_bd`;
 * `setup_parameters_from_seed`: `make_setup_parameters` with `key_ch = H2PV('KEY_CH_SALT' || seed)` sampled on
   the GPU with the reference's own distribution parameters (bd = q//2, wt = d), so that two parties derive
   the same row from a short public string.
@@ -69,6 +74,26 @@ def verify_batch_packed(pp, vk_packed, chmsgs, sig_packed, device: bool = False)
     eng, sch = _ctx(pp)
     return eng.lm_verify_packed(sch, vk_packed, key_bits(pp), chmsgs, sig_packed, sig_bits(pp), pp['vf_bd'],
                                 pp['vf_bd'], pp['vf_wt'], device=device)
+
+
+def aggregate_batch_packed(pp, agg_off, sig_packed, agmsgs, device: bool = False):
+    """Aggregates of many groups from packed sorted signatures uint8[total, l, 32*sig_bits] (agmsgs[g]: the aggregation
+    message of group g, committed first in tree mode as `bklm_one_time_agg_sigs.aggregate_batch` does) ->
+    (ag_packed uint8[n_agg, l, 32*sig_bits(pp, 'avf_bd')], in_range uint8[n_agg, l])."""
+    from .bklm_one_time_agg_sigs import _batch_messages, _ctx
+    eng, sch = _ctx(pp)
+    return eng.aggregate_packed_batch(sch, agg_off, sig_packed, sig_bits(pp), pp['vf_bd'], _batch_messages(pp, list(agmsgs)),
+                                      sig_bits(pp, 'avf_bd'), pp['avf_bd'], device=device, want_range=True)
+
+
+def aggregate_verify_batch_packed(pp, agg_off, vk_packed, chmsgs_sorted, agmsgs, ag_packed, device: bool = False):
+    """uint8[n_agg] verdicts of many aggregates from packed sorted keys uint8[total, 2, 32*key_bits] and packed aggregates
+    uint8[n_agg, l, 32*sig_bits(pp, 'avf_bd')]; an empty group or one above ag_cap verifies as 0."""
+    from .bklm_one_time_agg_sigs import _batch_messages, _ctx
+    eng, sch = _ctx(pp)
+    return eng.aggregate_verify_packed_batch(sch, agg_off, vk_packed, key_bits(pp), chmsgs_sorted,
+                                             _batch_messages(pp, list(agmsgs)), ag_packed, sig_bits(pp, 'avf_bd'),
+                                             pp['avf_bd'], pp['ag_cap'], pp['avf_bd'], pp['avf_wt'], device=device)
 
 
 def key_ch_from_seed(lp, secpar: int, seed: str) -> PolynomialVector:
