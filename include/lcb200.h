@@ -232,7 +232,8 @@ int lcb_bklm_aggregate_packed_batch(lcb_ctx* ctx, const lcb_scheme* sch, const i
                                     const uint8_t* agmsg, const int64_t* agmsg_off,
                                     int ag_bits, int ag_bias, uint8_t* ag_packed, uint8_t* in_range);
 /* aggregate_verify (:99-116) from packed keys uint8[total][2][32*vk_bits] (bias 0) and packed aggregates
- * uint8[n_agg][l][32*ag_bits] (bias ag_bias); verdict uint8[n_agg]. */
+ * uint8[n_agg][l][32*ag_bits] (bias ag_bias); verdict uint8[n_agg].  A key slot v >= q (possible at 14 and 16 bits) acts
+ * as v mod q, here and in lcb_bklm_aggregate_verify_batch. */
 int lcb_bklm_aggregate_verify_packed_batch(lcb_ctx* ctx, const lcb_scheme* sch, const int64_t* agg_off, int64_t n_agg,
                                            const uint8_t* vk_packed, int vk_bits,
                                            const uint8_t* chmsg_sorted, const int64_t* chmsg_off,

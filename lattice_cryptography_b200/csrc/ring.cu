@@ -14,6 +14,8 @@
 // for the life of the kernel; accumulation of the row-vector product is 64-bit (IMAD.WIDE) with a
 // single reduction per output coefficient.  Grids are persistent: (#SM x resident blocks) blocks
 // striding over the batch.
+#include <cstdlib>
+
 #include "engine.h"
 
 namespace lcb {
@@ -1443,6 +1445,17 @@ cudaError_t launch_agg_finish_n(const RingCtx& c, const int32_t* partial, int64_
     return cudaSuccess;
 }
 
+// Test knob LCB_SEG_RANGES: an upper limit on the ranges (warps / half-warps) per polynomial of the segmented kernels, so
+// that tests reach long ranges - in-register reductions, many flushes per range - without gigabytes of input.  It can
+// only lower the computed count; values below 1 are ignored.
+static int64_t seg_ranges(int64_t ranges) {
+    if (const char* env = getenv("LCB_SEG_RANGES")) {
+        const int64_t v = atoll(env);
+        if (v >= 1 && v < ranges) return v;
+    }
+    return ranges;
+}
+
 cudaError_t launch_agg_partial_seg(const RingCtx& c, const void* sigs, int sig_bits, int sig_bias, const int16_t* ag_pairs,
                                    const int32_t* gid, int64_t total, int64_t n_agg, int32_t* partial, cudaStream_t st) {
     if (total <= 0) return cudaSuccess;
@@ -1451,8 +1464,9 @@ cudaError_t launch_agg_partial_seg(const RingCtx& c, const void* sigs, int sig_b
     int64_t cap = (int64_t)c.num_sms * resident_blocks(kern, 32 * AGG_WARPS, 0) / c.l;
     cap = max((int64_t)1, min(cap, (int64_t)SEG_MAX_WARPS / AGG_WARPS));
     const int64_t need = (total + AGG_WARPS * AGG_DEPTH - 1) / (AGG_WARPS * AGG_DEPTH);
-    const int64_t chunks = min(need, cap);
-    const int64_t per_warp = (total + chunks * AGG_WARPS - 1) / (chunks * AGG_WARPS);
+    const int64_t ranges = seg_ranges(min(need, cap) * AGG_WARPS);      // warps past the last range find nothing to do
+    const int64_t chunks = (ranges + AGG_WARPS - 1) / AGG_WARPS;
+    const int64_t per_warp = (total + ranges - 1) / ranges;
     dim3 grid((unsigned)chunks, (unsigned)c.l);
     kern<<<grid, 32 * AGG_WARPS, 0, st>>>(c.m, c.l, static_cast<const int16_t*>(sigs), ag_pairs, gid, total, n_agg, per_warp,
                                           partial, sig_bias);
@@ -1466,8 +1480,9 @@ cudaError_t launch_aggv_partial_seg(const RingCtx& c, const void* vk_ntt, int vk
     if (vk_bits != 0 && vk_bits != 14) return cudaErrorNotSupported;
     auto kern = vk_bits == 14 ? k_aggv_partial_seg<14> : k_aggv_partial_seg<0>;
     int64_t blocks = (int64_t)persistent_grid(total, HWB, c.num_sms, resident_blocks(kern, RBS, 0));
-    blocks = min(blocks, (int64_t)SEG_MAX_WARPS / HWB);
-    const int64_t per_hw = (total + blocks * HWB - 1) / (blocks * HWB);
+    const int64_t ranges = seg_ranges(min(blocks, (int64_t)SEG_MAX_WARPS / HWB) * HWB);   // half-warps past the last range
+    blocks = (ranges + HWB - 1) / HWB;                                                  // run dead trips only
+    const int64_t per_hw = (total + ranges - 1) / ranges;
     if (per_hw > ((int64_t)1 << 20)) return cudaErrorInvalidValue;      // reduce64 bound (see the kernel)
     kern<<<(unsigned)blocks, RBS, 0, st>>>(c.m, c.scf, c.tab, static_cast<const uint16_t*>(vk_ntt), ch_pairs, ch_wt, ag_pairs,
                                            gid, total, n_agg, per_hw, partial);

@@ -179,3 +179,50 @@ def test_host_buffers_pipeline_over_several_chunks(engines):
     e.synchronize()
     sig_p, vk_p = sig_p.cpu().numpy(), vk_p.cpu().numpy()
     assert np.array_equal(e.lm_verify_packed(sch, vk_p, 14, h_msgs, sig_p, 11, 945, 945, 256), want)
+
+
+@pytest.mark.parametrize('secpar', [128, 256])
+def test_verify_packed_weight_below_d(engines, secpar):
+    """vf_wt < 256 selects the weight-checking k_verify<true, 11, 14> / <true, 13, 0> on the fused packed route.  The
+    signatures are built so that the equation holds (vk_right := key_ch * sig - vk_left * c), with one row of weight exactly
+    wt or wt + 1: the verdicts must equal the numpy rule max|sig| <= bd and every row weight <= wt."""
+    from lattice_cryptography_b200 import Engine
+    s = SHIPPED[secpar]
+    q, l = s['q'], s['l']
+    sch = scheme(secpar)
+    rng = np.random.default_rng(secpar + 1)
+    e = Engine(secpar, q, D, l)
+    try:
+        key_ch = rng.integers(-(q // 2), q // 2 + 1, (l, D)).astype(np.int16)
+        e.set_key_ch(key_ch)
+        sb, kb, bd = (11, 14, 945) if secpar == 128 else (13, 16, 3315)
+        for wt in (1, 10, 255):
+            sigs, want = [], []
+            for extra in (0, 1, 0, 1):
+                row = int(rng.integers(0, l))
+                z = np.zeros((l, D), np.int16)
+                for i in range(l):
+                    wi = wt + extra if i == row else int(rng.integers(1, wt + 1))
+                    z[i, rng.choice(D, wi, replace=False)] = rng.choice(np.array([-bd, -1, 1, bd], np.int16), wi)
+                sigs.append(z)
+                want.append(1 - extra)
+            sig = np.ascontiguousarray(np.stack(sigs))
+            n = len(sigs)
+            msgs = [f'weight {wt} {i}'.encode() for i in range(n)]
+            pairs = e.challenge(sch, msgs)
+            c = np.zeros((n, D), np.int16)
+            for i in range(n):
+                c[i, pairs[i, :, 0].astype(np.int64)] = pairs[i, :, 1]
+            lhs = sum(e.poly_mul(np.ascontiguousarray(np.broadcast_to(key_ch[j], (n, D))), np.ascontiguousarray(sig[:, j]))
+                      .astype(np.int64) for j in range(l))
+            vkl = rng.integers(-(q // 2), q // 2 + 1, (n, D)).astype(np.int16)
+            vkr = (lhs - e.poly_mul(vkl, c).astype(np.int64)) % q
+            vkr = np.where(vkr > q // 2, vkr - q, vkr).astype(np.int16)
+            vk = np.ascontiguousarray(np.stack([e.ntt_fwd(vkl), e.ntt_fwd(vkr)], axis=1))
+            rule = [int((np.abs(x.astype(np.int64)).max() <= bd) and (x != 0).sum(axis=1).max() <= wt) for x in sigs]
+            assert rule == want
+            assert e.lm_verify(sch, vk, msgs, sig, bd, wt).tolist() == want, wt
+            got = e.lm_verify_packed(sch, e.pack(vk, kb, 0), kb, msgs, e.pack(sig, sb, bd), sb, bd, bd, wt)
+            assert got.tolist() == want, wt
+    finally:
+        e.close()
