@@ -163,6 +163,45 @@ int lcb_lm_verify_packed_batch(lcb_ctx* ctx, const lcb_scheme* sch, const uint8_
                                const uint8_t* chmsg, const int64_t* chmsg_off, const uint8_t* sig_packed,
                                int sig_bits, int sig_bias, int64_t n, int bd, int wt, uint8_t* verdict);
 
+/* ---- The other records that leave a signer, on the packed wire format.  Same rules as the packed calls above: bits
+ * 1..16, biases 0..32767, packed buffers 4-byte aligned (LCB_ERR_INVALID otherwise); d == 256, q < 2^16 contexts only
+ * (LCB_ERR_INVALID, "the packed wire format is defined for d == 256, q < 2^16 contexts only"); host or device buffers
+ * with the usual synchronisation rules.  Each result is exactly that of the composition named, for any input bytes.
+ * Shipped packings: presignatures in ceil(log2(2 pvf_bd + 1)) bits with bias pvf_bd (11 / 13 bits), adaptor signatures
+ * with vf_bd (11 / 13), statements like keys (14 / 16 bits, bias 0).  Signatures made from genuine keys lie within
+ * sk_bd (1 + ch_wt) = vf_bd, so their in_range flags are 1. */
+
+/* sign (lm_one_time_sigs.py:163-170) / adaptor presign (adaptor_sigs.py:191-195) into packed rows:
+ * sig_packed uint8[n][l][32*sig_bits] (bias sig_bias), in_range (nullable) uint8[n][l].
+ * Exactly lcb_lm_sign_batch -> lcb_pack_batch(sig_bits, sig_bias), for any sk_ntt values.  11- and 13-bit rows in
+ * 16-byte aligned buffers are written by the sign kernel itself; other widths sign into engine scratch and pack. */
+int lcb_lm_sign_packed_batch(lcb_ctx* ctx, const lcb_scheme* sch, const uint16_t* sk_ntt, const uint8_t* chmsg,
+                             const int64_t* chmsg_off, int64_t n, int sig_bits, int sig_bias,
+                             uint8_t* sig_packed, uint8_t* in_range);
+
+/* adaptor verify (adaptor_sigs.py:247-266) from packed keys (bias 0), signatures (bias sig_bias) and statements
+ * st_packed uint8[n][32*st_bits] (NTT form, bias 0, packed like a key half).  Exactly unpack all three ->
+ * lcb_lm_verify_batch(st_ntt = the unpacked statements).  st_packed must not be NULL (preverify is
+ * lcb_lm_verify_packed_batch with bd = pvf_bd).  At most 2^30 items.  The shipped widths with st_bits == vk_bits are
+ * read by the verify kernel directly (16-bit key and statement rows from 16-byte aligned buffers); anything else is
+ * unpacked into engine scratch first. */
+int lcb_adaptor_verify_packed_batch(lcb_ctx* ctx, const lcb_scheme* sch, const uint8_t* vk_packed, int vk_bits,
+                                    const uint8_t* chmsg, const int64_t* chmsg_off, const uint8_t* sig_packed,
+                                    int sig_bits, int sig_bias, const uint8_t* st_packed, int st_bits,
+                                    int64_t n, int bd, int wt, uint8_t* verdict);
+
+/* adapt (adaptor_sigs.py:220-221): exactly unpack(presig) -> lcb_vec_add_batch(presig, wit) -> lcb_pack_batch.
+ * presig_packed uint8[npoly][32*presig_bits], wit_coef int16[npoly][d], sig_packed uint8[npoly][32*sig_bits],
+ * in_range (nullable) uint8[npoly]. */
+int lcb_adaptor_adapt_packed_batch(lcb_ctx* ctx, const uint8_t* presig_packed, int presig_bits, int presig_bias,
+                                   const int16_t* wit_coef, int64_t npoly, int sig_bits, int sig_bias,
+                                   uint8_t* sig_packed, uint8_t* in_range);
+
+/* extract (adaptor_sigs.py:224-226): exactly unpack both -> lcb_vec_sub_batch(sig, presig); wit_coef int16[npoly][d]. */
+int lcb_adaptor_extract_packed_batch(lcb_ctx* ctx, const uint8_t* sig_packed, int sig_bits, int sig_bias,
+                                     const uint8_t* presig_packed, int presig_bits, int presig_bias, int64_t npoly,
+                                     int16_t* wit_coef);
+
 /* make_agg_coefs (bklm_one_time_agg_sigs.py:78-81): coefficient i = H2P(ag_salt+str(first+i) || agmsg),
  * out_pairs int16[count][ag_wt][2].  ag_wt = ag_bd = 1 (the shipped tables: signed monomials) takes the dedicated
  * shared-message kernels; any other 1 <= ag_wt <= d, ag_bd >= 1 runs the full sampler per coefficient. */
@@ -291,7 +330,8 @@ int64_t lcb_launch_count(const lcb_ctx* ctx);
 /* Optional per-kernel timing with CUDA events on the ctx stream (what bench.py's roofline reads).
  * kernel names: sampler shake256 ntt_fwd ntt_inv poly_mul matvec sign verify vec_addsub agg_coefs
  * agg_partial agg_finish aggv_partial aggv_finish pack unpack, and for the batch calls group_ids agg_coefs_seg
- * agg_partial_seg aggv_partial_seg aggv_residues aggv_limits, and agg_finish_pack for packed aggregates.
+ * agg_partial_seg aggv_partial_seg aggv_residues aggv_limits, and agg_finish_pack for packed aggregates.  The fused packed
+ * routes are counted under the kernel they extend: packed signing under sign, packed verification under verify.
  * lcb_profile_read synchronises the stream. */
 int lcb_profile_enable(lcb_ctx* ctx, int on);
 int lcb_profile_reset(lcb_ctx* ctx);

@@ -1349,18 +1349,22 @@ int lcb_unpack_batch(lcb_ctx* c, const uint8_t* packed, int64_t npoly, int bits,
     return LCB_OK;
 }
 
-// lcb_lm_verify_batch on packed verification keys and signatures.  The batch is processed in chunks of 2^18:
-// challenge sampler -> k_verify reading the packed rows directly (the shipped 11/14- and 13/16-bit packings), or
-// unpack -> challenge sampler -> k_verify for any other width (unpacked copies bounded to ~2 GB of scratch).
-int lcb_lm_verify_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* vk_packed, int vk_bits,
-                               const uint8_t* chmsg, const int64_t* chmsg_off, const uint8_t* sig_packed, int sig_bits,
-                               int sig_bias, int64_t n, int bd, int wt, uint8_t* verdict) {
-    LCB_RANGE();
-    if (!c || !sch || !vk_packed || !chmsg_off || !sig_packed || !verdict || n < 0 || bd < 0 || wt < 0 ||
-        vk_bits < 1 || vk_bits > 16 || sig_bits < 1 || sig_bits > 16 || sig_bias < 0 || sig_bias > 32767)
-        return LCB_ERR_INVALID;
+}  // extern "C"
+
+namespace {
+
+// lcb_lm_verify_batch on packed verification keys and signatures, and on packed statements when st_packed is set
+// (adaptor verify: the statement is added to the right-hand side, as st_ntt is).  The batch is processed in chunks of
+// 2^18: challenge sampler -> k_verify reading the packed rows directly (the shipped 11/14- and 13/16-bit packings, with
+// statements at the key width), or unpack -> challenge sampler -> k_verify for any other width (unpacked copies
+// bounded to ~2 GB of scratch).  The caller has checked the arguments.
+int verify_packed(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* vk_packed, int vk_bits, const uint8_t* chmsg,
+                  const int64_t* chmsg_off, const uint8_t* sig_packed, int sig_bits, int sig_bias, const uint8_t* st_packed,
+                  int st_bits, int64_t n, int bd, int wt, uint8_t* verdict) {
     if (c->generic) return fail(c, LCB_ERR_INVALID, "the packed wire format is defined for d == 256, q < 2^16 contexts only");
-    if (!c->has_key_ch) return fail(c, LCB_ERR_NO_KEY_CH, "lcb_lm_verify_packed_batch before lcb_set_key_ch");
+    if (!c->has_key_ch)
+        return fail(c, LCB_ERR_NO_KEY_CH, std::string(st_packed ? "lcb_adaptor_verify_packed_batch" : "lcb_lm_verify_packed_batch") +
+                                              " before lcb_set_key_ch");
     if (n > ((int64_t)1 << 30)) return fail(c, LCB_ERR_INVALID, "more than 2^30 items in one verify call");
     if (n == 0) return LCB_OK;
     CK(c, cudaSetDevice(c->device));
@@ -1368,7 +1372,7 @@ int lcb_lm_verify_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t*
     int64_t total = 0;
     CK(c, last_offset(c, chmsg, chmsg_off, n, &total));
     Staging sg(c);
-    const uint8_t *d_vkp, *d_sigp, *d_msg;
+    const uint8_t *d_vkp, *d_sigp, *d_msg, *d_stp = nullptr;
     const int64_t* d_off;
     uint8_t* d_verdict;
     CK(c, sg.in(&d_vkp, vk_packed, (size_t)n * 2 * 32 * vk_bits));
@@ -1376,8 +1380,9 @@ int lcb_lm_verify_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t*
     CK(c, sg.in(&d_off, chmsg_off, (size_t)n + 1));
     bool piped = false;
     CK(c, sg.in_piped(&d_sigp, sig_packed, (size_t)n * l * 32 * sig_bits, &piped));
+    if (st_packed) CK(c, sg.in(&d_stp, st_packed, (size_t)n * 32 * st_bits));
     CK(c, sg.out(&d_verdict, verdict, (size_t)n));
-    if ((reinterpret_cast<uintptr_t>(d_vkp) | reinterpret_cast<uintptr_t>(d_sigp)) & 3u)
+    if ((reinterpret_cast<uintptr_t>(d_vkp) | reinterpret_cast<uintptr_t>(d_sigp) | reinterpret_cast<uintptr_t>(d_stp)) & 3u)
         return fail(c, LCB_ERR_INVALID, "packed buffers must be 4-byte aligned");
     const int64_t chunk = n < 2 * kPipeChunk ? n : 2 * kPipeChunk;
     // The two shipped packings (11/14 and 13/16 bits) are expanded inside k_verify; any other width is unpacked
@@ -1385,14 +1390,18 @@ int lcb_lm_verify_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t*
     // The fused route streams packed signature rows with 16-byte cp.async and reads 16-bit key slots with 128-bit
     // loads, so it needs 16-byte aligned buffers (staged host buffers always are); a caller-owned device buffer that
     // is only 4-byte aligned takes the unpack-first route instead of raising a sticky misaligned-address fault.
+    // Statements are read like key halves: they must have the key width and, at 16 bits, 16-byte aligned rows.
     const bool aligned16 = (reinterpret_cast<uintptr_t>(d_sigp) & 15u) == 0 &&
-                           (vk_bits == 14 || (reinterpret_cast<uintptr_t>(d_vkp) & 15u) == 0);
-    const bool fused = aligned16 && ((sig_bits == 11 && vk_bits == 14) || (sig_bits == 13 && vk_bits == 16));
-    uint16_t* d_vk = nullptr;
+                           (vk_bits == 14 || (reinterpret_cast<uintptr_t>(d_vkp) & 15u) == 0) &&
+                           (!d_stp || vk_bits == 14 || (reinterpret_cast<uintptr_t>(d_stp) & 15u) == 0);
+    const bool fused = aligned16 && (!d_stp || st_bits == vk_bits) &&
+                       ((sig_bits == 11 && vk_bits == 14) || (sig_bits == 13 && vk_bits == 16));
+    uint16_t *d_vk = nullptr, *d_st = nullptr;
     int16_t *d_sig = nullptr, *d_pairs;
     if (!fused) {
         CK(c, sg.alloc((void**)&d_vk, (size_t)chunk * 2 * D * sizeof(uint16_t)));
         CK(c, sg.alloc((void**)&d_sig, (size_t)chunk * l * D * sizeof(int16_t)));
+        if (d_stp) CK(c, sg.alloc((void**)&d_st, (size_t)chunk * D * sizeof(uint16_t)));
     }
     CK(c, sg.alloc((void**)&d_pairs, (size_t)chunk * sch->ch_wt * 2 * sizeof(int16_t)));
     // packed signatures in HOST memory cross PCIe chunk by chunk under the kernels of the previous chunk
@@ -1417,13 +1426,18 @@ int lcb_lm_verify_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t*
             CK(c, timed(c, K_VERIFY, [&] {
                 return launch_verify_packed(c->ring, d_sigp + (size_t)first * sig_row, sig_bits, sig_bias,
                                             d_vkp + (size_t)first * 2 * 32 * vk_bits, vk_bits, d_pairs, sch->ch_wt, m,
-                                            bd > 32767 ? 32767 : bd, wt, d_verdict + first, c->stream);
+                                            bd > 32767 ? 32767 : bd, wt, d_verdict + first, c->stream,
+                                            d_stp ? d_stp + (size_t)first * 32 * st_bits : nullptr);
             }));
             continue;
         }
         CK(c, timed(c, K_UNPACK, [&] {
             return launch_unpack(c->ring, d_vkp + (size_t)first * 2 * 32 * vk_bits, m * 2, vk_bits, 0, d_vk, c->stream);
         }));
+        if (d_stp)
+            CK(c, timed(c, K_UNPACK, [&] {
+                return launch_unpack(c->ring, d_stp + (size_t)first * 32 * st_bits, m, st_bits, 0, d_st, c->stream);
+            }));
         if (piped) CK(c, cudaStreamWaitEvent(c->stream, arrived[k], 0));
         CK(c, timed(c, K_UNPACK, [&] {
             return launch_unpack(c->ring, d_sigp + (size_t)first * l * 32 * sig_bits, m * l, sig_bits, sig_bias, d_sig,
@@ -1432,9 +1446,95 @@ int lcb_lm_verify_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t*
         int st = run_challenge(c, sch, d_msg, d_off + first, m, d_pairs);
         if (st != LCB_OK) return st;
         CK(c, timed(c, K_VERIFY, [&] {
-            return launch_verify(c->ring, d_sig, d_vk, d_pairs, sch->ch_wt, nullptr, nullptr, m, bd > 32767 ? 32767 : bd,
+            return launch_verify(c->ring, d_sig, d_vk, d_pairs, sch->ch_wt, nullptr, d_st, m, bd > 32767 ? 32767 : bd,
                                  wt, d_verdict + first, c->stream);
         }));
+    }
+    CK(c, sg.finish());
+    return LCB_OK;
+}
+
+// polynomials per chunk of the composed wire routes (sign, adapt, extract): bounds their int16 scratch
+constexpr int64_t kWireChunkPoly = (int64_t)1 << 20;
+
+}  // namespace
+
+extern "C" {
+
+int lcb_lm_verify_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* vk_packed, int vk_bits,
+                               const uint8_t* chmsg, const int64_t* chmsg_off, const uint8_t* sig_packed, int sig_bits,
+                               int sig_bias, int64_t n, int bd, int wt, uint8_t* verdict) {
+    LCB_RANGE();
+    if (!c || !sch || !vk_packed || !chmsg_off || !sig_packed || !verdict || n < 0 || bd < 0 || wt < 0 ||
+        vk_bits < 1 || vk_bits > 16 || sig_bits < 1 || sig_bits > 16 || sig_bias < 0 || sig_bias > 32767)
+        return LCB_ERR_INVALID;
+    return verify_packed(c, sch, vk_packed, vk_bits, chmsg, chmsg_off, sig_packed, sig_bits, sig_bias, nullptr, 0, n, bd,
+                         wt, verdict);
+}
+
+int lcb_adaptor_verify_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* vk_packed, int vk_bits,
+                                    const uint8_t* chmsg, const int64_t* chmsg_off, const uint8_t* sig_packed,
+                                    int sig_bits, int sig_bias, const uint8_t* st_packed, int st_bits, int64_t n, int bd,
+                                    int wt, uint8_t* verdict) {
+    LCB_RANGE();
+    if (!c || !sch || !vk_packed || !chmsg_off || !sig_packed || !st_packed || !verdict || n < 0 || bd < 0 || wt < 0 ||
+        !wire_args_ok(vk_bits, 0) || !wire_args_ok(sig_bits, sig_bias) || !wire_args_ok(st_bits, 0))
+        return LCB_ERR_INVALID;
+    return verify_packed(c, sch, vk_packed, vk_bits, chmsg, chmsg_off, sig_packed, sig_bits, sig_bias, st_packed, st_bits,
+                         n, bd, wt, verdict);
+}
+
+// lcb_lm_sign_batch -> lcb_pack_batch in one call.  Fused route (11- or 13-bit rows, 16-byte aligned): k_sign writes the
+// packed rows and in_range flags itself.  Anything else signs into int16 scratch and packs it with k_pack, in chunks.
+int lcb_lm_sign_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const uint16_t* sk_ntt, const uint8_t* chmsg,
+                             const int64_t* chmsg_off, int64_t n, int sig_bits, int sig_bias, uint8_t* sig_packed,
+                             uint8_t* in_range) {
+    LCB_RANGE();
+    if (!c || !sch || !sk_ntt || !chmsg_off || !sig_packed || n < 0 || !wire_args_ok(sig_bits, sig_bias))
+        return LCB_ERR_INVALID;
+    if (c->generic) return fail(c, LCB_ERR_INVALID, "the packed wire format is defined for d == 256, q < 2^16 contexts only");
+    if (n == 0) return LCB_OK;
+    CK(c, cudaSetDevice(c->device));
+    const int l = c->l;
+    int64_t total = 0;
+    CK(c, last_offset(c, chmsg, chmsg_off, n, &total));
+    Staging sg(c);
+    const uint16_t* d_sk;
+    const uint8_t* d_msg;
+    const int64_t* d_off;
+    uint8_t *d_sigp, *d_range;
+    int16_t* d_pairs;
+    const size_t row = (size_t)32 * sig_bits;
+    CK(c, sg.in(&d_sk, sk_ntt, (size_t)n * 2 * l * D, true));
+    CK(c, sg.in(&d_msg, chmsg, (size_t)total));
+    CK(c, sg.in(&d_off, chmsg_off, (size_t)n + 1));
+    CK(c, sg.out(&d_sigp, sig_packed, (size_t)n * l * row));
+    CK(c, sg.out(&d_range, in_range, (size_t)n * l));
+    if (reinterpret_cast<uintptr_t>(d_sigp) & 3u) return fail(c, LCB_ERR_INVALID, "packed buffer must be 4-byte aligned");
+    CK(c, sg.alloc((void**)&d_pairs, (size_t)n * sch->ch_wt * 2 * sizeof(int16_t)));
+    int st = run_challenge(c, sch, d_msg, d_off, n, d_pairs);
+    if (st != LCB_OK) return st;
+    // k_sign stores whole packed rows with 16-byte stores: a caller-owned device buffer that is only 4-byte aligned
+    // takes the composed route
+    if ((sig_bits == 11 || sig_bits == 13) && (reinterpret_cast<uintptr_t>(d_sigp) & 15u) == 0) {
+        CK(c, timed(c, K_SIGN, [&] {
+            return launch_sign_packed(c->ring, d_sk, d_pairs, sch->ch_wt, n, sig_bits, sig_bias, d_sigp, d_range, c->stream);
+        }));
+    } else {
+        const int64_t chunk = n < kWireChunkPoly / l ? n : kWireChunkPoly / l;
+        int16_t* d_sig;
+        CK(c, sg.alloc((void**)&d_sig, (size_t)chunk * l * D * sizeof(int16_t)));
+        for (int64_t first = 0; first < n; first += chunk) {
+            const int64_t m = n - first < chunk ? n - first : chunk;
+            CK(c, timed(c, K_SIGN, [&] {
+                return launch_sign(c->ring, d_sk + (size_t)first * 2 * l * D, d_pairs + (size_t)first * sch->ch_wt * 2,
+                                   sch->ch_wt, m, d_sig, c->stream);
+            }));
+            CK(c, timed(c, K_PACK, [&] {
+                return launch_pack(c->ring, d_sig, m * l, sig_bits, sig_bias, d_sigp + (size_t)first * l * row,
+                                   d_range ? d_range + (size_t)first * l : nullptr, c->stream);
+            }));
+        }
     }
     CK(c, sg.finish());
     return LCB_OK;
@@ -1840,6 +1940,85 @@ int lcb_vec_add_batch(lcb_ctx* c, const int16_t* a, const int16_t* b, int64_t np
 
 int lcb_vec_sub_batch(lcb_ctx* c, const int16_t* a, const int16_t* b, int64_t npoly, int16_t* out) {
     return vec_addsub(c, a, b, npoly, 1, out);
+}
+
+// adapt / extract on the wire format: unpack -> k_vec_addsub -> (pack), in chunks of bounded int16 scratch.  HBM streams of
+// a few thousand operations per signature, so they are composed from the existing kernels and exact by construction.
+int lcb_adaptor_adapt_packed_batch(lcb_ctx* c, const uint8_t* presig_packed, int presig_bits, int presig_bias,
+                                   const int16_t* wit_coef, int64_t npoly, int sig_bits, int sig_bias, uint8_t* sig_packed,
+                                   uint8_t* in_range) {
+    LCB_RANGE();
+    if (!c || !presig_packed || !wit_coef || !sig_packed || npoly < 0 || !wire_args_ok(presig_bits, presig_bias) ||
+        !wire_args_ok(sig_bits, sig_bias))
+        return LCB_ERR_INVALID;
+    if (c->generic) return fail(c, LCB_ERR_INVALID, "the packed wire format is defined for d == 256, q < 2^16 contexts only");
+    if (npoly == 0) return LCB_OK;
+    CK(c, cudaSetDevice(c->device));
+    Staging sg(c);
+    const uint8_t* d_prep;
+    const int16_t* d_wit;
+    uint8_t *d_sigp, *d_range;
+    CK(c, sg.in(&d_prep, presig_packed, (size_t)npoly * 32 * presig_bits));
+    CK(c, sg.in(&d_wit, wit_coef, (size_t)npoly * D, true));
+    CK(c, sg.out(&d_sigp, sig_packed, (size_t)npoly * 32 * sig_bits));
+    CK(c, sg.out(&d_range, in_range, (size_t)npoly));
+    if ((reinterpret_cast<uintptr_t>(d_prep) | reinterpret_cast<uintptr_t>(d_sigp)) & 3u)
+        return fail(c, LCB_ERR_INVALID, "packed buffers must be 4-byte aligned");
+    const int64_t chunk = npoly < kWireChunkPoly ? npoly : kWireChunkPoly;
+    int16_t *d_pre, *d_sig;
+    CK(c, sg.alloc((void**)&d_pre, (size_t)chunk * D * sizeof(int16_t)));
+    CK(c, sg.alloc((void**)&d_sig, (size_t)chunk * D * sizeof(int16_t)));
+    for (int64_t first = 0; first < npoly; first += chunk) {
+        const int64_t m = npoly - first < chunk ? npoly - first : chunk;
+        CK(c, timed(c, K_UNPACK, [&] {
+            return launch_unpack(c->ring, d_prep + (size_t)first * 32 * presig_bits, m, presig_bits, presig_bias, d_pre,
+                                 c->stream);
+        }));
+        CK(c, timed(c, K_ADDSUB, [&] { return launch_vec_addsub(c->ring, d_pre, d_wit + (size_t)first * D, m * D, 0, d_sig, c->stream); }));
+        CK(c, timed(c, K_PACK, [&] {
+            return launch_pack(c->ring, d_sig, m, sig_bits, sig_bias, d_sigp + (size_t)first * 32 * sig_bits,
+                               d_range ? d_range + first : nullptr, c->stream);
+        }));
+    }
+    CK(c, sg.finish());
+    return LCB_OK;
+}
+
+int lcb_adaptor_extract_packed_batch(lcb_ctx* c, const uint8_t* sig_packed, int sig_bits, int sig_bias,
+                                     const uint8_t* presig_packed, int presig_bits, int presig_bias, int64_t npoly,
+                                     int16_t* wit_coef) {
+    LCB_RANGE();
+    if (!c || !sig_packed || !presig_packed || !wit_coef || npoly < 0 || !wire_args_ok(sig_bits, sig_bias) ||
+        !wire_args_ok(presig_bits, presig_bias))
+        return LCB_ERR_INVALID;
+    if (c->generic) return fail(c, LCB_ERR_INVALID, "the packed wire format is defined for d == 256, q < 2^16 contexts only");
+    if (npoly == 0) return LCB_OK;
+    CK(c, cudaSetDevice(c->device));
+    Staging sg(c);
+    const uint8_t *d_sigp, *d_prep;
+    int16_t* d_wit;
+    CK(c, sg.in(&d_sigp, sig_packed, (size_t)npoly * 32 * sig_bits));
+    CK(c, sg.in(&d_prep, presig_packed, (size_t)npoly * 32 * presig_bits));
+    CK(c, sg.out(&d_wit, wit_coef, (size_t)npoly * D, true));
+    if ((reinterpret_cast<uintptr_t>(d_sigp) | reinterpret_cast<uintptr_t>(d_prep)) & 3u)
+        return fail(c, LCB_ERR_INVALID, "packed buffers must be 4-byte aligned");
+    const int64_t chunk = npoly < kWireChunkPoly ? npoly : kWireChunkPoly;
+    int16_t *d_sig, *d_pre;
+    CK(c, sg.alloc((void**)&d_sig, (size_t)chunk * D * sizeof(int16_t)));
+    CK(c, sg.alloc((void**)&d_pre, (size_t)chunk * D * sizeof(int16_t)));
+    for (int64_t first = 0; first < npoly; first += chunk) {
+        const int64_t m = npoly - first < chunk ? npoly - first : chunk;
+        CK(c, timed(c, K_UNPACK, [&] {
+            return launch_unpack(c->ring, d_sigp + (size_t)first * 32 * sig_bits, m, sig_bits, sig_bias, d_sig, c->stream);
+        }));
+        CK(c, timed(c, K_UNPACK, [&] {
+            return launch_unpack(c->ring, d_prep + (size_t)first * 32 * presig_bits, m, presig_bits, presig_bias, d_pre,
+                                 c->stream);
+        }));
+        CK(c, timed(c, K_ADDSUB, [&] { return launch_vec_addsub(c->ring, d_sig, d_pre, m * D, 1, d_wit + (size_t)first * D, c->stream); }));
+    }
+    CK(c, sg.finish());
+    return LCB_OK;
 }
 
 int lcb_adaptor_witness_verify_batch(lcb_ctx* c, const int16_t* wit_coef, const uint16_t* st_ntt, int64_t n, int bd,

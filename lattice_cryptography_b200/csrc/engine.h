@@ -146,10 +146,15 @@ cudaError_t launch_sign(const RingCtx& c, const uint16_t* sk_ntt, const int16_t*
 cudaError_t launch_verify(const RingCtx& c, const int16_t* vec_coef, const uint16_t* vk_ntt,
                           const int16_t* ch_pairs, int ch_wt, const uint16_t* rhs_only, const uint16_t* extra_rhs,
                           int64_t n, int bd, int wt, uint8_t* verdict, cudaStream_t st);
-// the same on packed wire-format rows (sig_bits/vk_bits = 11/14 or 13/16); cudaErrorNotSupported otherwise
+// the same on packed wire-format rows (sig_bits/vk_bits = 11/14 or 13/16); cudaErrorNotSupported otherwise.  st_packed
+// (adaptor verify; nullable): statements packed at vk_bits bits, bias 0, 16-byte aligned at 16 bits
 cudaError_t launch_verify_packed(const RingCtx& c, const uint8_t* sig_packed, int sig_bits, int sig_bias,
                                  const uint8_t* vk_packed, int vk_bits, const int16_t* ch_pairs, int ch_wt, int64_t n,
-                                 int bd, int wt, uint8_t* verdict, cudaStream_t st);
+                                 int bd, int wt, uint8_t* verdict, cudaStream_t st, const uint8_t* st_packed = nullptr);
+// sign straight into the wire format (sig_bits = 11 / 13, 16-byte aligned rows; cudaErrorNotSupported otherwise):
+// sig_packed uint8[n][l][32*sig_bits], in_range (nullable) uint8[n][l], as launch_sign -> launch_pack would write them
+cudaError_t launch_sign_packed(const RingCtx& c, const uint16_t* sk_ntt, const int16_t* ch_pairs, int ch_wt, int64_t n,
+                               int sig_bits, int sig_bias, uint8_t* sig_packed, uint8_t* in_range, cudaStream_t st);
 cudaError_t launch_vec_addsub(const RingCtx& c, const int16_t* a, const int16_t* b, int64_t nelem, int sub,
                               int16_t* out, cudaStream_t st);
 cudaError_t launch_agg_partial(const RingCtx& c, const int16_t* sigs, const int16_t* ag_pairs, int64_t count,

@@ -371,13 +371,66 @@ constexpr int SIGN_BLOCKS = 4;        // resident blocks per SM k_sign is compil
                                       // registers: 6.10 instead of 6.03 ms per 2^20, 6 at 80: 6.13 ms)
 #endif
 
+// Packed epilogue of k_sign<SIG_BITS>: one row of signature coefficients (lane t holds coefficients t + 16 j after the
+// inverse transform) -> 32*SIG_BITS bytes of the wire format (wire.cu) and the row's in_range flag, exactly as k_pack
+// would write them from the int16 row.  The half-warp's transposition buffer is free between two transforms and holds
+// both stages: (1) the biased 16-bit values in natural order, 16 consecutive values per 12-word group (the pitch makes
+// the 128-bit reads of step 2 conflict-free); (2) lane t packs values 16 t .. 16 t + 15 into SIG_BITS halfwords at
+// halfword SIG_BITS * t of the packed row; (3) the row leaves in 16-byte coalesced stores (352 / 416 bytes at 11 / 13
+// bits are multiples of 16).
+constexpr int SIGN_PACK_PITCH = 12;                       // words per group of 16 values
+constexpr int SIGN_PACK_ROW = 16 * SIGN_PACK_PITCH;       // word offset of the packed row in the buffer
+static_assert(SIGN_PACK_ROW + 8 * 16 <= XHALF, "the packed epilogue must fit the half-warp's transposition buffer");
+template <int SIG_BITS>
+__device__ __forceinline__ void sign_store_packed(const uint32_t (&a)[EPT], const ModQ& m, uint32_t bias, uint32_t* xb,
+                                                  int lane, unsigned mask, bool live, uint8_t* __restrict__ out_row,
+                                                  uint8_t* __restrict__ range_flag) {
+    uint16_t* v16 = reinterpret_cast<uint16_t*>(xb);
+#pragma unroll
+    for (int j = 0; j < EPT; ++j) v16[2 * SIGN_PACK_PITCH * j + lane] = (uint16_t)((uint32_t)center_lazy4(a[j], m) + bias);
+    __syncwarp();
+    const uint4 lo = *reinterpret_cast<const uint4*>(xb + SIGN_PACK_PITCH * lane);
+    const uint4 hi = *reinterpret_cast<const uint4*>(xb + SIGN_PACK_PITCH * lane + 4);
+    const uint32_t w[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
+    uint16_t* pk = reinterpret_cast<uint16_t*>(xb + SIGN_PACK_ROW) + SIG_BITS * lane;
+    constexpr uint32_t LIMIT = 1u << SIG_BITS;
+    bool ok = true;
+    uint32_t acc = 0;
+    int fill = 0, nh = 0;
+#pragma unroll
+    for (int i = 0; i < 16; ++i) {
+        const uint32_t v = (w[i >> 1] >> (16 * (i & 1))) & 0xFFFFu;
+        ok = ok && v < LIMIT;
+        acc |= (v & (LIMIT - 1)) << fill;
+        fill += SIG_BITS;
+        if (fill >= 16) {                       // at most one halfword per value: fill < 16 + SIG_BITS <= 32
+            pk[nh++] = (uint16_t)acc;
+            acc >>= 16;
+            fill -= 16;
+        }
+    }
+    __syncwarp();
+    if (live) {
+        const uint4* src = reinterpret_cast<const uint4*>(xb + SIGN_PACK_ROW);
+#pragma unroll
+        for (int k = lane; k < 2 * SIG_BITS; k += LANES) reinterpret_cast<uint4*>(out_row)[k] = src[k];
+    }
+    const unsigned bad = __ballot_sync(0xFFFFFFFFu, !ok) & mask;
+    if (live && range_flag && lane == 0) *range_flag = bad ? 0 : 1;
+    __syncwarp();                               // the buffer belongs to the next transform again
+}
+
 // sig = sk_left ** c + sk_right.  Both transforms are FP32-assisted (round 2): the challenge goes through
 // ntt_fwd_256_fp, every row through the decimation-in-time inverse ntt_inv_256_fp, whose closing twist absorbs the
 // d^-1 scaling; all per-lane twiddles sit in shared memory.  (Round 1: Shoup butterflies, 96 quarter-rate IMAD.HI per
 // row, 7.3 ms per 2^20 with the FMA-heavy pipe as the limiter.)
+// SIG_BITS = 0 writes int16 rows to sig; 11 / 13 write packed rows (bias sig_bias) to `sig` read as uint8 and, when
+// in_range is not null, one in_range flag per row (sign_store_packed).
+template <int SIG_BITS>
 __global__ void __launch_bounds__(RBS, SIGN_BLOCKS) k_sign(ModQ m, StageConstF scf, StageConstF iscf, const NttTables* __restrict__ tab, int l,
                                               const uint16_t* __restrict__ sk_ntt, const int16_t* __restrict__ ch_pairs,
-                                              int ch_wt, int64_t n, int16_t* __restrict__ sig) {
+                                              int ch_wt, int64_t n, int16_t* __restrict__ sig,
+                                              uint8_t* __restrict__ in_range, int sig_bias) {
     extern __shared__ __align__(16) uint32_t smem[];
     uint32_t* xbuf = smem;
     unsigned char* stage = reinterpret_cast<unsigned char*>(xbuf + (RBS / 32) * XWARP);
@@ -454,10 +507,17 @@ __global__ void __launch_bounds__(RBS, SIGN_BLOCKS) k_sign(ModQ m, StageConstF s
 #pragma unroll
             for (int k = 0; k < EPT; ++k) a[k] = barrett_lazy(c[k] * a[k], m) + b[k] + FP_BIAS;   // < 2q + 2^16, biased
             ntt_inv_256_fp(a, m, iscf, itwf, h.xb, h.lane);
-            if (live) {
-                int16_t* out = sig + (item * l + i) * D;
+            if constexpr (SIG_BITS == 0) {
+                if (live) {
+                    int16_t* out = sig + (item * l + i) * D;
 #pragma unroll
-                for (int j = 0; j < EPT; ++j) out[h.lane + 16 * j] = (int16_t)center_lazy4(a[j], m);
+                    for (int j = 0; j < EPT; ++j) out[h.lane + 16 * j] = (int16_t)center_lazy4(a[j], m);
+                }
+            } else {
+                const int64_t row = item * l + i;
+                sign_store_packed<SIG_BITS>(a, m, (uint32_t)sig_bias, h.xb, h.lane, h.mask, live,
+                                            reinterpret_cast<uint8_t*>(sig) + row * (32 * SIG_BITS),
+                                            in_range ? in_range + row : nullptr);
             }
         }
     }
@@ -484,7 +544,9 @@ __device__ __forceinline__ void load_u14x16(uint32_t (&r)[EPT], const uint32_t* 
 // SIG_BITS / VK_BITS: 0 = int16 coefficients / uint16 slots; otherwise the inputs are rows of the packed wire
 // format (wire.cu): signatures SIG_BITS bits per coefficient with bias sig_bias, keys VK_BITS (14) bits per slot.
 // The packed rows ride through the same cp.async stage buffers and are expanded on the way into registers.
-template <bool CHECK_WT, int SIG_BITS, int VK_BITS>
+// ST_BITS: 0 = extra_rhs holds uint16 statement slots; 14 = 14-bit packed statements (bias 0, 7 words per lane, read as
+// the key halves are).  A 16-bit packed statement has the bytes of a uint16 row and takes ST_BITS = 0.
+template <bool CHECK_WT, int SIG_BITS, int VK_BITS, int ST_BITS = 0>
 __global__ void __launch_bounds__(VBS, VERIFY_BLOCKS) k_verify(ModQ m, StageConst sc, StageConstF scf, const NttTables* __restrict__ tab,
                                                 const uint32_t* __restrict__ a_hat_g, int l,
                                                 const int16_t* __restrict__ vec_coef,
@@ -640,7 +702,10 @@ __global__ void __launch_bounds__(VBS, VERIFY_BLOCKS) k_verify(ModQ m, StageCons
         }
         if (extra_rhs) {
             uint32_t ex[EPT];
-            load_u16x16(ex, extra_rhs + item * D + 16 * h.lane);
+            if (ST_BITS == 14)
+                load_u14x16(ex, reinterpret_cast<const uint32_t*>(extra_rhs) + item * 112 + 7 * h.lane);
+            else
+                load_u16x16(ex, extra_rhs + item * D + 16 * h.lane);
 #pragma unroll
             for (int k = 0; k < EPT; ++k) rhs[k] += ex[k];
         }
@@ -1333,25 +1398,41 @@ cudaError_t launch_matvec(const RingCtx& c, const int16_t* vec_coef, int64_t nve
     return cudaGetLastError();
 }
 
-cudaError_t launch_sign(const RingCtx& c, const uint16_t* sk_ntt, const int16_t* ch_pairs, int ch_wt, int64_t n,
-                        int16_t* sig, cudaStream_t st) {
+template <int SIG_BITS>
+cudaError_t launch_sign_t(const RingCtx& c, const uint16_t* sk_ntt, const int16_t* ch_pairs, int ch_wt, int64_t n,
+                          void* sig, uint8_t* in_range, int sig_bias, cudaStream_t st) {
     if (n <= 0) return cudaSuccess;
     const size_t smem = (size_t)(RBS / 32) * XWARP * 4 + (size_t)HWB * SIGN_STAGE_BYTES + (size_t)TW_BYTES + (size_t)ITW_BYTES;
-    cudaError_t e = allow_smem(k_sign, smem);
+    cudaError_t e = allow_smem(k_sign<SIG_BITS>, smem);
     if (e != cudaSuccess) return e;
-    unsigned grid = persistent_grid(n, HWB, c.num_sms, resident_blocks(k_sign, RBS, smem));
-    k_sign<<<grid, RBS, smem, st>>>(c.m, c.scf, c.iscf, c.tab, c.l, sk_ntt, ch_pairs, ch_wt, n, sig);
+    unsigned grid = persistent_grid(n, HWB, c.num_sms, resident_blocks(k_sign<SIG_BITS>, RBS, smem));
+    k_sign<SIG_BITS><<<grid, RBS, smem, st>>>(c.m, c.scf, c.iscf, c.tab, c.l, sk_ntt, ch_pairs, ch_wt, n,
+                                              static_cast<int16_t*>(sig), in_range, sig_bias);
     return cudaGetLastError();
 }
 
-template <int SIG_BITS, int VK_BITS>
+cudaError_t launch_sign(const RingCtx& c, const uint16_t* sk_ntt, const int16_t* ch_pairs, int ch_wt, int64_t n,
+                        int16_t* sig, cudaStream_t st) {
+    return launch_sign_t<0>(c, sk_ntt, ch_pairs, ch_wt, n, sig, nullptr, 0, st);
+}
+
+// The two shipped signature widths are written by k_sign itself; anything else is reported as unsupported and the
+// caller signs into int16 scratch and packs.
+cudaError_t launch_sign_packed(const RingCtx& c, const uint16_t* sk_ntt, const int16_t* ch_pairs, int ch_wt, int64_t n,
+                               int sig_bits, int sig_bias, uint8_t* sig_packed, uint8_t* in_range, cudaStream_t st) {
+    if (sig_bits == 11) return launch_sign_t<11>(c, sk_ntt, ch_pairs, ch_wt, n, sig_packed, in_range, sig_bias, st);
+    if (sig_bits == 13) return launch_sign_t<13>(c, sk_ntt, ch_pairs, ch_wt, n, sig_packed, in_range, sig_bias, st);
+    return cudaErrorNotSupported;
+}
+
+template <int SIG_BITS, int VK_BITS, int ST_BITS = 0>
 cudaError_t launch_verify_t(const RingCtx& c, const void* vec, const void* vk, const int16_t* ch_pairs, int ch_wt,
                             const uint16_t* rhs_only, const uint16_t* extra_rhs, int64_t n, int bd, int wt, int sig_bias,
                             uint8_t* verdict, cudaStream_t st) {
     if (n <= 0) return cudaSuccess;
     if (n > ((int64_t)1 << 30)) return cudaErrorInvalidValue;      // 32-bit item indices inside the kernel
     size_t smem = verify_smem(c.l);
-    auto kern = wt < D ? k_verify<true, SIG_BITS, VK_BITS> : k_verify<false, SIG_BITS, VK_BITS>;
+    auto kern = wt < D ? k_verify<true, SIG_BITS, VK_BITS, ST_BITS> : k_verify<false, SIG_BITS, VK_BITS, ST_BITS>;
     cudaError_t e = allow_smem(kern, smem);
     if (e != cudaSuccess) return e;
     unsigned grid = persistent_grid(n, VHWB, c.num_sms, resident_blocks(kern, VBS, smem));
@@ -1369,13 +1450,18 @@ cudaError_t launch_verify(const RingCtx& c, const int16_t* vec_coef, const uint1
 
 // The two shipped packings are expanded inside the kernel; anything else is reported as unsupported and the
 // caller unpacks first.
+// Packed statements (adaptor verify) have the width of the keys: 14 bits are read by k_verify<..., 11, 14, 14>; 16-bit
+// rows are uint16 rows, read as such.
 cudaError_t launch_verify_packed(const RingCtx& c, const uint8_t* sig_packed, int sig_bits, int sig_bias,
                                  const uint8_t* vk_packed, int vk_bits, const int16_t* ch_pairs, int ch_wt, int64_t n,
-                                 int bd, int wt, uint8_t* verdict, cudaStream_t st) {
+                                 int bd, int wt, uint8_t* verdict, cudaStream_t st, const uint8_t* st_packed) {
+    const uint16_t* ex = reinterpret_cast<const uint16_t*>(st_packed);
+    if (sig_bits == 11 && vk_bits == 14 && st_packed)
+        return launch_verify_t<11, 14, 14>(c, sig_packed, vk_packed, ch_pairs, ch_wt, nullptr, ex, n, bd, wt, sig_bias, verdict, st);
     if (sig_bits == 11 && vk_bits == 14)
         return launch_verify_t<11, 14>(c, sig_packed, vk_packed, ch_pairs, ch_wt, nullptr, nullptr, n, bd, wt, sig_bias, verdict, st);
     if (sig_bits == 13 && vk_bits == 16)
-        return launch_verify_t<13, 0>(c, sig_packed, vk_packed, ch_pairs, ch_wt, nullptr, nullptr, n, bd, wt, sig_bias, verdict, st);
+        return launch_verify_t<13, 0>(c, sig_packed, vk_packed, ch_pairs, ch_wt, nullptr, ex, n, bd, wt, sig_bias, verdict, st);
     return cudaErrorNotSupported;
 }
 

@@ -346,6 +346,59 @@ class Engine(object):
                                                       _addr(verdict)))
         return verdict
 
+    def lm_sign_packed(self, sch: LcbScheme, sk_ntt, chmsgs, sig_bits: int, sig_bias: int, device: bool = False,
+                       want_range: bool = False):
+        """lm_sign straight into the wire format: -> uint8[n, l, 32*sig_bits] (and in_range uint8[n, l] when want_range),
+        exactly pack(lm_sign(...), sig_bits, sig_bias)."""
+        blob, off = self._rag(chmsgs)
+        n = self._count(off)
+        _want(sk_ntt, 'sk_ntt', self.nt, (n, 2, self.l, self.d))
+        sig = self._out((n, self.l, self.d * sig_bits // 8), np.uint8, device)
+        ok = self._out((n, self.l), np.uint8, device) if want_range else None
+        self._ck(self._lib.lcb_lm_sign_packed_batch(self._ctx, byref(sch), _addr(sk_ntt), _addr(blob), _addr(off), n,
+                                                    sig_bits, sig_bias, _addr(sig), _addr(ok)))
+        return (sig, ok) if want_range else sig
+
+    def adaptor_verify_packed(self, sch: LcbScheme, vk_packed, vk_bits: int, chmsgs, sig_packed, sig_bits: int,
+                              sig_bias: int, st_packed, st_bits: int, bd: int, wt: int, device: bool = False, out=None):
+        """lm_verify(..., st_ntt=...) from packed keys uint8[n, 2, 32*vk_bits], signatures uint8[n, l, 32*sig_bits] and
+        statements uint8[n, 32*st_bits] (bias 0)."""
+        blob, off = self._rag(chmsgs)
+        n = self._count(off)
+        _want(vk_packed, 'vk_packed', np.uint8, (n, 2, self.d * vk_bits // 8))
+        _want(sig_packed, 'sig_packed', np.uint8, (n, self.l, self.d * sig_bits // 8))
+        _want(st_packed, 'st_packed', np.uint8, (n, self.d * st_bits // 8))
+        verdict = _want(out, 'out', np.uint8, (n,)) if out is not None else self._out((n,), np.uint8, device)
+        self._ck(self._lib.lcb_adaptor_verify_packed_batch(self._ctx, byref(sch), _addr(vk_packed), vk_bits, _addr(blob),
+                                                           _addr(off), _addr(sig_packed), sig_bits, sig_bias,
+                                                           _addr(st_packed), st_bits, n, bd, wt, _addr(verdict)))
+        return verdict
+
+    def adapt_packed(self, presig_packed, presig_bits: int, presig_bias: int, wit_coef, sig_bits: int, sig_bias: int,
+                     device: bool = False, want_range: bool = False):
+        """presig uint8[..., 32*presig_bits] + wit int16[..., 256] -> uint8[..., 32*sig_bits] (and in_range uint8[...]),
+        exactly pack(vec_add(unpack(presig), wit))."""
+        npoly = _lead(presig_packed, 'presig_packed', np.uint8, self.d * presig_bits // 8)
+        lead = tuple(presig_packed.shape[:-1])
+        _want(wit_coef, 'wit_coef', self.ct, lead + (self.d,))
+        sig = self._out(lead + (self.d * sig_bits // 8,), np.uint8, device)
+        ok = self._out(lead, np.uint8, device) if want_range else None
+        self._ck(self._lib.lcb_adaptor_adapt_packed_batch(self._ctx, _addr(presig_packed), presig_bits, presig_bias,
+                                                          _addr(wit_coef), npoly, sig_bits, sig_bias, _addr(sig), _addr(ok)))
+        return (sig, ok) if want_range else sig
+
+    def extract_packed(self, sig_packed, sig_bits: int, sig_bias: int, presig_packed, presig_bits: int, presig_bias: int,
+                       device: bool = False):
+        """-> int16[..., 256] = vec_sub(unpack(sig), unpack(presig))."""
+        npoly = _lead(sig_packed, 'sig_packed', np.uint8, self.d * sig_bits // 8)
+        lead = tuple(sig_packed.shape[:-1])
+        _want(presig_packed, 'presig_packed', np.uint8, lead + (self.d * presig_bits // 8,))
+        wit = self._out(lead + (self.d,), self.ct, device)
+        self._ck(self._lib.lcb_adaptor_extract_packed_batch(self._ctx, _addr(sig_packed), sig_bits, sig_bias,
+                                                            _addr(presig_packed), presig_bits, presig_bias, npoly,
+                                                            _addr(wit)))
+        return wit
+
     # ------------------------------------------------------------------ BKLM aggregation
     def agg_coefs(self, sch: LcbScheme, agmsg, first: int, count: int, device: bool = False):
         if isinstance(agmsg, (str, bytes, bytearray)):

@@ -9,6 +9,12 @@ module is therefore OPT-IN and does not change what the drop-in API computes:
   13 at 256) instead of 16 - 4,576 / 9,568 bytes per signature instead of 6,656 / 11,776;
 * `pack_keys` / `unpack_keys`: NTT-form verification keys in `key_bits(pp)` bits (14 / 16);
 * `verify_batch_packed`: `lm_one_time_sigs.verify_batch` straight from the packed records;
+* `sign_batch_packed`: `lm_one_time_sigs.sign_batch` straight into packed signatures (bias `vf_bd`), without the int16
+  signatures making a round trip;
+* adaptor signatures (`adaptor_sigs`) on packed records, every width and bias taken from the adaptor `pp`:
+  `presign_batch_packed` (presignatures in `sig_bits(pp, 'pvf_bd')` bits, bias `pvf_bd`: 11 / 13), `preverify_batch_packed`,
+  `adapt_batch_packed` (adaptor signatures in `sig_bits(pp)` bits, bias `vf_bd`: 11 / 13), `adaptor_verify_batch_packed`
+  (statements packed like keys with `pack_keys`) and `extract_batch_packed` (int16 witnesses);
 * `aggregate_batch_packed` / `aggregate_verify_batch_packed`: the batched BKLM calls of `bklm_one_time_agg_sigs`
   (many independent aggregates, sorted signatures / keys of group g at agg_off[g] .. agg_off[g+1]) from packed
   signatures and keys, with packed aggregates.  An aggregate is encoded as a signature with the aggregate bound:
@@ -74,6 +80,56 @@ def verify_batch_packed(pp, vk_packed, chmsgs, sig_packed, device: bool = False)
     eng, sch = _ctx(pp)
     return eng.lm_verify_packed(sch, vk_packed, key_bits(pp), chmsgs, sig_packed, sig_bits(pp), pp['vf_bd'],
                                 pp['vf_bd'], pp['vf_wt'], device=device)
+
+
+def sign_batch_packed(pp, sk_ntt, chmsgs, device: bool = False):
+    """LM signatures straight into the wire format: sk_ntt uint16[N, 2, l, 256] -> (uint8[N, l, 32*sig_bits], in_range
+    uint8[N, l]), exactly `pack_signatures(pp, sign_batch(pp, sk_ntt, chmsgs))`."""
+    from .lm_one_time_sigs import _ctx
+    eng, sch = _ctx(pp)
+    return eng.lm_sign_packed(sch, sk_ntt, chmsgs, sig_bits(pp), pp['vf_bd'], device=device, want_range=True)
+
+
+def presign_batch_packed(pp, sk_ntt, chmsgs, device: bool = False):
+    """Adaptor presignatures (adaptor `pp`; chmsgs from `adaptor_sigs.challenge_messages`) -> (uint8[N, l,
+    32*sig_bits(pp, 'pvf_bd')], in_range uint8[N, l]), bias pvf_bd."""
+    from .adaptor_sigs import _ctx
+    eng, sch = _ctx(pp)
+    return eng.lm_sign_packed(sch, sk_ntt, chmsgs, sig_bits(pp, 'pvf_bd'), pp['pvf_bd'], device=device, want_range=True)
+
+
+def preverify_batch_packed(pp, vk_packed, chmsgs, presig_packed, device: bool = False):
+    """N preverify verdicts from packed keys and packed presignatures (bound pvf_bd, weight pvf_wt)."""
+    from .adaptor_sigs import _ctx
+    eng, sch = _ctx(pp)
+    return eng.lm_verify_packed(sch, vk_packed, key_bits(pp), chmsgs, presig_packed, sig_bits(pp, 'pvf_bd'), pp['pvf_bd'],
+                                pp['pvf_bd'], pp['pvf_wt'], device=device)
+
+
+def adapt_batch_packed(pp, presig_packed, wit_coef, device: bool = False):
+    """Packed presignatures + witnesses int16[N, l, 256] -> (adaptor signatures uint8[N, l, 32*sig_bits(pp)], in_range
+    uint8[N, l]), bias vf_bd."""
+    from .adaptor_sigs import _ctx
+    eng, _ = _ctx(pp)
+    return eng.adapt_packed(presig_packed, sig_bits(pp, 'pvf_bd'), pp['pvf_bd'], wit_coef, sig_bits(pp), pp['vf_bd'],
+                            device=device, want_range=True)
+
+
+def extract_batch_packed(pp, presig_packed, sig_packed, device: bool = False):
+    """Witnesses int16[N, l, 256] = signature - presignature, from the two packed records."""
+    from .adaptor_sigs import _ctx
+    eng, _ = _ctx(pp)
+    return eng.extract_packed(sig_packed, sig_bits(pp), pp['vf_bd'], presig_packed, sig_bits(pp, 'pvf_bd'), pp['pvf_bd'],
+                              device=device)
+
+
+def adaptor_verify_batch_packed(pp, vk_packed, chmsgs, st_packed, sig_packed, device: bool = False):
+    """N adaptor verify verdicts from packed keys, packed statements uint8[N, 32*key_bits] (`pack_keys(pp, st_ntt)`)
+    and packed adaptor signatures (bound vf_bd, weight vf_wt)."""
+    from .adaptor_sigs import _ctx
+    eng, sch = _ctx(pp)
+    return eng.adaptor_verify_packed(sch, vk_packed, key_bits(pp), chmsgs, sig_packed, sig_bits(pp), pp['vf_bd'], st_packed,
+                                     key_bits(pp), pp['vf_bd'], pp['vf_wt'], device=device)
 
 
 def aggregate_batch_packed(pp, agg_off, sig_packed, agmsgs, device: bool = False):
