@@ -179,6 +179,31 @@ int lcb_lm_sign_packed_batch(lcb_ctx* ctx, const lcb_scheme* sch, const uint16_t
                              const int64_t* chmsg_off, int64_t n, int sig_bits, int sig_bias,
                              uint8_t* sig_packed, uint8_t* in_range);
 
+/* ---- Keys on the packed wire format.  A packed signing key is uint8[2][l][32*sk_bits]: the rows of sk_left, then those of
+ * sk_right, each a COEFFICIENT-form polynomial packed as above (x = centred coefficient, bias sk_bias).  Shipped packing:
+ * sk_bits = ceil(log2(2 sk_bd + 1)) with bias sk_bd - 7 bits / bias 45 at secpar 128, 8 bits / bias 65 at 256: 224 / 256
+ * bytes per row, 5,824 / 11,776 bytes per key instead of 13,312 / 23,552 for the uint16 NTT form.  Verification keys keep
+ * their packing (NTT form, 14 / 16 bits, bias 0).  Same rules as the packed calls above (bits 1..16, biases 0..32767, packed
+ * buffers 4-byte aligned, d == 256 and q < 2^16 only, host or device buffers), at most 2^30 items.  Signing keys are secret:
+ * host-resident ones are staged through engine scratch that is cleared afterwards. */
+
+/* keygen (lm_one_time_sigs.py:64-97,126-138) into packed keys: exactly lcb_lm_keygen_batch(sk_coef, vk_ntt) ->
+ * lcb_pack_batch(sk_coef, sk_bits, sk_bias, sk_in_range) and lcb_pack_batch(vk_ntt, vk_bits, 0).  sk_packed
+ * uint8[n][2][l][32*sk_bits], sk_in_range uint8[n][2][l], vk_packed uint8[n][2][32*vk_bits]; each may be NULL, but not both
+ * sk_packed and vk_packed.  The 16-bit keys stay in engine scratch, chunk by chunk.  Needs key_ch (LCB_ERR_NO_KEY_CH). */
+int lcb_lm_keygen_packed_batch(lcb_ctx* ctx, const lcb_scheme* sch, const uint8_t* seeds, const int64_t* seed_off, int64_t n,
+                               int sk_bits, int sk_bias, uint8_t* sk_packed, uint8_t* sk_in_range, int vk_bits,
+                               uint8_t* vk_packed);
+
+/* sign (lm_one_time_sigs.py:163-170) / adaptor presign (adaptor_sigs.py:191-195) from packed signing keys into packed rows:
+ * exactly lcb_unpack_batch(sk_packed, 2 n l, sk_bits, sk_bias) -> lcb_ntt_fwd_batch -> lcb_lm_sign_packed_batch(sig_bits,
+ * sig_bias), for any bytes in sk_packed.  sig_packed uint8[n][l][32*sig_bits], in_range (nullable) uint8[n][l].  7- and 8-bit
+ * keys with 11- and 13-bit signatures, monomial challenges (ch_bd == 1) and 16-byte aligned buffers are signed by one kernel
+ * that sums the rotations of the packed rows; anything else is unpacked and transformed into engine scratch first. */
+int lcb_lm_sign_packed_sk_batch(lcb_ctx* ctx, const lcb_scheme* sch, const uint8_t* sk_packed, int sk_bits, int sk_bias,
+                                const uint8_t* chmsg, const int64_t* chmsg_off, int64_t n, int sig_bits, int sig_bias,
+                                uint8_t* sig_packed, uint8_t* in_range);
+
 /* adaptor verify (adaptor_sigs.py:247-266) from packed keys (bias 0), signatures (bias sig_bias) and statements
  * st_packed uint8[n][32*st_bits] (NTT form, bias 0, packed like a key half).  Exactly unpack all three ->
  * lcb_lm_verify_batch(st_ntt = the unpacked statements).  st_packed must not be NULL (preverify is
@@ -331,7 +356,8 @@ int64_t lcb_launch_count(const lcb_ctx* ctx);
  * kernel names: sampler shake256 ntt_fwd ntt_inv poly_mul matvec sign verify vec_addsub agg_coefs
  * agg_partial agg_finish aggv_partial aggv_finish pack unpack, and for the batch calls group_ids agg_coefs_seg
  * agg_partial_seg aggv_partial_seg aggv_residues aggv_limits, and agg_finish_pack for packed aggregates.  The fused packed
- * routes are counted under the kernel they extend: packed signing under sign, packed verification under verify.
+ * routes are counted under the kernel they extend: packed signing (from NTT-form or packed signing keys) under sign, packed
+ * verification under verify.
  * lcb_profile_read synchronises the stream. */
 int lcb_profile_enable(lcb_ctx* ctx, int on);
 int lcb_profile_reset(lcb_ctx* ctx);

@@ -69,6 +69,9 @@ PROTOTYPES = {
     'lcb_lm_verify_packed_batch': (c_int, [c_void_p, POINTER(LcbScheme), _P, c_int, _P, _P, _P, c_int, c_int, c_int64,
                                            c_int, c_int, _P]),
     'lcb_lm_sign_packed_batch': (c_int, [c_void_p, POINTER(LcbScheme), _P, _P, _P, c_int64, c_int, c_int, _P, _P]),
+    'lcb_lm_keygen_packed_batch': (c_int, [c_void_p, POINTER(LcbScheme), _P, _P, c_int64, c_int, c_int, _P, _P, c_int, _P]),
+    'lcb_lm_sign_packed_sk_batch': (c_int, [c_void_p, POINTER(LcbScheme), _P, c_int, c_int, _P, _P, c_int64, c_int, c_int, _P,
+                                            _P]),
     'lcb_adaptor_verify_packed_batch': (c_int, [c_void_p, POINTER(LcbScheme), _P, c_int, _P, _P, _P, c_int, c_int, _P, c_int,
                                                 c_int64, c_int, c_int, _P]),
     'lcb_adaptor_adapt_packed_batch': (c_int, [c_void_p, _P, c_int, c_int, _P, c_int64, c_int, c_int, _P, _P]),

@@ -1132,11 +1132,23 @@ int lcb_poly_mul_batch(lcb_ctx* c, const int16_t* a, const int16_t* b, int64_t n
     return LCB_OK;
 }
 
-int lcb_lm_keygen_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* seeds, const int64_t* seed_off, int64_t n,
-                        int16_t* sk_coef, uint16_t* sk_ntt, uint16_t* vk_ntt, int16_t* vk_coef) {
-    LCB_RANGE();
-    if (!c || !sch || !seed_off || n < 0) return LCB_ERR_INVALID;
-    if (!c->has_key_ch) return fail(c, LCB_ERR_NO_KEY_CH, "lcb_lm_keygen_batch before lcb_set_key_ch");
+}  // extern "C"
+
+namespace {
+
+// Packed outputs of lcb_lm_keygen_packed_batch: each chunk's int16 signing keys and uint16 verification keys are packed
+// before the next chunk reuses the scratch.  sk / vk may each be null.
+struct KeyPack {
+    int sk_bits, sk_bias;
+    uint8_t *sk, *sk_range;
+    int vk_bits;
+    uint8_t* vk;
+};
+
+// The body of lcb_lm_keygen_batch (pk == null) and of lcb_lm_keygen_packed_batch (pk set, every unpacked output null).
+int keygen(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* seeds, const int64_t* seed_off, int64_t n, int16_t* sk_coef,
+           uint16_t* sk_ntt, uint16_t* vk_ntt, int16_t* vk_coef, const KeyPack* pk, const char* name) {
+    if (!c->has_key_ch) return fail(c, LCB_ERR_NO_KEY_CH, std::string(name) + " before lcb_set_key_ch");
     if (n == 0) return LCB_OK;
     CK(c, cudaSetDevice(c->device));
     const int l = c->l;
@@ -1158,6 +1170,14 @@ int lcb_lm_keygen_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* seeds,
     CK(c, sg.out(&d_sk_ntt, sk_ntt, (size_t)n * 2 * l * D_, true));
     CK(c, sg.out(&d_vk_ntt, vk_ntt, (size_t)n * 2 * D_));
     CK(c, sg.out(&d_vk_coef, vk_coef, (size_t)n * 2 * D_));
+    uint8_t *d_skp = nullptr, *d_skr = nullptr, *d_vkp = nullptr;
+    if (pk) {
+        CK(c, sg.out(&d_skp, pk->sk, (size_t)n * 2 * l * 32 * pk->sk_bits, true));
+        CK(c, sg.out(&d_skr, pk->sk_range, (size_t)n * 2 * l));
+        CK(c, sg.out(&d_vkp, pk->vk, (size_t)n * 2 * 32 * pk->vk_bits));
+        if ((reinterpret_cast<uintptr_t>(d_skp) | reinterpret_cast<uintptr_t>(d_vkp)) & 3u)
+            return fail(c, LCB_ERR_INVALID, "packed buffers must be 4-byte aligned");
+    }
     // Signing keys pass through HBM in coefficient form between the sampler and the row-vector
     // product; when the caller does not want them, a bounded scratch chunk is reused.
     // Both halves of a key come from ONE paired sampler launch (stream 2i = left, 2i+1 = right: twice the
@@ -1176,6 +1196,8 @@ int lcb_lm_keygen_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* seeds,
     }
     int16_t* scratch = nullptr;
     if (!d_sk_coef) CK(c, sg.alloc((void**)&scratch, (size_t)chunk * 2 * l * D_ * sizeof(int16_t), true));
+    uint16_t* vk_scratch = nullptr;                                // NTT-form verification keys of a chunk, to be packed
+    if (d_vkp) CK(c, sg.alloc((void**)&vk_scratch, (size_t)chunk * 2 * D_ * sizeof(uint16_t)));
     for (int64_t start = 0; start < n; start += chunk) {
         const int64_t cnt = (n - start < chunk) ? n - start : chunk;
         int16_t* skc = d_sk_coef ? d_sk_coef + start * 2 * l * D_ : scratch;
@@ -1188,15 +1210,51 @@ int lcb_lm_keygen_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* seeds,
         CK(c, sampler_scratch(c, left));
         CK(c, timed(c, K_SAMPLER, [&] { return launch_sampler(left, c->stream); }));
         uint16_t* o_sk = d_sk_ntt ? d_sk_ntt + start * 2 * l * D_ : nullptr;
-        uint16_t* o_vk = d_vk_ntt ? d_vk_ntt + start * 2 * D_ : nullptr;
+        uint16_t* o_vk = d_vk_ntt ? d_vk_ntt + start * 2 * D_ : vk_scratch;
         int16_t* o_vkc = d_vk_coef ? d_vk_coef + start * 2 * D_ : nullptr;
         CK(c, timed(c, K_MATVEC, [&] {
             return c->generic ? g_launch_matvec(c->gen, skc, cnt * 2, o_sk, o_vk, o_vkc, c->stream)
                               : launch_matvec(c->ring, skc, cnt * 2, o_sk, o_vk, o_vkc, c->stream);
         }));
+        if (d_skp)
+            CK(c, timed(c, K_PACK, [&] {
+                return launch_pack(c->ring, skc, cnt * 2 * l, pk->sk_bits, pk->sk_bias, d_skp + start * 2 * l * 32 * pk->sk_bits,
+                                   d_skr ? d_skr + start * 2 * l : nullptr, c->stream);
+            }));
+        if (d_vkp)
+            CK(c, timed(c, K_PACK, [&] {
+                return launch_pack(c->ring, vk_scratch, cnt * 2, pk->vk_bits, 0, d_vkp + start * 2 * 32 * pk->vk_bits, nullptr,
+                                   c->stream);
+            }));
     }
     CK(c, sg.finish());
     return LCB_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int lcb_lm_keygen_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* seeds, const int64_t* seed_off, int64_t n,
+                        int16_t* sk_coef, uint16_t* sk_ntt, uint16_t* vk_ntt, int16_t* vk_coef) {
+    LCB_RANGE();
+    if (!c || !sch || !seed_off || n < 0) return LCB_ERR_INVALID;
+    return keygen(c, sch, seeds, seed_off, n, sk_coef, sk_ntt, vk_ntt, vk_coef, nullptr, "lcb_lm_keygen_batch");
+}
+
+// lcb_lm_keygen_batch -> lcb_pack_batch (signing keys, coefficient form) and lcb_pack_batch (verification keys, bias 0), chunk
+// by chunk inside the keygen loop: the 16-bit keys never leave engine scratch.
+int lcb_lm_keygen_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* seeds, const int64_t* seed_off, int64_t n,
+                               int sk_bits, int sk_bias, uint8_t* sk_packed, uint8_t* sk_in_range, int vk_bits,
+                               uint8_t* vk_packed) {
+    LCB_RANGE();
+    if (!c || !sch || !seed_off || n < 0 || (!sk_packed && !vk_packed) || !wire_args_ok(sk_bits, sk_bias) ||
+        !wire_args_ok(vk_bits, 0))
+        return LCB_ERR_INVALID;
+    if (c->generic) return fail(c, LCB_ERR_INVALID, "the packed wire format is defined for d == 256, q < 2^16 contexts only");
+    if (n > ((int64_t)1 << 30)) return fail(c, LCB_ERR_INVALID, "more than 2^30 items in one keygen call");
+    const KeyPack pk{sk_bits, sk_bias, sk_packed, sk_packed ? sk_in_range : nullptr, vk_bits, vk_packed};
+    return keygen(c, sch, seeds, seed_off, n, nullptr, nullptr, nullptr, nullptr, &pk, "lcb_lm_keygen_packed_batch");
 }
 
 int lcb_challenge_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* chmsg, const int64_t* chmsg_off, int64_t n,
@@ -1484,33 +1542,18 @@ int lcb_adaptor_verify_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const uin
                          n, bd, wt, verdict);
 }
 
-// lcb_lm_sign_batch -> lcb_pack_batch in one call.  Fused route (11- or 13-bit rows, 16-byte aligned): k_sign writes the
-// packed rows and in_range flags itself.  Anything else signs into int16 scratch and packs it with k_pack, in chunks.
-int lcb_lm_sign_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const uint16_t* sk_ntt, const uint8_t* chmsg,
-                             const int64_t* chmsg_off, int64_t n, int sig_bits, int sig_bias, uint8_t* sig_packed,
-                             uint8_t* in_range) {
-    LCB_RANGE();
-    if (!c || !sch || !sk_ntt || !chmsg_off || !sig_packed || n < 0 || !wire_args_ok(sig_bits, sig_bias))
-        return LCB_ERR_INVALID;
-    if (c->generic) return fail(c, LCB_ERR_INVALID, "the packed wire format is defined for d == 256, q < 2^16 contexts only");
-    if (n == 0) return LCB_OK;
-    CK(c, cudaSetDevice(c->device));
+}  // extern "C"
+
+namespace {
+
+// The body of lcb_lm_sign_packed_batch over device buffers (d_range nullable): lcb_lm_sign_batch -> lcb_pack_batch.  Fused
+// route (11- or 13-bit rows, 16-byte aligned): k_sign writes the packed rows and in_range flags itself.  Anything else signs
+// into int16 scratch and packs it with k_pack, in chunks.
+int sign_packed(lcb_ctx* c, Staging& sg, const lcb_scheme* sch, const uint16_t* d_sk, const uint8_t* d_msg, const int64_t* d_off,
+                int64_t n, int sig_bits, int sig_bias, uint8_t* d_sigp, uint8_t* d_range) {
     const int l = c->l;
-    int64_t total = 0;
-    CK(c, last_offset(c, chmsg, chmsg_off, n, &total));
-    Staging sg(c);
-    const uint16_t* d_sk;
-    const uint8_t* d_msg;
-    const int64_t* d_off;
-    uint8_t *d_sigp, *d_range;
-    int16_t* d_pairs;
     const size_t row = (size_t)32 * sig_bits;
-    CK(c, sg.in(&d_sk, sk_ntt, (size_t)n * 2 * l * D, true));
-    CK(c, sg.in(&d_msg, chmsg, (size_t)total));
-    CK(c, sg.in(&d_off, chmsg_off, (size_t)n + 1));
-    CK(c, sg.out(&d_sigp, sig_packed, (size_t)n * l * row));
-    CK(c, sg.out(&d_range, in_range, (size_t)n * l));
-    if (reinterpret_cast<uintptr_t>(d_sigp) & 3u) return fail(c, LCB_ERR_INVALID, "packed buffer must be 4-byte aligned");
+    int16_t* d_pairs;
     CK(c, sg.alloc((void**)&d_pairs, (size_t)n * sch->ch_wt * 2 * sizeof(int16_t)));
     int st = run_challenge(c, sch, d_msg, d_off, n, d_pairs);
     if (st != LCB_OK) return st;
@@ -1534,6 +1577,101 @@ int lcb_lm_sign_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const uint16_t* 
                 return launch_pack(c->ring, d_sig, m * l, sig_bits, sig_bias, d_sigp + (size_t)first * l * row,
                                    d_range ? d_range + (size_t)first * l : nullptr, c->stream);
             }));
+        }
+    }
+    return LCB_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int lcb_lm_sign_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const uint16_t* sk_ntt, const uint8_t* chmsg,
+                             const int64_t* chmsg_off, int64_t n, int sig_bits, int sig_bias, uint8_t* sig_packed,
+                             uint8_t* in_range) {
+    LCB_RANGE();
+    if (!c || !sch || !sk_ntt || !chmsg_off || !sig_packed || n < 0 || !wire_args_ok(sig_bits, sig_bias))
+        return LCB_ERR_INVALID;
+    if (c->generic) return fail(c, LCB_ERR_INVALID, "the packed wire format is defined for d == 256, q < 2^16 contexts only");
+    if (n == 0) return LCB_OK;
+    CK(c, cudaSetDevice(c->device));
+    const int l = c->l;
+    int64_t total = 0;
+    CK(c, last_offset(c, chmsg, chmsg_off, n, &total));
+    Staging sg(c);
+    const uint16_t* d_sk;
+    const uint8_t* d_msg;
+    const int64_t* d_off;
+    uint8_t *d_sigp, *d_range;
+    const size_t row = (size_t)32 * sig_bits;
+    CK(c, sg.in(&d_sk, sk_ntt, (size_t)n * 2 * l * D, true));
+    CK(c, sg.in(&d_msg, chmsg, (size_t)total));
+    CK(c, sg.in(&d_off, chmsg_off, (size_t)n + 1));
+    CK(c, sg.out(&d_sigp, sig_packed, (size_t)n * l * row));
+    CK(c, sg.out(&d_range, in_range, (size_t)n * l));
+    if (reinterpret_cast<uintptr_t>(d_sigp) & 3u) return fail(c, LCB_ERR_INVALID, "packed buffer must be 4-byte aligned");
+    int st = sign_packed(c, sg, sch, d_sk, d_msg, d_off, n, sig_bits, sig_bias, d_sigp, d_range);
+    if (st != LCB_OK) return st;
+    CK(c, sg.finish());
+    return LCB_OK;
+}
+
+// unpack -> lcb_ntt_fwd_batch -> lcb_lm_sign_packed_batch in one call.  Fused route (sign_sk_fused_applies: 7- / 8-bit keys,
+// 11- / 13-bit signatures, monomial challenges; both packed buffers 16-byte aligned): k_sign_sk sums the rotations of the
+// packed coefficient-form rows directly.  Anything else unpacks and transforms the keys into bounded secret scratch, chunk
+// by chunk, and signs each chunk with the body of lcb_lm_sign_packed_batch.
+int lcb_lm_sign_packed_sk_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* sk_packed, int sk_bits, int sk_bias,
+                                const uint8_t* chmsg, const int64_t* chmsg_off, int64_t n, int sig_bits, int sig_bias,
+                                uint8_t* sig_packed, uint8_t* in_range) {
+    LCB_RANGE();
+    if (!c || !sch || !sk_packed || !chmsg_off || !sig_packed || n < 0 || !wire_args_ok(sk_bits, sk_bias) ||
+        !wire_args_ok(sig_bits, sig_bias))
+        return LCB_ERR_INVALID;
+    if (c->generic) return fail(c, LCB_ERR_INVALID, "the packed wire format is defined for d == 256, q < 2^16 contexts only");
+    if (n > ((int64_t)1 << 30)) return fail(c, LCB_ERR_INVALID, "more than 2^30 items in one sign call");
+    if (n == 0) return LCB_OK;
+    CK(c, cudaSetDevice(c->device));
+    const int l = c->l;
+    int64_t total = 0;
+    CK(c, last_offset(c, chmsg, chmsg_off, n, &total));
+    Staging sg(c);
+    const uint8_t *d_skp, *d_msg;
+    const int64_t* d_off;
+    uint8_t *d_sigp, *d_range;
+    const size_t sk_item = (size_t)2 * l * 32 * sk_bits, sig_item = (size_t)l * 32 * sig_bits;
+    CK(c, sg.in(&d_skp, sk_packed, (size_t)n * sk_item, true));
+    CK(c, sg.in(&d_msg, chmsg, (size_t)total));
+    CK(c, sg.in(&d_off, chmsg_off, (size_t)n + 1));
+    CK(c, sg.out(&d_sigp, sig_packed, (size_t)n * sig_item));
+    CK(c, sg.out(&d_range, in_range, (size_t)n * l));
+    if ((reinterpret_cast<uintptr_t>(d_skp) | reinterpret_cast<uintptr_t>(d_sigp)) & 3u)
+        return fail(c, LCB_ERR_INVALID, "packed buffers must be 4-byte aligned");
+    const bool aligned16 = ((reinterpret_cast<uintptr_t>(d_skp) | reinterpret_cast<uintptr_t>(d_sigp)) & 15u) == 0;
+    if (aligned16 && sign_sk_fused_applies(sk_bits, sig_bits, sch->ch_bd, sch->ch_wt)) {
+        int16_t* d_pairs;
+        CK(c, sg.alloc((void**)&d_pairs, (size_t)n * sch->ch_wt * 2 * sizeof(int16_t)));
+        int st = run_challenge(c, sch, d_msg, d_off, n, d_pairs);
+        if (st != LCB_OK) return st;
+        CK(c, timed(c, K_SIGN, [&] {
+            return launch_sign_sk_packed(c->ring, d_skp, sk_bits, sk_bias, d_pairs, sch->ch_bd, sch->ch_wt, n, sig_bits, sig_bias,
+                                         d_sigp, d_range, c->stream);
+        }));
+    } else {
+        const int64_t chunk = n < kWireChunkPoly / (2 * l) ? n : kWireChunkPoly / (2 * l);
+        int16_t* d_coef;
+        uint16_t* d_ntt;
+        CK(c, sg.alloc((void**)&d_coef, (size_t)chunk * 2 * l * D * sizeof(int16_t), true));
+        CK(c, sg.alloc((void**)&d_ntt, (size_t)chunk * 2 * l * D * sizeof(uint16_t), true));
+        for (int64_t first = 0; first < n; first += chunk) {
+            const int64_t m = n - first < chunk ? n - first : chunk;
+            CK(c, timed(c, K_UNPACK, [&] {
+                return launch_unpack(c->ring, d_skp + (size_t)first * sk_item, m * 2 * l, sk_bits, sk_bias, d_coef, c->stream);
+            }));
+            CK(c, timed(c, K_NTT_FWD, [&] { return launch_ntt_fwd(c->ring, d_coef, m * 2 * l, d_ntt, c->stream); }));
+            Staging chunk_sg(c);                 // the chunk's challenge pairs and int16 scratch go back to the pool after it
+            int st = sign_packed(c, chunk_sg, sch, d_ntt, d_msg, d_off + first, m, sig_bits, sig_bias,
+                                 d_sigp + (size_t)first * sig_item, d_range ? d_range + (size_t)first * l : nullptr);
+            if (st != LCB_OK) return st;
         }
     }
     CK(c, sg.finish());

@@ -155,6 +155,18 @@ cudaError_t launch_verify_packed(const RingCtx& c, const uint8_t* sig_packed, in
 // sig_packed uint8[n][l][32*sig_bits], in_range (nullable) uint8[n][l], as launch_sign -> launch_pack would write them
 cudaError_t launch_sign_packed(const RingCtx& c, const uint16_t* sk_ntt, const int16_t* ch_pairs, int ch_wt, int64_t n,
                                int sig_bits, int sig_bias, uint8_t* sig_packed, uint8_t* in_range, cudaStream_t st);
+// sign from packed coefficient-form signing keys straight into the wire format (sign_sk.cu): sk_packed uint8[n][2][l][32*sk_bits]
+// (bias sk_bias) -> sig_packed uint8[n][l][32*sig_bits], in_range (nullable) uint8[n][l], exactly as unpack -> launch_ntt_fwd ->
+// launch_sign_packed would write them.  Rows of both packed buffers 16-byte aligned; cudaErrorNotSupported unless
+// sign_sk_fused_applies.
+inline bool sign_sk_fused_applies(int sk_bits, int sig_bits, int ch_bd, int ch_wt) {
+    // bytes as fields (sk_bits <= 8), monomial challenges (ch_bd = 1): the 16-bit lane sums of the kernel stay below
+    // ch_wt * 255 < 2^16 for every ch_wt <= d
+    return (sk_bits == 7 || sk_bits == 8) && (sig_bits == 11 || sig_bits == 13) && ch_bd == 1 && ch_wt >= 1 && ch_wt <= D;
+}
+cudaError_t launch_sign_sk_packed(const RingCtx& c, const uint8_t* sk_packed, int sk_bits, int sk_bias,
+                                  const int16_t* ch_pairs, int ch_bd, int ch_wt, int64_t n, int sig_bits, int sig_bias,
+                                  uint8_t* sig_packed, uint8_t* in_range, cudaStream_t st);
 cudaError_t launch_vec_addsub(const RingCtx& c, const int16_t* a, const int16_t* b, int64_t nelem, int sub,
                               int16_t* out, cudaStream_t st);
 cudaError_t launch_agg_partial(const RingCtx& c, const int16_t* sigs, const int16_t* ag_pairs, int64_t count,

@@ -359,6 +359,34 @@ class Engine(object):
                                                     sig_bits, sig_bias, _addr(sig), _addr(ok)))
         return (sig, ok) if want_range else sig
 
+    def lm_keygen_packed(self, sch: LcbScheme, seeds, sk_bits: int, sk_bias: int, vk_bits: int, want_sk: bool = True,
+                         want_sk_range: bool = False, want_vk: bool = True, device: bool = False):
+        """lm_keygen straight into the wire format: -> (sk_packed uint8[n, 2, l, 32*sk_bits] (coefficient form, bias sk_bias),
+        sk_in_range uint8[n, 2, l], vk_packed uint8[n, 2, 32*vk_bits] (NTT form, bias 0)), each None unless wanted; exactly
+        pack(sk_coef, sk_bits, sk_bias) and pack(vk_ntt, vk_bits, 0) of lm_keygen."""
+        blob, off = self._rag(seeds)
+        n = self._count(off)
+        sk = self._out((n, 2, self.l, self.d * sk_bits // 8), np.uint8, device) if want_sk else None
+        ok = self._out((n, 2, self.l), np.uint8, device) if want_sk and want_sk_range else None
+        vk = self._out((n, 2, self.d * vk_bits // 8), np.uint8, device) if want_vk else None
+        self._ck(self._lib.lcb_lm_keygen_packed_batch(self._ctx, byref(sch), _addr(blob), _addr(off), n, sk_bits, sk_bias,
+                                                      _addr(sk), _addr(ok), vk_bits, _addr(vk)))
+        return sk, ok, vk
+
+    def lm_sign_packed_sk(self, sch: LcbScheme, sk_packed, sk_bits: int, sk_bias: int, chmsgs, sig_bits: int,
+                          sig_bias: int, device: bool = False, want_range: bool = False):
+        """lm_sign from packed coefficient-form signing keys uint8[n, 2, l, 32*sk_bits] into the wire format: -> uint8[n, l,
+        32*sig_bits] (and in_range uint8[n, l] when want_range), exactly lm_sign_packed(ntt_fwd(unpack(sk_packed, sk_bits,
+        sk_bias)), ...)."""
+        blob, off = self._rag(chmsgs)
+        n = self._count(off)
+        _want(sk_packed, 'sk_packed', np.uint8, (n, 2, self.l, self.d * sk_bits // 8))
+        sig = self._out((n, self.l, self.d * sig_bits // 8), np.uint8, device)
+        ok = self._out((n, self.l), np.uint8, device) if want_range else None
+        self._ck(self._lib.lcb_lm_sign_packed_sk_batch(self._ctx, byref(sch), _addr(sk_packed), sk_bits, sk_bias, _addr(blob),
+                                                       _addr(off), n, sig_bits, sig_bias, _addr(sig), _addr(ok)))
+        return (sig, ok) if want_range else sig
+
     def adaptor_verify_packed(self, sch: LcbScheme, vk_packed, vk_bits: int, chmsgs, sig_packed, sig_bits: int,
                               sig_bias: int, st_packed, st_bits: int, bd: int, wt: int, device: bool = False, out=None):
         """lm_verify(..., st_ntt=...) from packed keys uint8[n, 2, 32*vk_bits], signatures uint8[n, l, 32*sig_bits] and

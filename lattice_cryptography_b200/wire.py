@@ -15,6 +15,11 @@ module is therefore OPT-IN and does not change what the drop-in API computes:
   `presign_batch_packed` (presignatures in `sig_bits(pp, 'pvf_bd')` bits, bias `pvf_bd`: 11 / 13), `preverify_batch_packed`,
   `adapt_batch_packed` (adaptor signatures in `sig_bits(pp)` bits, bias `vf_bd`: 11 / 13), `adaptor_verify_batch_packed`
   (statements packed like keys with `pack_keys`) and `extract_batch_packed` (int16 witnesses);
+* signing keys in COEFFICIENT form, `signing_key_bits(pp)` bits (7 at secpar 128, 8 at 256) with bias sk_bd - 5,824 /
+  11,776 bytes per key instead of 13,312 / 23,552 for the uint16 NTT form: `pack_signing_keys` / `unpack_signing_keys`,
+  `keygen_batch_packed` (packed signing and verification keys straight from the seeds) and `sign_batch_packed_sk` /
+  `presign_batch_packed_sk` (packed signatures / presignatures straight from packed signing keys), so that the one-time
+  signature lifecycle runs on packed records only;
 * `aggregate_batch_packed` / `aggregate_verify_batch_packed`: the batched BKLM calls of `bklm_one_time_agg_sigs`
   (many independent aggregates, sorted signatures / keys of group g at agg_off[g] .. agg_off[g+1]) from packed
   signatures and keys, with packed aggregates.  An aggregate is encoded as a signature with the aggregate bound:
@@ -50,6 +55,11 @@ def key_bits(pp: Dict[str, Any]) -> int:
     return ceil(log2(pp['scheme_parameters'].lp.modulus))
 
 
+def signing_key_bits(pp: Dict[str, Any]) -> int:
+    """Bits per signing-key coefficient: the sampler draws them from [-sk_bd, sk_bd]."""
+    return max(1, ceil(log2(2 * pp['sk_bd'] + 1)))
+
+
 def _engine(pp):
     sp = pp['scheme_parameters']
     return engine_for(sp.lp, sp.secpar)
@@ -72,6 +82,48 @@ def pack_keys(pp, vk_ntt, device: bool = False):
 
 def unpack_keys(pp, packed, device: bool = False):
     return _engine(pp).unpack(packed, key_bits(pp), 0, dtype=np.uint16, device=device)
+
+
+def pack_signing_keys(pp, sk_coef, device: bool = False):
+    """sk_coef int16[..., 2, l, 256] (coefficient form, as `lm_keygen` returns it) -> (uint8[..., 2, l, 32*signing_key_bits],
+    in_range uint8[..., 2, l]), bias sk_bd."""
+    return _engine(pp).pack(sk_coef, signing_key_bits(pp), pp['sk_bd'], device=device, want_range=True)
+
+
+def unpack_signing_keys(pp, packed, device: bool = False):
+    return _engine(pp).unpack(packed, signing_key_bits(pp), pp['sk_bd'], dtype=np.int16, device=device)
+
+
+def keygen_batch_packed(pp, seeds, device: bool = False):
+    """Packed keys straight from the seeds (the seed forms of `lm_one_time_sigs.keygen_batch`, including the output of
+    `random_seed_batch`): -> (sk_packed uint8[N, 2, l, 32*signing_key_bits(pp)], vk_packed uint8[N, 2, 32*key_bits(pp)]),
+    exactly `pack_signing_keys` / `pack_keys` of the keys `keygen_batch` makes; no 16-bit key leaves the engine."""
+    from .lm_one_time_sigs import SecretSeed, _ctx
+    eng, sch = _ctx(pp)
+    if isinstance(seeds, tuple) and len(seeds) == 2 and not isinstance(seeds[0], (str, SecretSeed)):
+        strs = seeds                # already (byte blob, int64 offsets), e.g. from random_seed_batch
+    else:
+        strs = [s.seed if isinstance(s, SecretSeed) else s for s in seeds]
+    sk, _, vk = eng.lm_keygen_packed(sch, strs, signing_key_bits(pp), pp['sk_bd'], key_bits(pp), device=device)
+    return sk, vk
+
+
+def sign_batch_packed_sk(pp, sk_packed, chmsgs, device: bool = False):
+    """LM signatures from packed signing keys straight into the wire format: -> (uint8[N, l, 32*sig_bits], in_range
+    uint8[N, l]), bias vf_bd; exactly `sign_batch_packed(pp, ntt_fwd(unpack_signing_keys(pp, sk_packed)), chmsgs)`."""
+    from .lm_one_time_sigs import _ctx
+    eng, sch = _ctx(pp)
+    return eng.lm_sign_packed_sk(sch, sk_packed, signing_key_bits(pp), pp['sk_bd'], chmsgs, sig_bits(pp), pp['vf_bd'],
+                                 device=device, want_range=True)
+
+
+def presign_batch_packed_sk(pp, sk_packed, chmsgs, device: bool = False):
+    """Adaptor presignatures (adaptor `pp`) from packed signing keys -> (uint8[N, l, 32*sig_bits(pp, 'pvf_bd')], in_range
+    uint8[N, l]), bias pvf_bd."""
+    from .adaptor_sigs import _ctx
+    eng, sch = _ctx(pp)
+    return eng.lm_sign_packed_sk(sch, sk_packed, signing_key_bits(pp), pp['sk_bd'], chmsgs, sig_bits(pp, 'pvf_bd'),
+                                 pp['pvf_bd'], device=device, want_range=True)
 
 
 def verify_batch_packed(pp, vk_packed, chmsgs, sig_packed, device: bool = False):
