@@ -316,6 +316,48 @@ int lcb_vec_sub_batch(lcb_ctx* ctx, const int16_t* a, const int16_t* b, int64_t 
 int lcb_adaptor_witness_verify_batch(lcb_ctx* ctx, const int16_t* wit_coef, const uint16_t* st_ntt, int64_t n,
                                      int bd, int wt, uint8_t* verdict);
 
+/* ---- Adaptor witnesses on the packed wire format.  A packed witness is uint8[l][32*wit_bits]: coefficient-form rows packed
+ * like a signature (x = centred coefficient, bias wit_bias).  Shipped packings: generated witnesses in
+ * ceil(log2(2 wit_bd + 1)) = 2 bits with bias wit_bd = 1 (832 / 1,472 bytes per witness at secpar 128 / 256 instead of
+ * 6,656 / 11,776 as int16); extracted witnesses in ceil(log2(2 ext_wit_bd + 1)) bits with bias ext_wit_bd (12 / 14 bits),
+ * lossless for every witness witness_verify can accept.  Statements are packed like key halves (NTT form, bias 0, 14 / 16
+ * bits).  Same rules as the packed calls above (bits 1..16, biases 0..32767, packed buffers 4-byte aligned, d == 256 and
+ * q < 2^16 only, host or device buffers).  Each result is exactly that of the composition named, for any input bytes.
+ * Witnesses are secret: host-resident ones are staged through engine scratch that is cleared afterwards. */
+
+/* witgen (adaptor_sigs.py:80-101,140-151) into packed records: exactly lcb_adaptor_witgen_batch(wit_coef, st_ntt) ->
+ * lcb_pack_batch(wit_coef, wit_bits, wit_bias, wit_in_range) and lcb_pack_batch(st_ntt, st_bits, 0).  wit_packed
+ * uint8[n][l][32*wit_bits], wit_in_range uint8[n][l], st_packed uint8[n][32*st_bits]; each may be NULL, but not both
+ * wit_packed and st_packed.  The 16-bit witnesses stay in engine scratch, chunk by chunk.  Needs key_ch
+ * (LCB_ERR_NO_KEY_CH); at most 2^30 items. */
+int lcb_adaptor_witgen_packed_batch(lcb_ctx* ctx, const lcb_scheme* sch, const uint8_t* seeds, const int64_t* seed_off,
+                                    int64_t n, int wit_bits, int wit_bias, uint8_t* wit_packed, uint8_t* wit_in_range,
+                                    int st_bits, uint8_t* st_packed);
+
+/* witness_verify (adaptor_sigs.py:229-237) on packed witnesses and statements: exactly lcb_unpack_batch of both (statements
+ * with bias 0, as uint16) -> lcb_adaptor_witness_verify_batch.  Needs key_ch; at most 2^30 items.  Witness / statement
+ * widths 2 / 14 and 12 / 14 (secpar 128), 2 / 16 and 14 / 16 (secpar 256), with statements at the key width ceil(log2 q),
+ * 16-byte aligned witness rows and 16-bit statement rows, are read by the verify kernel directly; anything else is
+ * unpacked into engine scratch first. */
+int lcb_adaptor_witness_verify_packed_batch(lcb_ctx* ctx, const uint8_t* wit_packed, int wit_bits, int wit_bias,
+                                            const uint8_t* st_packed, int st_bits, int64_t n, int bd, int wt,
+                                            uint8_t* verdict);
+
+/* adapt (adaptor_sigs.py:220-221) with a packed witness: exactly unpack both -> lcb_vec_add_batch(presig, wit) ->
+ * lcb_pack_batch(sig_bits, sig_bias, in_range).  presig_packed uint8[npoly][32*presig_bits], wit_packed
+ * uint8[npoly][32*wit_bits], sig_packed uint8[npoly][32*sig_bits], in_range (nullable) uint8[npoly].  One kernel pass at
+ * every width. */
+int lcb_adaptor_adapt_packed_wit_batch(lcb_ctx* ctx, const uint8_t* presig_packed, int presig_bits, int presig_bias,
+                                       const uint8_t* wit_packed, int wit_bits, int wit_bias, int64_t npoly, int sig_bits,
+                                       int sig_bias, uint8_t* sig_packed, uint8_t* in_range);
+
+/* extract (adaptor_sigs.py:224-226) into packed witnesses: exactly unpack both -> lcb_vec_sub_batch(sig, presig) ->
+ * lcb_pack_batch(wit_bits, wit_bias, in_range).  wit_packed uint8[npoly][32*wit_bits], in_range (nullable) uint8[npoly].
+ * At 2 bits a valid witness that is not the genuine one does not fit: in_range says so. */
+int lcb_adaptor_extract_packed_wit_batch(lcb_ctx* ctx, const uint8_t* sig_packed, int sig_bits, int sig_bias,
+                                         const uint8_t* presig_packed, int presig_bits, int presig_bias, int64_t npoly,
+                                         int wit_bits, int wit_bias, uint8_t* wit_packed, uint8_t* in_range);
+
 /* ---- Multi-device context: ONE call shards a HOST-resident batch over several GPUs of the box (SURVEY.md 8(b), 8(e)).
  * devices[] lists CUDA ordinals (an ordinal may repeat: two contexts on one GPU).  Independent units (keygen, sign,
  * verify) are split into contiguous ranges by the reference's distribute_tasks rule (lm_one_time_sigs.py:194-215: the
@@ -357,7 +399,8 @@ int64_t lcb_launch_count(const lcb_ctx* ctx);
  * agg_partial agg_finish aggv_partial aggv_finish pack unpack, and for the batch calls group_ids agg_coefs_seg
  * agg_partial_seg aggv_partial_seg aggv_residues aggv_limits, and agg_finish_pack for packed aggregates.  The fused packed
  * routes are counted under the kernel they extend: packed signing (from NTT-form or packed signing keys) under sign, packed
- * verification under verify.
+ * verification (including witness verification on packed witnesses) under verify, adapt / extract on packed witnesses
+ * under vec_addsub.
  * lcb_profile_read synchronises the stream. */
 int lcb_profile_enable(lcb_ctx* ctx, int on);
 int lcb_profile_reset(lcb_ctx* ctx);

@@ -76,6 +76,13 @@ PROTOTYPES = {
                                                 c_int64, c_int, c_int, _P]),
     'lcb_adaptor_adapt_packed_batch': (c_int, [c_void_p, _P, c_int, c_int, _P, c_int64, c_int, c_int, _P, _P]),
     'lcb_adaptor_extract_packed_batch': (c_int, [c_void_p, _P, c_int, c_int, _P, c_int, c_int, c_int64, _P]),
+    'lcb_adaptor_witgen_packed_batch': (c_int, [c_void_p, POINTER(LcbScheme), _P, _P, c_int64, c_int, c_int, _P, _P, c_int,
+                                                _P]),
+    'lcb_adaptor_witness_verify_packed_batch': (c_int, [c_void_p, _P, c_int, c_int, _P, c_int, c_int64, c_int, c_int, _P]),
+    'lcb_adaptor_adapt_packed_wit_batch': (c_int, [c_void_p, _P, c_int, c_int, _P, c_int, c_int, c_int64, c_int, c_int, _P,
+                                                   _P]),
+    'lcb_adaptor_extract_packed_wit_batch': (c_int, [c_void_p, _P, c_int, c_int, _P, c_int, c_int, c_int64, c_int, c_int,
+                                                     _P, _P]),
     'lcb_bklm_agg_coefs': (c_int, [c_void_p, POINTER(LcbScheme), _P, c_int64, c_int64, c_int64, _P]),
     'lcb_bklm_aggregate_partial': (c_int, [c_void_p, POINTER(LcbScheme), _P, _P, _P, c_int64, c_int64, c_int64, _P]),
     'lcb_bklm_aggregate_finish': (c_int, [c_void_p, _P, _P]),

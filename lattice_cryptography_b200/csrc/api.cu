@@ -2017,11 +2017,24 @@ int lcb_bklm_aggregate_verify_packed_batch(lcb_ctx* c, const lcb_scheme* sch, co
     return LCB_OK;
 }
 
-int lcb_adaptor_witgen_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* seeds, const int64_t* seed_off,
-                             int64_t n, int16_t* wit_coef, uint16_t* st_ntt, int16_t* st_coef) {
-    LCB_RANGE();
-    if (!c || !sch || !seed_off || n < 0) return LCB_ERR_INVALID;
-    if (!c->has_key_ch) return fail(c, LCB_ERR_NO_KEY_CH, "lcb_adaptor_witgen_batch before lcb_set_key_ch");
+}  // extern "C"
+
+namespace {
+
+// Packed outputs of lcb_adaptor_witgen_packed_batch: each chunk's int16 witnesses and uint16 NTT-form statements are packed
+// before the next chunk reuses the scratch.  wit / st may each be null.
+struct WitPack {
+    int wit_bits, wit_bias;
+    uint8_t *wit, *wit_range;
+    int st_bits;
+    uint8_t* st;
+};
+
+// The body of lcb_adaptor_witgen_batch (wp == null: one pass over the whole batch) and of lcb_adaptor_witgen_packed_batch
+// (wp set, every unpacked output null: chunks of kWireChunkPoly / l witnesses in secret scratch).
+int witgen(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* seeds, const int64_t* seed_off, int64_t n, int16_t* wit_coef,
+           uint16_t* st_ntt, int16_t* st_coef, const WitPack* wp, const char* name) {
+    if (!c->has_key_ch) return fail(c, LCB_ERR_NO_KEY_CH, std::string(name) + " before lcb_set_key_ch");
     if (n == 0) return LCB_OK;
     CK(c, cudaSetDevice(c->device));
     const int l = c->l;
@@ -2031,27 +2044,85 @@ int lcb_adaptor_witgen_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* s
     int64_t total = 0;
     CK(c, last_offset(c, seeds, seed_off, n, &total));
     Staging sg(c);
+    const uint8_t* d_seeds;
+    const int64_t* d_off;
     int16_t *d_wit, *d_st_coef;
     uint16_t* d_st_ntt;
-    CK(c, sg.in(&a.msgs, seeds, (size_t)total));
-    CK(c, sg.in(&a.off, seed_off, (size_t)n + 1));
+    CK(c, sg.in(&d_seeds, seeds, (size_t)total));
+    CK(c, sg.in(&d_off, seed_off, (size_t)n + 1));
     const size_t D_ = (size_t)c->d * ew(c);
     CK(c, sg.out(&d_wit, wit_coef, (size_t)n * l * D_, true));
     CK(c, sg.out(&d_st_ntt, st_ntt, (size_t)n * D_));
     CK(c, sg.out(&d_st_coef, st_coef, (size_t)n * D_));
-    if (!d_wit) CK(c, sg.alloc((void**)&d_wit, (size_t)n * l * D_ * sizeof(int16_t), true));
-    if (sch->wit_wt < c->d) CK(c, cudaMemsetAsync(d_wit, 0, (size_t)n * l * D_ * sizeof(int16_t), c->stream));
-    a.n = n;
-    a.out_dense = d_wit;
-    a.dense_stride = (int64_t)l * c->d;
-    CK(c, sampler_scratch(c, a));
-    CK(c, timed(c, K_SAMPLER, [&] { return launch_sampler(a, c->stream); }));
-    CK(c, timed(c, K_MATVEC, [&] {
-        return c->generic ? g_launch_matvec(c->gen, d_wit, n, nullptr, d_st_ntt, d_st_coef, c->stream)
-                          : launch_matvec(c->ring, d_wit, n, nullptr, d_st_ntt, d_st_coef, c->stream);
-    }));
+    uint8_t *d_witp = nullptr, *d_witr = nullptr, *d_stp = nullptr;
+    if (wp) {
+        CK(c, sg.out(&d_witp, wp->wit, (size_t)n * l * 32 * wp->wit_bits, true));
+        CK(c, sg.out(&d_witr, wp->wit_range, (size_t)n * l));
+        CK(c, sg.out(&d_stp, wp->st, (size_t)n * 32 * wp->st_bits));
+        if ((reinterpret_cast<uintptr_t>(d_witp) | reinterpret_cast<uintptr_t>(d_stp)) & 3u)
+            return fail(c, LCB_ERR_INVALID, "packed buffers must be 4-byte aligned");
+    }
+    const int64_t chunk = wp && n > kWireChunkPoly / l ? kWireChunkPoly / l : n;
+    int16_t* scratch = nullptr;
+    if (!d_wit) CK(c, sg.alloc((void**)&scratch, (size_t)chunk * l * D_ * sizeof(int16_t), true));
+    uint16_t* st_scratch = nullptr;                                // NTT-form statements of a chunk, to be packed
+    if (d_stp) CK(c, sg.alloc((void**)&st_scratch, (size_t)chunk * D_ * sizeof(uint16_t)));
+    for (int64_t start = 0; start < n; start += chunk) {
+        const int64_t cnt = (n - start < chunk) ? n - start : chunk;
+        int16_t* wit = d_wit ? d_wit + start * l * D_ : scratch;
+        // the sampler writes only the wit_wt nonzero coefficients of each polynomial
+        if (sch->wit_wt < c->d) CK(c, cudaMemsetAsync(wit, 0, (size_t)cnt * l * D_ * sizeof(int16_t), c->stream));
+        a.msgs = d_seeds;
+        a.off = d_off + start;
+        a.n = cnt;
+        a.out_dense = wit;
+        a.dense_stride = (int64_t)l * c->d;
+        CK(c, sampler_scratch(c, a));
+        CK(c, timed(c, K_SAMPLER, [&] { return launch_sampler(a, c->stream); }));
+        uint16_t* o_st = d_st_ntt ? d_st_ntt + start * D_ : st_scratch;
+        int16_t* o_stc = d_st_coef ? d_st_coef + start * D_ : nullptr;
+        CK(c, timed(c, K_MATVEC, [&] {
+            return c->generic ? g_launch_matvec(c->gen, wit, cnt, nullptr, o_st, o_stc, c->stream)
+                              : launch_matvec(c->ring, wit, cnt, nullptr, o_st, o_stc, c->stream);
+        }));
+        if (d_witp)
+            CK(c, timed(c, K_PACK, [&] {
+                return launch_pack(c->ring, wit, cnt * l, wp->wit_bits, wp->wit_bias, d_witp + start * l * 32 * wp->wit_bits,
+                                   d_witr ? d_witr + start * l : nullptr, c->stream);
+            }));
+        if (d_stp)
+            CK(c, timed(c, K_PACK, [&] {
+                return launch_pack(c->ring, st_scratch, cnt, wp->st_bits, 0, d_stp + start * 32 * wp->st_bits, nullptr, c->stream);
+            }));
+    }
     CK(c, sg.finish());
     return LCB_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int lcb_adaptor_witgen_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* seeds, const int64_t* seed_off,
+                             int64_t n, int16_t* wit_coef, uint16_t* st_ntt, int16_t* st_coef) {
+    LCB_RANGE();
+    if (!c || !sch || !seed_off || n < 0) return LCB_ERR_INVALID;
+    return witgen(c, sch, seeds, seed_off, n, wit_coef, st_ntt, st_coef, nullptr, "lcb_adaptor_witgen_batch");
+}
+
+// lcb_adaptor_witgen_batch -> lcb_pack_batch (witnesses, coefficient form) and lcb_pack_batch (statements, NTT form, bias 0),
+// chunk by chunk inside the witgen loop: the 16-bit witnesses never leave engine scratch.
+int lcb_adaptor_witgen_packed_batch(lcb_ctx* c, const lcb_scheme* sch, const uint8_t* seeds, const int64_t* seed_off,
+                                    int64_t n, int wit_bits, int wit_bias, uint8_t* wit_packed, uint8_t* wit_in_range,
+                                    int st_bits, uint8_t* st_packed) {
+    LCB_RANGE();
+    if (!c || !sch || !seed_off || n < 0 || (!wit_packed && !st_packed) || !wire_args_ok(wit_bits, wit_bias) ||
+        !wire_args_ok(st_bits, 0))
+        return LCB_ERR_INVALID;
+    if (c->generic) return fail(c, LCB_ERR_INVALID, "the packed wire format is defined for d == 256, q < 2^16 contexts only");
+    if (n > ((int64_t)1 << 30)) return fail(c, LCB_ERR_INVALID, "more than 2^30 items in one witgen call");
+    const WitPack wp{wit_bits, wit_bias, wit_packed, wit_packed ? wit_in_range : nullptr, st_bits, st_packed};
+    return witgen(c, sch, seeds, seed_off, n, nullptr, nullptr, nullptr, &wp, "lcb_adaptor_witgen_packed_batch");
 }
 
 static int vec_addsub(lcb_ctx* c, const int16_t* a, const int16_t* b, int64_t npoly, int sub, int16_t* out) {
@@ -2179,6 +2250,112 @@ int lcb_adaptor_witness_verify_batch(lcb_ctx* c, const int16_t* wit_coef, const 
                           : launch_verify(c->ring, d_wit, nullptr, nullptr, 0, d_st, nullptr, n, bd > 32767 ? 32767 : bd, wt, d_verdict,
                                           c->stream);
     }));
+    CK(c, sg.finish());
+    return LCB_OK;
+}
+
+// adapt / extract with packed witnesses: unpack both -> k_vec_addsub -> pack in ONE kernel (k_addsub_packed, every width),
+// counted under vec_addsub.  a = presig (adapt) or sig (extract), b = wit (adapt) or presig (extract).
+static int addsub_packed(lcb_ctx* c, const uint8_t* a, int a_bits, int a_bias, bool a_secret, const uint8_t* b, int b_bits,
+                         int b_bias, bool b_secret, int sub, int64_t npoly, int bits, int bias, bool out_secret, uint8_t* out,
+                         uint8_t* in_range) {
+    if (!c || !a || !b || !out || npoly < 0 || !wire_args_ok(a_bits, a_bias) || !wire_args_ok(b_bits, b_bias) ||
+        !wire_args_ok(bits, bias))
+        return LCB_ERR_INVALID;
+    if (c->generic) return fail(c, LCB_ERR_INVALID, "the packed wire format is defined for d == 256, q < 2^16 contexts only");
+    if (npoly == 0) return LCB_OK;
+    CK(c, cudaSetDevice(c->device));
+    Staging sg(c);
+    const uint8_t *d_a, *d_b;
+    uint8_t *d_out, *d_range;
+    CK(c, sg.in(&d_a, a, (size_t)npoly * 32 * a_bits, a_secret));
+    CK(c, sg.in(&d_b, b, (size_t)npoly * 32 * b_bits, b_secret));
+    CK(c, sg.out(&d_out, out, (size_t)npoly * 32 * bits, out_secret));
+    CK(c, sg.out(&d_range, in_range, (size_t)npoly));
+    if ((reinterpret_cast<uintptr_t>(d_a) | reinterpret_cast<uintptr_t>(d_b) | reinterpret_cast<uintptr_t>(d_out)) & 3u)
+        return fail(c, LCB_ERR_INVALID, "packed buffers must be 4-byte aligned");
+    CK(c, timed(c, K_ADDSUB, [&] {
+        return launch_addsub_packed(c->ring, d_a, a_bits, a_bias, d_b, b_bits, b_bias, sub, npoly, bits, bias, d_out, d_range,
+                                    c->stream);
+    }));
+    CK(c, sg.finish());
+    return LCB_OK;
+}
+
+int lcb_adaptor_adapt_packed_wit_batch(lcb_ctx* c, const uint8_t* presig_packed, int presig_bits, int presig_bias,
+                                       const uint8_t* wit_packed, int wit_bits, int wit_bias, int64_t npoly, int sig_bits,
+                                       int sig_bias, uint8_t* sig_packed, uint8_t* in_range) {
+    LCB_RANGE();
+    return addsub_packed(c, presig_packed, presig_bits, presig_bias, false, wit_packed, wit_bits, wit_bias, true, 0, npoly,
+                         sig_bits, sig_bias, false, sig_packed, in_range);
+}
+
+int lcb_adaptor_extract_packed_wit_batch(lcb_ctx* c, const uint8_t* sig_packed, int sig_bits, int sig_bias,
+                                         const uint8_t* presig_packed, int presig_bits, int presig_bias, int64_t npoly,
+                                         int wit_bits, int wit_bias, uint8_t* wit_packed, uint8_t* in_range) {
+    LCB_RANGE();
+    return addsub_packed(c, sig_packed, sig_bits, sig_bias, false, presig_packed, presig_bits, presig_bias, false, 1, npoly,
+                         wit_bits, wit_bias, true, wit_packed, in_range);
+}
+
+// unpack witnesses and statements -> lcb_adaptor_witness_verify_batch.  Fused route (witness / statement widths 2 / 14,
+// 12 / 14, 2 / 16, 14 / 16 with statements at the key width ceil(log2 q); 16-byte aligned witness rows and 16-bit
+// statement rows): k_verify reads both packed rows directly.  Anything else unpacks chunks of kWireChunkPoly / l items into
+// secret scratch and runs the witness-verify launch on them.
+int lcb_adaptor_witness_verify_packed_batch(lcb_ctx* c, const uint8_t* wit_packed, int wit_bits, int wit_bias,
+                                            const uint8_t* st_packed, int st_bits, int64_t n, int bd, int wt,
+                                            uint8_t* verdict) {
+    LCB_RANGE();
+    if (!c || !wit_packed || !st_packed || !verdict || n < 0 || bd < 0 || wt < 0 || !wire_args_ok(wit_bits, wit_bias) ||
+        !wire_args_ok(st_bits, 0))
+        return LCB_ERR_INVALID;
+    if (c->generic) return fail(c, LCB_ERR_INVALID, "the packed wire format is defined for d == 256, q < 2^16 contexts only");
+    if (!c->has_key_ch) return fail(c, LCB_ERR_NO_KEY_CH, "lcb_adaptor_witness_verify_packed_batch before lcb_set_key_ch");
+    if (n > ((int64_t)1 << 30)) return fail(c, LCB_ERR_INVALID, "more than 2^30 items in one verify call");
+    if (n == 0) return LCB_OK;
+    CK(c, cudaSetDevice(c->device));
+    const int l = c->l;
+    Staging sg(c);
+    const uint8_t *d_witp, *d_stp;
+    uint8_t* d_verdict;
+    const size_t wit_item = (size_t)l * 32 * wit_bits;
+    CK(c, sg.in(&d_witp, wit_packed, (size_t)n * wit_item, true));
+    CK(c, sg.in(&d_stp, st_packed, (size_t)n * 32 * st_bits));
+    CK(c, sg.out(&d_verdict, verdict, (size_t)n));
+    if ((reinterpret_cast<uintptr_t>(d_witp) | reinterpret_cast<uintptr_t>(d_stp)) & 3u)
+        return fail(c, LCB_ERR_INVALID, "packed buffers must be 4-byte aligned");
+    const int bd_k = bd > 32767 ? 32767 : bd;
+    // k_verify stages witness rows with 16-byte cp.async and reads 16-bit statement rows with 128-bit loads: a caller-owned
+    // device buffer that is only 4-byte aligned takes the composed route
+    const bool aligned16 = (reinterpret_cast<uintptr_t>(d_witp) & 15u) == 0 &&
+                           (st_bits == 14 || (reinterpret_cast<uintptr_t>(d_stp) & 15u) == 0);
+    const bool fused = aligned16 && st_bits == ceil_log2(c->q) &&
+                       ((st_bits == 14 && (wit_bits == 2 || wit_bits == 12)) || (st_bits == 16 && (wit_bits == 2 || wit_bits == 14)));
+    if (fused) {
+        CK(c, timed(c, K_VERIFY, [&] {
+            return launch_verify_rhs_packed(c->ring, d_witp, wit_bits, wit_bias, reinterpret_cast<const uint16_t*>(d_stp), n,
+                                            bd_k, wt, d_verdict, c->stream, st_bits);
+        }));
+    } else {
+        const int64_t chunk = n < kWireChunkPoly / l ? n : kWireChunkPoly / l;
+        int16_t* d_wit;
+        uint16_t* d_st;
+        CK(c, sg.alloc((void**)&d_wit, (size_t)chunk * l * D * sizeof(int16_t), true));
+        CK(c, sg.alloc((void**)&d_st, (size_t)chunk * D * sizeof(uint16_t)));
+        for (int64_t first = 0; first < n; first += chunk) {
+            const int64_t m = n - first < chunk ? n - first : chunk;
+            CK(c, timed(c, K_UNPACK, [&] {
+                return launch_unpack(c->ring, d_witp + (size_t)first * wit_item, m * l, wit_bits, wit_bias, d_wit, c->stream);
+            }));
+            CK(c, timed(c, K_UNPACK, [&] {
+                return launch_unpack(c->ring, d_stp + (size_t)first * 32 * st_bits, m, st_bits, 0, d_st, c->stream);
+            }));
+            CK(c, timed(c, K_VERIFY, [&] {
+                return launch_verify(c->ring, d_wit, nullptr, nullptr, 0, d_st, nullptr, m, bd_k, wt, d_verdict + first,
+                                     c->stream);
+            }));
+        }
+    }
     CK(c, sg.finish());
     return LCB_OK;
 }

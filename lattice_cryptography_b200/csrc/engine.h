@@ -192,14 +192,21 @@ cudaError_t launch_aggv_limits(const RingCtx& c, const int64_t* agg_off, int64_t
                                uint8_t* verdict, cudaStream_t st);
 cudaError_t launch_aggv_limits_packed(const RingCtx& c, const int64_t* agg_off, int64_t n_agg, const uint8_t* ag_packed, int bits,
                                       int bias, int64_t ag_cap, uint8_t* verdict, cudaStream_t st);
+// witness-verify form of k_verify on packed rows (bias `bias`): (bits, rhs_bits) = (12 | 14, 16), (2, 16), (2 | 12, 14); a
+// 14-bit rhs_only is a packed row uint8[n][32*14] (bias 0).  cudaErrorNotSupported otherwise.
 cudaError_t launch_verify_rhs_packed(const RingCtx& c, const uint8_t* vec_packed, int bits, int bias, const uint16_t* rhs_only,
-                                     int64_t n, int bd, int wt, uint8_t* verdict, cudaStream_t st);
+                                     int64_t n, int bd, int wt, uint8_t* verdict, cudaStream_t st, int rhs_bits = 16);
 
 // wire format (wire.cu): `bits`-bit little-endian packing of (x + bias) mod 2^16, 32*bits bytes per polynomial
 cudaError_t launch_pack(const RingCtx& c, const void* in, int64_t npoly, int bits, int bias, uint8_t* out,
                         uint8_t* in_range, cudaStream_t st);
 cudaError_t launch_unpack(const RingCtx& c, const uint8_t* in, int64_t npoly, int bits, int bias, void* out,
                           cudaStream_t st);
+// unpack both operands -> k_vec_addsub (a + b, or a - b when sub) -> k_pack in one pass, any widths 1..16 (adaptor adapt /
+// extract on the wire format): a, b, out uint8[npoly][32*bits of each], in_range (nullable) uint8[npoly]
+cudaError_t launch_addsub_packed(const RingCtx& c, const uint8_t* a, int a_bits, int a_bias, const uint8_t* b, int b_bits,
+                                 int b_bias, int sub, int64_t npoly, int bits, int bias, uint8_t* out, uint8_t* in_range,
+                                 cudaStream_t st);
 // k_agg_finish + k_pack in one pass: BKLM partial sums int32[npoly][256] -> packed aggregates and in_range flags
 cudaError_t launch_agg_finish_pack(const RingCtx& c, const int32_t* partial, int64_t npoly, int bits, int bias, uint8_t* out,
                                    uint8_t* in_range, cudaStream_t st);

@@ -546,7 +546,8 @@ __device__ __forceinline__ void load_u14x16(uint32_t (&r)[EPT], const uint32_t* 
 // The packed rows ride through the same cp.async stage buffers and are expanded on the way into registers.
 // ST_BITS: 0 = extra_rhs holds uint16 statement slots; 14 = 14-bit packed statements (bias 0, 7 words per lane, read as
 // the key halves are).  A 16-bit packed statement has the bytes of a uint16 row and takes ST_BITS = 0.
-template <bool CHECK_WT, int SIG_BITS, int VK_BITS, int ST_BITS = 0>
+// RHS_BITS: the same for rhs_only in the witness-verify form (14 = packed adaptor statements).
+template <bool CHECK_WT, int SIG_BITS, int VK_BITS, int ST_BITS = 0, int RHS_BITS = 0>
 __global__ void __launch_bounds__(VBS, VERIFY_BLOCKS) k_verify(ModQ m, StageConst sc, StageConstF scf, const NttTables* __restrict__ tab,
                                                 const uint32_t* __restrict__ a_hat_g, int l,
                                                 const int16_t* __restrict__ vec_coef,
@@ -697,6 +698,8 @@ __global__ void __launch_bounds__(VBS, VERIFY_BLOCKS) k_verify(ModQ m, StageCons
             }
 #pragma unroll
             for (int k = 0; k < EPT; ++k) acc[k] += (uint64_t)(c[k] - FP_BIAS) * (m.cq2 - vl[k]);
+        } else if (RHS_BITS == 14) {
+            load_u14x16(rhs, reinterpret_cast<const uint32_t*>(rhs_only) + item * 112 + 7 * h.lane);
         } else {
             load_u16x16(rhs, rhs_only + item * D + 16 * h.lane);
         }
@@ -1425,14 +1428,14 @@ cudaError_t launch_sign_packed(const RingCtx& c, const uint16_t* sk_ntt, const i
     return cudaErrorNotSupported;
 }
 
-template <int SIG_BITS, int VK_BITS, int ST_BITS = 0>
+template <int SIG_BITS, int VK_BITS, int ST_BITS = 0, int RHS_BITS = 0>
 cudaError_t launch_verify_t(const RingCtx& c, const void* vec, const void* vk, const int16_t* ch_pairs, int ch_wt,
                             const uint16_t* rhs_only, const uint16_t* extra_rhs, int64_t n, int bd, int wt, int sig_bias,
                             uint8_t* verdict, cudaStream_t st) {
     if (n <= 0) return cudaSuccess;
     if (n > ((int64_t)1 << 30)) return cudaErrorInvalidValue;      // 32-bit item indices inside the kernel
     size_t smem = verify_smem(c.l);
-    auto kern = wt < D ? k_verify<true, SIG_BITS, VK_BITS, ST_BITS> : k_verify<false, SIG_BITS, VK_BITS, ST_BITS>;
+    auto kern = wt < D ? k_verify<true, SIG_BITS, VK_BITS, ST_BITS, RHS_BITS> : k_verify<false, SIG_BITS, VK_BITS, ST_BITS, RHS_BITS>;
     cudaError_t e = allow_smem(kern, smem);
     if (e != cudaSuccess) return e;
     unsigned grid = persistent_grid(n, VHWB, c.num_sms, resident_blocks(kern, VBS, smem));
@@ -1465,15 +1468,22 @@ cudaError_t launch_verify_packed(const RingCtx& c, const uint8_t* sig_packed, in
     return cudaErrorNotSupported;
 }
 
-// Witness-verify form on packed rows of BKLM aggregates: the two widths of the shipped parameter sets (12 / 14 bits);
-// the decoder of k_verify is the one of the signature widths, and at even widths every value starts in the same
-// half-word phase.
+// Witness-verify form on packed rows: BKLM aggregates (12 / 14 bits, uint16 right-hand sides) and adaptor witnesses with
+// packed statements (witnesses 2 bits, or 12 / 14 as extracted; statements 14 or 16 bits, bias 0).  The decoder of
+// k_verify is the one of the signature widths, and at even widths every value starts in the same half-word phase.  A
+// 16-bit statement row has the bytes of a uint16 row; 14-bit rows are read by k_verify<..., RHS_BITS = 14>.
 cudaError_t launch_verify_rhs_packed(const RingCtx& c, const uint8_t* vec_packed, int bits, int bias, const uint16_t* rhs_only,
-                                     int64_t n, int bd, int wt, uint8_t* verdict, cudaStream_t st) {
-    if (bits == 12)
+                                     int64_t n, int bd, int wt, uint8_t* verdict, cudaStream_t st, int rhs_bits) {
+    if (rhs_bits == 16 && bits == 12)
         return launch_verify_t<12, 0>(c, vec_packed, nullptr, nullptr, 0, rhs_only, nullptr, n, bd, wt, bias, verdict, st);
-    if (bits == 14)
+    if (rhs_bits == 16 && bits == 14)
         return launch_verify_t<14, 0>(c, vec_packed, nullptr, nullptr, 0, rhs_only, nullptr, n, bd, wt, bias, verdict, st);
+    if (rhs_bits == 16 && bits == 2)
+        return launch_verify_t<2, 0>(c, vec_packed, nullptr, nullptr, 0, rhs_only, nullptr, n, bd, wt, bias, verdict, st);
+    if (rhs_bits == 14 && bits == 2)
+        return launch_verify_t<2, 0, 0, 14>(c, vec_packed, nullptr, nullptr, 0, rhs_only, nullptr, n, bd, wt, bias, verdict, st);
+    if (rhs_bits == 14 && bits == 12)
+        return launch_verify_t<12, 0, 0, 14>(c, vec_packed, nullptr, nullptr, 0, rhs_only, nullptr, n, bd, wt, bias, verdict, st);
     return cudaErrorNotSupported;
 }
 

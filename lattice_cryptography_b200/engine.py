@@ -427,6 +427,34 @@ class Engine(object):
                                                             _addr(wit)))
         return wit
 
+    def adapt_packed_wit(self, presig_packed, presig_bits: int, presig_bias: int, wit_packed, wit_bits: int, wit_bias: int,
+                         sig_bits: int, sig_bias: int, device: bool = False, want_range: bool = False):
+        """presig uint8[..., 32*presig_bits] + packed wit uint8[..., 32*wit_bits] -> uint8[..., 32*sig_bits] (and in_range
+        uint8[...]), exactly pack(vec_add(unpack(presig), unpack(wit)))."""
+        npoly = _lead(presig_packed, 'presig_packed', np.uint8, self.d * presig_bits // 8)
+        lead = tuple(presig_packed.shape[:-1])
+        _want(wit_packed, 'wit_packed', np.uint8, lead + (self.d * wit_bits // 8,))
+        sig = self._out(lead + (self.d * sig_bits // 8,), np.uint8, device)
+        ok = self._out(lead, np.uint8, device) if want_range else None
+        self._ck(self._lib.lcb_adaptor_adapt_packed_wit_batch(self._ctx, _addr(presig_packed), presig_bits, presig_bias,
+                                                              _addr(wit_packed), wit_bits, wit_bias, npoly, sig_bits, sig_bias,
+                                                              _addr(sig), _addr(ok)))
+        return (sig, ok) if want_range else sig
+
+    def extract_packed_wit(self, sig_packed, sig_bits: int, sig_bias: int, presig_packed, presig_bits: int,
+                           presig_bias: int, wit_bits: int, wit_bias: int, device: bool = False, want_range: bool = False):
+        """-> packed witnesses uint8[..., 32*wit_bits] (and in_range uint8[...]), exactly
+        pack(vec_sub(unpack(sig), unpack(presig)), wit_bits, wit_bias)."""
+        npoly = _lead(sig_packed, 'sig_packed', np.uint8, self.d * sig_bits // 8)
+        lead = tuple(sig_packed.shape[:-1])
+        _want(presig_packed, 'presig_packed', np.uint8, lead + (self.d * presig_bits // 8,))
+        wit = self._out(lead + (self.d * wit_bits // 8,), np.uint8, device)
+        ok = self._out(lead, np.uint8, device) if want_range else None
+        self._ck(self._lib.lcb_adaptor_extract_packed_wit_batch(self._ctx, _addr(sig_packed), sig_bits, sig_bias,
+                                                                _addr(presig_packed), presig_bits, presig_bias, npoly,
+                                                                wit_bits, wit_bias, _addr(wit), _addr(ok)))
+        return (wit, ok) if want_range else wit
+
     # ------------------------------------------------------------------ BKLM aggregation
     def agg_coefs(self, sch: LcbScheme, agmsg, first: int, count: int, device: bool = False):
         if isinstance(agmsg, (str, bytes, bytearray)):
@@ -559,6 +587,20 @@ class Engine(object):
                                                     _addr(st_ntt), _addr(st_coef)))
         return wit, st_ntt, st_coef
 
+    def witgen_packed(self, sch: LcbScheme, seeds, wit_bits: int, wit_bias: int, st_bits: int, want_wit: bool = True,
+                      want_wit_range: bool = False, want_st: bool = True, device: bool = False):
+        """witgen straight into the wire format: -> (wit_packed uint8[n, l, 32*wit_bits] (coefficient form, bias wit_bias),
+        wit_in_range uint8[n, l], st_packed uint8[n, 32*st_bits] (NTT form, bias 0)), each None unless wanted; exactly
+        pack(wit, wit_bits, wit_bias) and pack(st_ntt, st_bits, 0) of witgen."""
+        blob, off = self._rag(seeds)
+        n = self._count(off)
+        wit = self._out((n, self.l, self.d * wit_bits // 8), np.uint8, device) if want_wit else None
+        ok = self._out((n, self.l), np.uint8, device) if want_wit and want_wit_range else None
+        st = self._out((n, self.d * st_bits // 8), np.uint8, device) if want_st else None
+        self._ck(self._lib.lcb_adaptor_witgen_packed_batch(self._ctx, byref(sch), _addr(blob), _addr(off), n, wit_bits,
+                                                           wit_bias, _addr(wit), _addr(ok), st_bits, _addr(st)))
+        return wit, ok, st
+
     def vec_add(self, a, b, device: bool = False):
         npoly = _lead(a, 'a', self.ct, self.d)
         _want(b, 'b', self.ct, tuple(a.shape))
@@ -580,6 +622,18 @@ class Engine(object):
         verdict = self._out((n,), np.uint8, device)
         self._ck(self._lib.lcb_adaptor_witness_verify_batch(self._ctx, _addr(wit_coef), _addr(st_ntt), n, bd, wt,
                                                             _addr(verdict)))
+        return verdict
+
+    def witness_verify_packed(self, wit_packed, wit_bits: int, wit_bias: int, st_packed, st_bits: int, bd: int, wt: int,
+                              device: bool = False):
+        """witness_verify from packed witnesses uint8[n, l, 32*wit_bits] and statements uint8[n, 32*st_bits] (bias 0):
+        exactly witness_verify(unpack(wit), unpack(st))."""
+        n = int(wit_packed.shape[0]) if len(getattr(wit_packed, 'shape', ())) else 0
+        _want(wit_packed, 'wit_packed', np.uint8, (n, self.l, self.d * wit_bits // 8))
+        _want(st_packed, 'st_packed', np.uint8, (n, self.d * st_bits // 8))
+        verdict = self._out((n,), np.uint8, device)
+        self._ck(self._lib.lcb_adaptor_witness_verify_packed_batch(self._ctx, _addr(wit_packed), wit_bits, wit_bias,
+                                                                   _addr(st_packed), st_bits, n, bd, wt, _addr(verdict)))
         return verdict
 
 

@@ -15,6 +15,13 @@ module is therefore OPT-IN and does not change what the drop-in API computes:
   `presign_batch_packed` (presignatures in `sig_bits(pp, 'pvf_bd')` bits, bias `pvf_bd`: 11 / 13), `preverify_batch_packed`,
   `adapt_batch_packed` (adaptor signatures in `sig_bits(pp)` bits, bias `vf_bd`: 11 / 13), `adaptor_verify_batch_packed`
   (statements packed like keys with `pack_keys`) and `extract_batch_packed` (int16 witnesses);
+* adaptor witnesses on packed records, so that the adaptor lifecycle runs on packed records only.  A witness is packed
+  like a signature with a witness bound: `pack_witnesses` / `unpack_witnesses` (`bound_key='wit_bd'`: 2 bits, bias 1 -
+  832 / 1,472 bytes per witness instead of 6,656 / 11,776; `'ext_wit_bd'`: 12 / 14 bits, lossless for every witness
+  that witness verification can accept); `witgen_batch_packed` (packed witnesses and statements straight from the
+  seeds), `adapt_batch_packed_wit` (adapt with a packed witness), `extract_batch_packed_wit` (packed witnesses out of
+  extract, with in_range flags: a 2-bit extraction cannot hold a valid witness that is not the genuine one) and
+  `witness_verify_batch_packed` (bound ext_wit_bd, weight ext_wit_wt);
 * signing keys in COEFFICIENT form, `signing_key_bits(pp)` bits (7 at secpar 128, 8 at 256) with bias sk_bd - 5,824 /
   11,776 bytes per key instead of 13,312 / 23,552 for the uint16 NTT form: `pack_signing_keys` / `unpack_signing_keys`,
   `keygen_batch_packed` (packed signing and verification keys straight from the seeds) and `sign_batch_packed_sk` /
@@ -182,6 +189,60 @@ def adaptor_verify_batch_packed(pp, vk_packed, chmsgs, st_packed, sig_packed, de
     eng, sch = _ctx(pp)
     return eng.adaptor_verify_packed(sch, vk_packed, key_bits(pp), chmsgs, sig_packed, sig_bits(pp), pp['vf_bd'], st_packed,
                                      key_bits(pp), pp['vf_bd'], pp['vf_wt'], device=device)
+
+
+def pack_witnesses(pp, wit_coef, device: bool = False, bound_key: str = 'wit_bd'):
+    """Adaptor witnesses int16[..., l, 256] -> (uint8[..., l, 32*sig_bits(pp, bound_key)], in_range uint8[..., l]), bias
+    pp[bound_key]."""
+    return _engine(pp).pack(wit_coef, sig_bits(pp, bound_key), pp[bound_key], device=device, want_range=True)
+
+
+def unpack_witnesses(pp, packed, device: bool = False, bound_key: str = 'wit_bd'):
+    return _engine(pp).unpack(packed, sig_bits(pp, bound_key), pp[bound_key], dtype=np.int16, device=device)
+
+
+def witgen_batch_packed(pp, seeds, device: bool = False):
+    """Adaptor witnesses and statements straight from the seeds (the seed forms of `adaptor_sigs.witgen_batch`) ->
+    (wit_packed uint8[N, l, 32*sig_bits(pp, 'wit_bd')], st_packed uint8[N, 32*key_bits(pp)]), exactly
+    `pack_witnesses` / `pack_keys` of what `witgen_batch` makes; no 16-bit witness leaves the engine."""
+    from .adaptor_sigs import SecretSeed, _ctx
+    eng, sch = _ctx(pp)
+    if isinstance(seeds, tuple) and len(seeds) == 2 and not isinstance(seeds[0], (str, SecretSeed)):
+        strs = seeds                # already (byte blob, int64 offsets)
+    else:
+        strs = [s.seed if isinstance(s, SecretSeed) else s for s in seeds]
+    wit, _, st = eng.witgen_packed(sch, strs, sig_bits(pp, 'wit_bd'), pp['wit_bd'], key_bits(pp), device=device)
+    return wit, st
+
+
+def adapt_batch_packed_wit(pp, presig_packed, wit_packed, device: bool = False):
+    """Packed presignatures + packed witnesses (`pack_witnesses`) -> (adaptor signatures uint8[N, l, 32*sig_bits(pp)],
+    in_range uint8[N, l]), bias vf_bd; exactly `adapt_batch_packed(pp, presig_packed, unpack_witnesses(pp, wit_packed))`."""
+    from .adaptor_sigs import _ctx
+    eng, _ = _ctx(pp)
+    return eng.adapt_packed_wit(presig_packed, sig_bits(pp, 'pvf_bd'), pp['pvf_bd'], wit_packed, sig_bits(pp, 'wit_bd'),
+                                pp['wit_bd'], sig_bits(pp), pp['vf_bd'], device=device, want_range=True)
+
+
+def extract_batch_packed_wit(pp, presig_packed, sig_packed, device: bool = False, bound_key: str = 'ext_wit_bd'):
+    """Packed witnesses = signature - presignature, from the two packed records -> (uint8[N, l, 32*sig_bits(pp,
+    bound_key)], in_range uint8[N, l]), bias pp[bound_key].  The default width holds every witness that
+    `witness_verify_batch_packed` can accept; at bound_key='wit_bd' a valid witness that is not the genuine one reads
+    in_range 0."""
+    from .adaptor_sigs import _ctx
+    eng, _ = _ctx(pp)
+    return eng.extract_packed_wit(sig_packed, sig_bits(pp), pp['vf_bd'], presig_packed, sig_bits(pp, 'pvf_bd'),
+                                  pp['pvf_bd'], sig_bits(pp, bound_key), pp[bound_key], device=device, want_range=True)
+
+
+def witness_verify_batch_packed(pp, wit_packed, st_packed, device: bool = False, bound_key: str = 'wit_bd'):
+    """N witness verdicts (uint8) from packed witnesses uint8[N, l, 32*sig_bits(pp, bound_key)] (bias pp[bound_key]) and
+    packed statements uint8[N, 32*key_bits(pp)], with bound ext_wit_bd and weight ext_wit_wt as
+    `adaptor_sigs.witness_verify_batch`."""
+    from .adaptor_sigs import _ctx
+    eng, _ = _ctx(pp)
+    return eng.witness_verify_packed(wit_packed, sig_bits(pp, bound_key), pp[bound_key], st_packed, key_bits(pp),
+                                     pp['ext_wit_bd'], pp['ext_wit_wt'], device=device)
 
 
 def aggregate_batch_packed(pp, agg_off, sig_packed, agmsgs, device: bool = False):
