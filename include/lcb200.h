@@ -358,6 +358,40 @@ int lcb_adaptor_extract_packed_wit_batch(lcb_ctx* ctx, const uint8_t* sig_packed
                                          const uint8_t* presig_packed, int presig_bits, int presig_bias, int64_t npoly,
                                          int wit_bits, int wit_bias, uint8_t* wit_packed, uint8_t* in_range);
 
+/* ---- Content-mode hash inputs from packed keys and raw messages (d = 256, q < 2^16 for lcb_content_str_batch).
+ * In content mode (the Python layer's one_time_keys.set_content_str(True)) str() / repr() of a verification key or a
+ * public statement is
+ *     '<' + name + ' ' + SHAKE256(name || le16(secpar) || its int16 coefficient rows, little-endian).hexdigest(16) + '>'
+ * with name OneTimeVerificationKey (rows: left, then right) or OneTimePublicStatement (one row): always 57 bytes.  Every
+ * challenge message (lm_one_time_sigs.py:148, adaptor_sigs.py:176) and every BKLM aggregation message
+ * (bklm_one_time_agg_sigs.py:65) contains such strings, so these three calls build the chmsg / agmsg inputs of every sign,
+ * verify, adaptor and BKLM entry point above from packed keys without a host round trip. */
+#define LCB_CONTENT_VK 0   /* packed uint8[n][2][32*bits]: left half, then right half */
+#define LCB_CONTENT_ST 1   /* packed uint8[n][32*bits]                               */
+/* Row i of out uint8[n][57] is exactly repr() of the key (kind LCB_CONTENT_VK) or statement (LCB_CONTENT_ST) whose NTT
+ * form is lcb_unpack_batch(packed, bits, bias 0): unpack -> lcb_ntt_inv_batch -> the digest above over the centred int16
+ * coefficients -> '<name ' + 32 lowercase hex digits + '>', for any input bytes (slots v >= q included); secpar is the
+ * context's.  bits = 16 is the byte layout of a plain uint16 NTT array.  bits 1..16, packed buffer 4-byte aligned, at most
+ * 2^30 items, n == 0 returns LCB_OK; LCB_ERR_INVALID with "the packed wire format is defined for d == 256, q < 2^16
+ * contexts only" on any other context. */
+int lcb_content_str_batch(lcb_ctx* ctx, int kind, const uint8_t* packed, int bits, int64_t n, uint8_t* out);
+/* Challenge messages: item i of out is [st_str_i + ', '] + vk_str_i + ', ' + msg_i (st_str nullable: without it the LM
+ * challenge str(otvk) + ', ' + msg, with it the adaptor challenge str(st) + ', ' + str(otvk) + ', ' + msg), at
+ * out[out_off[i] .. out_off[i+1]), out_off[0] = 0.  st_str / vk_str uint8[n][57] (lcb_content_str_batch rows), msg ragged
+ * (item i = msg[msg_off[i] .. msg_off[i+1]); msg_off[0] need not be 0).  The caller sizes out as
+ * msg_off[n] - msg_off[0] + 59 n bytes, or + 118 n with st_str; out_off int64[n+1].  Pure byte assembly: valid on every
+ * context.  At most 2^30 items. */
+int lcb_challenge_inputs_batch(lcb_ctx* ctx, const uint8_t* st_str, const uint8_t* vk_str, const uint8_t* msg,
+                               const int64_t* msg_off, int64_t n, uint8_t* out, int64_t* out_off);
+/* BKLM aggregation messages: group g (its sorted items agg_off[g] .. agg_off[g+1], agg_off as in
+ * lcb_bklm_aggregate_batch) is '[' + ', '.join("(" + vk_str + ", '" + msg + "')") + ']' over its items - str(list(zip(keys,
+ * msgs))) for bitstring messages, '[]' for an empty group - at agmsg[agmsg_off[g] .. agmsg_off[g+1]), agmsg_off[0] = 0.
+ * vk_str_sorted uint8[total][57], msg_sorted ragged as in lcb_challenge_inputs_batch (msg_off int64[total+1]); message
+ * bytes are written as given.  Group g takes 2 + sum(63 + len_i) + 2 max(count_g - 1, 0) bytes; agmsg_off int64[n_agg+1].
+ * At most 2^30 items.  The challenge messages of the same items come from lcb_challenge_inputs_batch on the same arrays. */
+int lcb_aggregation_inputs_batch(lcb_ctx* ctx, const int64_t* agg_off, int64_t n_agg, const uint8_t* vk_str_sorted,
+                                 const uint8_t* msg_sorted, const int64_t* msg_off, uint8_t* agmsg, int64_t* agmsg_off);
+
 /* ---- Multi-device context: ONE call shards a HOST-resident batch over several GPUs of the box (SURVEY.md 8(b), 8(e)).
  * devices[] lists CUDA ordinals (an ordinal may repeat: two contexts on one GPU).  Independent units (keygen, sign,
  * verify) are split into contiguous ranges by the reference's distribute_tasks rule (lm_one_time_sigs.py:194-215: the
@@ -400,7 +434,8 @@ int64_t lcb_launch_count(const lcb_ctx* ctx);
  * agg_partial_seg aggv_partial_seg aggv_residues aggv_limits, and agg_finish_pack for packed aggregates.  The fused packed
  * routes are counted under the kernel they extend: packed signing (from NTT-form or packed signing keys) under sign, packed
  * verification (including witness verification on packed witnesses) under verify, adapt / extract on packed witnesses
- * under vec_addsub.
+ * under vec_addsub.  The content-mode hash inputs: content_str (after unpack and ntt_inv), challenge_inputs, and
+ * group_ids + aggregation_inputs.
  * lcb_profile_read synchronises the stream. */
 int lcb_profile_enable(lcb_ctx* ctx, int on);
 int lcb_profile_reset(lcb_ctx* ctx);

@@ -20,6 +20,9 @@ LCB_ERR_NO_DEVICE = -3
 LCB_ERR_NO_KEY_CH = -4
 LCB_ERR_OOM = -5
 
+LCB_CONTENT_VK = 0
+LCB_CONTENT_ST = 1
+
 
 class LcbError(RuntimeError):
     def __init__(self, status: int, what: str):
@@ -83,6 +86,9 @@ PROTOTYPES = {
                                                    _P]),
     'lcb_adaptor_extract_packed_wit_batch': (c_int, [c_void_p, _P, c_int, c_int, _P, c_int, c_int, c_int64, c_int, c_int,
                                                      _P, _P]),
+    'lcb_content_str_batch': (c_int, [c_void_p, c_int, _P, c_int, c_int64, _P]),
+    'lcb_challenge_inputs_batch': (c_int, [c_void_p, _P, _P, _P, _P, c_int64, _P, _P]),
+    'lcb_aggregation_inputs_batch': (c_int, [c_void_p, _P, c_int64, _P, _P, _P, _P, _P]),
     'lcb_bklm_agg_coefs': (c_int, [c_void_p, POINTER(LcbScheme), _P, c_int64, c_int64, c_int64, _P]),
     'lcb_bklm_aggregate_partial': (c_int, [c_void_p, POINTER(LcbScheme), _P, _P, _P, c_int64, c_int64, c_int64, _P]),
     'lcb_bklm_aggregate_finish': (c_int, [c_void_p, _P, _P]),

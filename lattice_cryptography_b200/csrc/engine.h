@@ -211,4 +211,17 @@ cudaError_t launch_addsub_packed(const RingCtx& c, const uint8_t* a, int a_bits,
 cudaError_t launch_agg_finish_pack(const RingCtx& c, const int32_t* partial, int64_t npoly, int bits, int bias, uint8_t* out,
                                    uint8_t* in_range, cudaStream_t st);
 
+// content-mode hash inputs (content.cu).  coef int16[n][rows][256] (rows 1 or 2) -> out uint8[n][57]: '<' + name + ' ' +
+// SHAKE256(prefix || rows).hexdigest(16) + '>'; prefix = name || le16(secpar) (24 bytes), head = '<' + name + ' '
+cudaError_t launch_content_str(const RingCtx& c, const int16_t* coef, int64_t n, int rows, const uint8_t (&prefix)[24],
+                               const uint8_t (&head)[24], uint8_t* out, cudaStream_t st);
+// out / out_off (lcb_challenge_inputs_batch); msg_i = msg[msg_off[i] - shift .. msg_off[i+1] - shift); out_len bytes of out
+cudaError_t launch_challenge_inputs(const RingCtx& c, const uint8_t* st_str, const uint8_t* vk_str, const uint8_t* msg,
+                                    int64_t shift, const int64_t* msg_off, int64_t n, int64_t out_len, uint8_t* out,
+                                    int64_t* out_off, cudaStream_t st);
+// agmsg of lcb_aggregation_inputs_batch at the group offsets ag_off[n_agg+1] the caller computed; gid from launch_group_ids
+cudaError_t launch_aggregation_inputs(const RingCtx& c, const int64_t* agg_off, const int64_t* ag_off, int64_t n_agg,
+                                      const int32_t* gid, int64_t total, const uint8_t* vk_str, const uint8_t* msg,
+                                      int64_t shift, const int64_t* msg_off, int64_t out_len, uint8_t* out, cudaStream_t st);
+
 }  // namespace lcb

@@ -455,6 +455,60 @@ class Engine(object):
                                                                 wit_bits, wit_bias, _addr(wit), _addr(ok)))
         return (wit, ok) if want_range else wit
 
+    # ------------------------------------------------------------------ content-mode hash inputs
+    _CONTENT_KINDS = {'vk': (_ffi.LCB_CONTENT_VK, 2), 'st': (_ffi.LCB_CONTENT_ST, 1)}
+
+    def content_str(self, kind: str, packed, bits: int, device: bool = False):
+        """Content-mode repr() of packed NTT-form keys (kind 'vk': uint8[n, 2, 32*bits]) or statements ('st': uint8[n,
+        32*bits]), bias 0 -> uint8[n, 57] (include/lcb200.h, lcb_content_str_batch).  At bits = 16 a plain uint16 NTT array
+        (uint16[n, 2, 256] / uint16[n, 256]) is accepted as it is."""
+        if kind not in self._CONTENT_KINDS:
+            raise ValueError(f"kind must be 'vk' or 'st', not {kind!r}")
+        code, rows = self._CONTENT_KINDS[kind]
+        if not isinstance(bits, int) or not 1 <= bits <= 16:
+            raise ValueError(f'bits must be in 1..16, not {bits}')
+        n = int(packed.shape[0]) if len(getattr(packed, 'shape', ())) else 0
+        lead = (n, 2) if rows == 2 else (n,)
+        if bits == 16 and (packed.dtype == np.uint16 or str(packed.dtype) == 'torch.uint16'):
+            _want(packed, 'packed', np.uint16, lead + (self.d,))
+        else:
+            _want(packed, 'packed', np.uint8, lead + (self.d * bits // 8,))
+        out = self._out((n, 57), np.uint8, device)
+        self._ck(self._lib.lcb_content_str_batch(self._ctx, code, _addr(packed), bits, n, _addr(out)))
+        return out
+
+    def challenge_inputs(self, vk_str, msgs, st_str=None, device: bool = False):
+        """Challenge messages [st_str_i + ', '] + vk_str_i + ', ' + msg_i from 57-byte content strings uint8[n, 57] and
+        ragged messages -> (blob uint8[total], offsets int64[n+1]), the chmsgs form every sign / verify call takes."""
+        mblob, moff = self._rag(msgs)
+        n = self._count(moff)
+        _want(vk_str, 'vk_str', np.uint8, (n, 57))
+        if st_str is not None:
+            _want(st_str, 'st_str', np.uint8, (n, 57))
+        total = int(moff[-1]) - int(moff[0]) + n * (118 if st_str is not None else 59)
+        out = self._out((total,), np.uint8, device)
+        out_off = self._out((n + 1,), np.int64, device)
+        self._ck(self._lib.lcb_challenge_inputs_batch(self._ctx, _addr(st_str), _addr(vk_str), _addr(mblob), _addr(moff), n,
+                                                      _addr(out), _addr(out_off)))
+        return out, out_off
+
+    def aggregation_inputs(self, agg_off, vk_str_sorted, msgs_sorted, device: bool = False):
+        """BKLM aggregation messages '[' + ', '.join("(" + vk_str + ", '" + msg + "')") + ']' of many groups (sorted items
+        agg_off[g] .. agg_off[g+1]) -> (blob uint8[total], offsets int64[n_agg+1])."""
+        mblob, moff = self._rag(msgs_sorted)
+        total = self._count(moff)
+        _want(vk_str_sorted, 'vk_str_sorted', np.uint8, (total, 57))
+        n_agg = self._groups(agg_off, total)
+        ha = agg_off.cpu().numpy() if _is_torch(agg_off) else agg_off
+        hm = moff.cpu().numpy() if _is_torch(moff) else moff
+        counts = np.diff(ha)
+        size = int((2 + 63 * counts + (hm[ha[1:]] - hm[ha[:-1]]) + 2 * np.maximum(counts - 1, 0)).sum()) if n_agg else 0
+        out = self._out((size,), np.uint8, device)
+        out_off = self._out((n_agg + 1,), np.int64, device)
+        self._ck(self._lib.lcb_aggregation_inputs_batch(self._ctx, _addr(agg_off), n_agg, _addr(vk_str_sorted), _addr(mblob),
+                                                        _addr(moff), _addr(out), _addr(out_off)))
+        return out, out_off
+
     # ------------------------------------------------------------------ BKLM aggregation
     def agg_coefs(self, sch: LcbScheme, agmsg, first: int, count: int, device: bool = False):
         if isinstance(agmsg, (str, bytes, bytearray)):

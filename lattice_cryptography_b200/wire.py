@@ -38,7 +38,11 @@ module is therefore OPT-IN and does not change what the drop-in API computes:
 
 * `one_time_keys.set_content_str(True)` (re-exported here as `set_content_str`): `str()` / `repr()` of
   verification keys and public statements become content digests, so signatures verify against pickled or
-  re-created key objects (changes the challenge bytes, hence every signature; off by default).
+  re-created key objects (changes the challenge bytes, hence every signature; off by default).  In that mode a packed
+  key received over the wire identifies its key, and the hash inputs are built on the GPU from packed records and raw
+  messages: `content_strs` (the 57-byte repr() of packed keys or statements), `challenge_inputs` (the `chmsgs` of every
+  packed sign / verify / adaptor call) and `aggregation_inputs` (the per-group sort order, sorted `chmsgs` and
+  aggregation messages of the packed BKLM calls).  The drop-in `challenge_messages` keeps building them on the host.
 
 Bit layout (include/lcb200.h): value i of a polynomial at bit offset i*bits, least significant bit first.
 """
@@ -263,6 +267,54 @@ def aggregate_verify_batch_packed(pp, agg_off, vk_packed, chmsgs_sorted, agmsgs,
     return eng.aggregate_verify_packed_batch(sch, agg_off, vk_packed, key_bits(pp), chmsgs_sorted,
                                              _batch_messages(pp, list(agmsgs)), ag_packed, sig_bits(pp, 'avf_bd'),
                                              pp['avf_bd'], pp['ag_cap'], pp['avf_bd'], pp['avf_wt'], device=device)
+
+
+def content_strs(pp, packed, kind: str = 'vk', device: bool = False):
+    """Content-mode repr() of packed keys uint8[N, 2, 32*key_bits] (kind 'vk') or packed statements uint8[N, 32*key_bits]
+    ('st') -> uint8[N, 57], byte for byte what `repr()` of the drop-in objects gives after `set_content_str(True)`."""
+    return _engine(pp).content_str(kind, packed, key_bits(pp), device=device)
+
+
+def challenge_inputs(pp, vk_packed, msgs, st_packed=None, device: bool = False):
+    """Content-mode challenge messages of packed keys (and packed statements for the adaptor challenge) and raw messages
+    -> (blob, offsets): exactly `lm_one_time_sigs.challenge_messages` (or `adaptor_sigs.challenge_messages`) of the
+    drop-in objects in content mode, ready as `chmsgs` for `sign_batch_packed_sk`, `verify_batch_packed`,
+    `presign_batch_packed_sk`, `preverify_batch_packed` and `adaptor_verify_batch_packed`."""
+    eng = _engine(pp)
+    vk_str = content_strs(pp, vk_packed, 'vk', device=device)
+    st_str = content_strs(pp, st_packed, 'st', device=device) if st_packed is not None else None
+    return eng.challenge_inputs(vk_str, msgs, st_str=st_str, device=device)
+
+
+def aggregation_inputs(pp, agg_off, vk_packed, msgs, device: bool = False):
+    """The BKLM inputs of many groups (items agg_off[g] .. agg_off[g+1] of packed keys uint8[total, 2, 32*key_bits] and
+    bitstring messages) in content mode -> (order, chmsgs_sorted, agmsgs):
+      order          int64[total], within every group the stable sort by content string of `prepare_make_agg_coefs`;
+      chmsgs_sorted  (blob, offsets) challenge messages of the sorted items;
+      agmsgs         list of the n_agg aggregation messages str(list(zip(sorted keys, sorted messages))).
+    Permute the packed signatures / keys by `order` and pass these to `aggregate_batch_packed` /
+    `aggregate_verify_batch_packed`.  Each key is hashed once, on the GPU; the sort runs on the host over the 57-byte
+    strings."""
+    from .lattice_algebra import is_bitstring
+    msgs = list(msgs)
+    if not all(is_bitstring(m) for m in msgs):
+        raise ValueError("Input messages must be bitstrings.")
+    agg_off = np.ascontiguousarray(agg_off, dtype=np.int64)
+    total = len(msgs)
+    if agg_off.ndim != 1 or agg_off.shape[0] < 1 or int(agg_off[0]) != 0 or int(agg_off[-1]) != total or \
+            bool((np.diff(agg_off) < 0).any()):
+        raise ValueError(f'agg_off must start at 0, never decrease and end at the number of messages ({total})')
+    eng = _engine(pp)
+    vk_str = content_strs(pp, vk_packed, 'vk')
+    gid = np.repeat(np.arange(agg_off.shape[0] - 1), np.diff(agg_off))
+    order = np.lexsort((vk_str.view('S57').reshape(-1), gid)).astype(np.int64) if total else np.zeros(0, np.int64)
+    vk_sorted = np.ascontiguousarray(vk_str[order])
+    msgs_sorted = [msgs[i] for i in order]
+    chmsgs = eng.challenge_inputs(vk_sorted, msgs_sorted, device=device)
+    blob, off = eng.aggregation_inputs(agg_off, vk_sorted, msgs_sorted)
+    raw = blob.tobytes()
+    agmsgs = [raw[int(off[g]):int(off[g + 1])].decode() for g in range(off.shape[0] - 1)]
+    return order, chmsgs, agmsgs
 
 
 def key_ch_from_seed(lp, secpar: int, seed: str) -> PolynomialVector:
