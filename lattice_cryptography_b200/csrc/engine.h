@@ -1,4 +1,4 @@
-// engine.h — host-side declarations shared by api.cu, sampler.cu and ring.cu.
+// engine.h — host-side declarations shared by the C ABI files (api*.cu) and the kernel files (sampler.cu, ring.cu, ...).
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
