@@ -268,8 +268,18 @@ int lcb_ctx_create(lcb_ctx** out, int device, int secpar, int q, int d, int l) {
 
     // ---- tables: psi = least element of order exactly 2d (LatticeParameters.rou in lattice_algebra)
     const uint32_t uq = (uint32_t)q;
-    uint32_t psi = 2;
-    while (!(powmod(psi, 2 * d, uq) == 1 && powmod(psi, d, uq) != 1)) ++psi;
+    // The elements of order 2d are the odd powers of any one of them, so the least is found among d candidates instead of
+    // by counting up from 2 (tens of millions of steps for q near 2^31 and small d)
+    uint32_t root = 0;
+    for (uint32_t h = 2; root == 0; ++h) {
+        const uint32_t r = (uint32_t)powmod(h, (uq - 1) / (2 * d), uq);
+        if (powmod(r, d, uq) == uq - 1) root = r;
+    }
+    uint32_t psi = root;
+    for (uint32_t k = 3, r2 = (uint32_t)powmod(root, 2, uq), x = root; k < 2 * (uint32_t)d; k += 2) {
+        x = (uint32_t)((uint64_t)x * r2 % uq);
+        if (x < psi) psi = x;
+    }
     c->rou = (int)psi;
     {
         // Tables of the generic kernels (ring_generic.cu): zetas in bit-reversed order, their inverses, Shoup
@@ -307,6 +317,7 @@ int lcb_ctx_create(lcb_ctx** out, int device, int secpar, int q, int d, int l) {
         c->gen.a_hat = c->d_a_hat;
         c->gen.l = l;
         c->gen.num_sms = prop.multiProcessorCount;
+        c->gen.smem_optin = prop.sharedMemPerBlockOptin;
         c->gen.wide = c->wide;
         c->ring.l = l;
         c->ring.num_sms = prop.multiProcessorCount;

@@ -92,6 +92,7 @@ struct GenCtx {
     GenRing r;
     const uint32_t* a_hat;     // device, uint32[l][d]: NTT(key_ch)
     int l, num_sms;
+    size_t smem_optin;         // the device's opt-in shared-memory limit per block (bytes)
     bool wide;                 // int32 / uint32 element formats (q >= 2^16)
 };
 

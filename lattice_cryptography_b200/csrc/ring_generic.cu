@@ -311,8 +311,9 @@ __global__ void __launch_bounds__(GBS) g_k_verify(GenRing r, const uint32_t* __r
 template <typename CT>
 __global__ void g_k_vec_addsub(GenRing r, const CT* __restrict__ a, const CT* __restrict__ b, int64_t nelem, int sub, CT* __restrict__ out) {
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nelem; i += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t v = (int64_t)a[i] + (sub ? -(int64_t)b[i] : (int64_t)b[i]);
-        out[i] = (CT)g_centre(g_residue(v, r), r);
+        // each operand reduced on its own: a +- b of two int32 values can reach -2^32, below what pos_off lifts
+        const uint32_t x = g_residue((int64_t)a[i], r), y = g_residue((int64_t)b[i], r);
+        out[i] = (CT)g_centre(g_csub(sub ? x + r.q - y : x + y, r.q), r);
     }
 }
 
@@ -372,22 +373,24 @@ __global__ void __launch_bounds__(GBS) g_k_aggv_partial(GenRing r, const NT* __r
 // sparse polynomial given as ag_wt (index, value) pairs.
 // aggregate: per signature NTT(ag_i) and l forward transforms, products accumulated in the NTT domain in a per-block
 // shared array [l][d]; each block inverse-transforms its sum once and adds it to partial, which therefore stays a
-// coefficient-domain sum like the monomial kernel's.
+// coefficient-domain sum like the monomial kernel's.  One launch covers the polynomials p0 .. p0 + np - 1 of the vector
+// (the accumulator of all l may exceed the shared memory of a block; see g_launch_agg_partial_poly).
 template <typename CT, typename PT>
-__global__ void __launch_bounds__(GBS) g_k_agg_partial_poly(GenRing r, int l, const CT* __restrict__ sigs, const CT* __restrict__ ag_pairs,
-                                                            int ag_wt, int64_t count, PT* __restrict__ partial) {
+__global__ void __launch_bounds__(GBS) g_k_agg_partial_poly(GenRing r, int l, int p0, int np, const CT* __restrict__ sigs,
+                                                            const CT* __restrict__ ag_pairs, int ag_wt, int64_t count,
+                                                            PT* __restrict__ partial) {
     extern __shared__ __align__(16) uint32_t smem[];
     const WarpSlot s = warp_slot(smem, r.d);
-    uint32_t* acc = smem + (size_t)GW * 3 * r.d;               // [l][d], shared by the block
-    for (int e = threadIdx.x; e < l * r.d; e += GBS) acc[e] = 0;
+    uint32_t* acc = smem + (size_t)GW * 3 * r.d;               // [np][d], shared by the block
+    for (int e = threadIdx.x; e < np * r.d; e += GBS) acc[e] = 0;
     __syncthreads();
     for (int64_t t = (int64_t)blockIdx.x * GW + s.warp; t < count; t += (int64_t)gridDim.x * GW) {
         g_load_pairs(s.z, ag_pairs + t * ag_wt * 2, ag_wt, r, s.lane);
         g_ntt_fwd(s.z, r, s.lane);
-        for (int i = 0; i < l; ++i) {
+        for (int i = 0; i < np; ++i) {
             int64_t ma = 0;
             int nz = 0;
-            g_load_coef(s.x, sigs + (t * l + i) * r.d, r, s.lane, ma, nz);
+            g_load_coef(s.x, sigs + (t * l + p0 + i) * r.d, r, s.lane, ma, nz);
             g_ntt_fwd(s.x, r, s.lane);
             for (int e = s.lane; e < r.d; e += 32) {
                 const uint32_t v = g_mul(s.x[e], s.z[e], r);
@@ -403,9 +406,9 @@ __global__ void __launch_bounds__(GBS) g_k_agg_partial_poly(GenRing r, int l, co
         }
     }
     __syncthreads();
-    for (int i = s.warp; i < l; i += GW) {
+    for (int i = s.warp; i < np; i += GW) {
         g_ntt_inv(acc + (size_t)i * r.d, r, s.lane);
-        for (int e = s.lane; e < r.d; e += 32) atomicAdd(&partial[(size_t)i * r.d + e], (PT)acc[(size_t)i * r.d + e]);
+        for (int e = s.lane; e < r.d; e += 32) atomicAdd(&partial[(size_t)(p0 + i) * r.d + e], (PT)acc[(size_t)i * r.d + e]);
     }
 }
 
@@ -548,13 +551,34 @@ cudaError_t g_launch_agg_partial(const GenCtx& c, const void* sigs, const void* 
     G_LAUNCH((g_k_agg_partial<int16_t, int32_t>), grid, GBS, g_smem(c.r), st, c.r, c.l, (const int16_t*)sigs, (const int16_t*)ag_pairs, count, (int32_t*)partial);
 }
 
+// The block's [np][d] accumulator sits beside the warps' work arrays.  At d = 1024 a whole vector of l >= 45 polynomials
+// exceeds the opt-in shared-memory limit (227 KB on the B200; l = 64 would need 304 KB), so the vector is summed in slices
+// of as many polynomials as fit, one launch each.
+template <typename CT, typename PT>
+cudaError_t g_agg_partial_poly_slices(const GenCtx& c, const CT* sigs, const CT* ag_pairs, int ag_wt, int64_t count, PT* partial,
+                                      cudaStream_t st) {
+    const size_t row = (size_t)c.r.d * sizeof(uint32_t);
+    const int fit = c.smem_optin > g_smem(c.r) ? (int)((c.smem_optin - g_smem(c.r)) / row) : 0;
+    const int slice = fit < c.l ? fit : c.l;
+    if (slice < 1) return cudaErrorInvalidConfiguration;
+    cudaError_t e = cudaFuncSetAttribute(g_k_agg_partial_poly<CT, PT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)(g_smem(c.r) + slice * row));
+    if (e != cudaSuccess) return e;
+    const unsigned grid = g_grid(count, c.num_sms / 2 + 1);
+    for (int p0 = 0; p0 < c.l; p0 += slice) {
+        const int np = c.l - p0 < slice ? c.l - p0 : slice;
+        g_k_agg_partial_poly<CT, PT><<<grid, GBS, g_smem(c.r) + np * row, st>>>(c.r, c.l, p0, np, sigs, ag_pairs, ag_wt, count, partial);
+        if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
+
 cudaError_t g_launch_agg_partial_poly(const GenCtx& c, const void* sigs, const void* ag_pairs, int ag_wt, int64_t count,
                                       void* partial, cudaStream_t st) {
     if (count <= 0) return cudaSuccess;
-    const size_t smem = g_smem(c.r) + (size_t)c.l * c.r.d * sizeof(uint32_t);
-    const unsigned grid = g_grid(count, c.num_sms / 2 + 1);
-    if (c.wide) G_LAUNCH((g_k_agg_partial_poly<int32_t, unsigned long long>), grid, GBS, smem, st, c.r, c.l, (const int32_t*)sigs, (const int32_t*)ag_pairs, ag_wt, count, (unsigned long long*)partial);
-    G_LAUNCH((g_k_agg_partial_poly<int16_t, int32_t>), grid, GBS, smem, st, c.r, c.l, (const int16_t*)sigs, (const int16_t*)ag_pairs, ag_wt, count, (int32_t*)partial);
+    if (c.wide)
+        return g_agg_partial_poly_slices(c, (const int32_t*)sigs, (const int32_t*)ag_pairs, ag_wt, count, (unsigned long long*)partial, st);
+    return g_agg_partial_poly_slices(c, (const int16_t*)sigs, (const int16_t*)ag_pairs, ag_wt, count, (int32_t*)partial, st);
 }
 
 cudaError_t g_launch_aggv_partial_poly(const GenCtx& c, const void* vk_ntt, const void* ch_pairs, int ch_wt, const void* ag_pairs,
