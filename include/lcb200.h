@@ -392,6 +392,31 @@ int lcb_challenge_inputs_batch(lcb_ctx* ctx, const uint8_t* st_str, const uint8_
 int lcb_aggregation_inputs_batch(lcb_ctx* ctx, const int64_t* agg_off, int64_t n_agg, const uint8_t* vk_str_sorted,
                                  const uint8_t* msg_sorted, const int64_t* msg_off, uint8_t* agmsg, int64_t* agmsg_off);
 
+/* ---- Putting a content-mode BKLM batch into sorted order on the device.  BKLM hashes and sums the items of an aggregate
+ * sorted by str(otvk) (bklm_one_time_agg_sigs.py prepare_make_agg_coefs / prepare_aggregate, a stable sort); in content
+ * mode those strings are the 57-byte rows of lcb_content_str_batch.  These three calls give that order and move packed
+ * keys, signatures, content strings and messages into it, so that unsorted records go to lcb_challenge_inputs_batch,
+ * lcb_aggregation_inputs_batch and the packed BKLM batch calls without a host pass.  Host or device buffers; host offset
+ * and index arrays are checked (LCB_ERR_INVALID), device ones are trusted, but no kernel reads outside its source for any
+ * index value: an index outside [0, n_src) gives an all-zero row or an empty item.  At most 2^30 items; n == 0 / n_agg ==
+ * 0 return LCB_OK.  Pure byte work: valid on every context. */
+/* order int64[total], total = agg_off[n_agg] (agg_off as in lcb_bklm_aggregate_batch): positions agg_off[g] ..
+ * agg_off[g+1] hold the items of group g sorted by their 57-byte rows (uint8[total][57], unsigned byte order), equal rows
+ * in ascending index: the str-sorted order of prepare_make_agg_coefs.  agg_off is read on the host whichever side it is
+ * on (the group sizes choose the kernels: groups of up to 32 items one thread per item, up to 1,024 one block per group,
+ * larger ones a radix sort), so a device agg_off costs one synchronisation. */
+int lcb_content_order_batch(lcb_ctx* ctx, const int64_t* agg_off, int64_t n_agg, const uint8_t* rows, int64_t* order);
+/* dst[k] = src[index[k]], rows of row_bytes bytes: src uint8[n_src][row_bytes], index int64[n], dst uint8[n][row_bytes].
+ * Any row length and alignment (16-byte units where the row length and both buffers allow it). */
+int lcb_gather_rows_batch(lcb_ctx* ctx, const uint8_t* src, int64_t n_src, int64_t row_bytes, const int64_t* index,
+                          int64_t n, uint8_t* dst);
+/* Item k of out = item index[k] of the ragged (blob, off): blob[off[index[k]] .. off[index[k]+1]) (off int64[n_src+1],
+ * off[0] need not be 0), at out[out_off[k] .. out_off[k+1]); out_off int64[n+1], out_off[0] = 0; out_cap = bytes available
+ * in out.  Gathered bytes beyond out_cap give LCB_ERR_INVALID before anything is written to out.  That check reads the
+ * total on the host: the single synchronisation of this call, which is otherwise as asynchronous as the others. */
+int lcb_gather_ragged_batch(lcb_ctx* ctx, const uint8_t* blob, const int64_t* off, int64_t n_src, const int64_t* index,
+                            int64_t n, uint8_t* out, int64_t out_cap, int64_t* out_off);
+
 /* ---- Multi-device context: ONE call shards a HOST-resident batch over several GPUs of the box (SURVEY.md 8(b), 8(e)).
  * devices[] lists CUDA ordinals (an ordinal may repeat: two contexts on one GPU).  Independent units (keygen, sign,
  * verify) are split into contiguous ranges by the reference's distribute_tasks rule (lm_one_time_sigs.py:194-215: the
@@ -435,7 +460,8 @@ int64_t lcb_launch_count(const lcb_ctx* ctx);
  * routes are counted under the kernel they extend: packed signing (from NTT-form or packed signing keys) under sign, packed
  * verification (including witness verification on packed witnesses) under verify, adapt / extract on packed witnesses
  * under vec_addsub.  The content-mode hash inputs: content_str (after unpack and ntt_inv), challenge_inputs, and
- * group_ids + aggregation_inputs.
+ * group_ids + aggregation_inputs; the content-mode order: content_order (after group_ids for groups of up to 32 items),
+ * gather_rows and gather_ragged (the scan and the copy).
  * lcb_profile_read synchronises the stream. */
 int lcb_profile_enable(lcb_ctx* ctx, int on);
 int lcb_profile_reset(lcb_ctx* ctx);

@@ -89,6 +89,9 @@ PROTOTYPES = {
     'lcb_content_str_batch': (c_int, [c_void_p, c_int, _P, c_int, c_int64, _P]),
     'lcb_challenge_inputs_batch': (c_int, [c_void_p, _P, _P, _P, _P, c_int64, _P, _P]),
     'lcb_aggregation_inputs_batch': (c_int, [c_void_p, _P, c_int64, _P, _P, _P, _P, _P]),
+    'lcb_content_order_batch': (c_int, [c_void_p, _P, c_int64, _P, _P]),
+    'lcb_gather_rows_batch': (c_int, [c_void_p, _P, c_int64, c_int64, _P, c_int64, _P]),
+    'lcb_gather_ragged_batch': (c_int, [c_void_p, _P, _P, c_int64, _P, c_int64, _P, c_int64, _P]),
     'lcb_bklm_agg_coefs': (c_int, [c_void_p, POINTER(LcbScheme), _P, c_int64, c_int64, c_int64, _P]),
     'lcb_bklm_aggregate_partial': (c_int, [c_void_p, POINTER(LcbScheme), _P, _P, _P, c_int64, c_int64, c_int64, _P]),
     'lcb_bklm_aggregate_finish': (c_int, [c_void_p, _P, _P]),

@@ -20,7 +20,7 @@ const char* const kKernelNames[K_COUNT] = {"sampler", "shake256", "ntt_fwd", "nt
                                            "aggv_partial", "aggv_finish", "pack", "unpack", "group_ids",
                                            "agg_coefs_seg", "agg_partial_seg", "aggv_partial_seg", "aggv_residues",
                                            "aggv_limits", "agg_finish_pack", "content_str", "challenge_inputs",
-                                           "aggregation_inputs"};
+                                           "aggregation_inputs", "content_order", "gather_rows", "gather_ragged"};
 
 uint64_t powmod(uint64_t b, uint64_t e, uint64_t q) {
     uint64_t r = 1;

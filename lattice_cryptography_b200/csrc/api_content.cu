@@ -1,5 +1,8 @@
 // api_content.cu — content-mode hash inputs of the C ABI (content.cu): the content strings of packed keys and
-// statements, and the challenge and aggregation hash inputs built from them and the raw messages.
+// statements, and the challenge and aggregation hash inputs built from them and the raw messages; the per-group sort of
+// content strings and the row / ragged gathers that put a batch into that order (order.cu).
+#include <cstdlib>
+
 #include "api_internal.h"
 
 using namespace lcb;
@@ -43,6 +46,25 @@ int stage_messages(lcb_ctx* c, Staging& sg, const uint8_t* msg, int64_t first, i
 int put_offset(lcb_ctx* c, int64_t* dst, int64_t v) {
     CK(c, cudaMemcpyAsync(dst, &v, sizeof(int64_t), cudaMemcpyDefault, c->stream));
     CK(c, cudaStreamSynchronize(c->stream));
+    return LCB_OK;
+}
+
+// Test knobs LCB_ORDER_SMALL_MAX / LCB_ORDER_BLOCK_MAX: the largest group of the per-item path (default 32) and of the
+// per-block path (default ORDER_BLOCK_MAX) of lcb_content_order_batch, so that tests reach every path with small groups.
+// They can only lower the defaults; negative values are ignored.
+int order_limit(const char* name, int dflt) {
+    if (const char* env = getenv(name)) {
+        const long v = atol(env);
+        if (v >= 0 && v < dflt) return (int)v;
+    }
+    return dflt;
+}
+
+// host index arrays are checked; device ones are trusted (the kernels treat an index outside [0, n_src) as empty)
+int check_index(lcb_ctx* c, const int64_t* index, int64_t n, int64_t n_src) {
+    if (on_device(index)) return LCB_OK;
+    for (int64_t k = 0; k < n; ++k)
+        if (index[k] < 0 || index[k] >= n_src) return fail(c, LCB_ERR_INVALID, "index outside [0, n_src)");
     return LCB_OK;
 }
 
@@ -175,6 +197,146 @@ int lcb_aggregation_inputs_batch(lcb_ctx* c, const int64_t* agg_off, int64_t n_a
     CK(c, timed(c, K_AGGREGATION_INPUTS, [&] {
         return launch_aggregation_inputs(c->ring, d_agg, d_ag, n_agg, d_gid, total, d_vk, d_msg, shift, d_moff, out_len, d_out,
                                          c->stream);
+    }));
+    CK(c, sg.finish());
+    return LCB_OK;
+}
+
+int lcb_content_order_batch(lcb_ctx* c, const int64_t* agg_off, int64_t n_agg, const uint8_t* rows, int64_t* order) {
+    LCB_RANGE();
+    if (!c || !agg_off || n_agg < 0) return LCB_ERR_INVALID;
+    if (int st = within_limit(c, n_agg, "aggregates in one call")) return st;
+    if (n_agg == 0) return LCB_OK;
+    CK(c, cudaSetDevice(c->device));
+    // the group sizes choose the paths: the offsets are read on the host, and checked there whichever side they come from
+    std::vector<int64_t> h_agg;
+    int64_t total = 0;
+    int st = read_offsets(c, agg_off, n_agg, false, true, &total, h_agg, "agg_off");
+    if (st != LCB_OK) return st;
+    if (h_agg[0] != 0) return fail(c, LCB_ERR_INVALID, "agg_off must start at 0");
+    for (int64_t g = 0; g < n_agg; ++g)
+        if (h_agg[(size_t)g + 1] < h_agg[(size_t)g]) return fail(c, LCB_ERR_INVALID, "agg_off must not decrease");
+    if (total > ((int64_t)1 << 30)) return fail(c, LCB_ERR_INVALID, "at most 2^30 items per batch call");
+    if (total == 0) return LCB_OK;
+    if (!rows || !order) return LCB_ERR_INVALID;
+    const int small_max = order_limit("LCB_ORDER_SMALL_MAX", 32);
+    const int block_max = order_limit("LCB_ORDER_BLOCK_MAX", ORDER_BLOCK_MAX);
+    bool any_small = false;
+    std::vector<int32_t> blk;                                    // groups of the per-block path
+    std::vector<int64_t> la0, lbase{0};                          // the largest groups: first item, concatenated position
+    for (int64_t g = 0; g < n_agg; ++g) {
+        const int64_t cnt = h_agg[(size_t)g + 1] - h_agg[(size_t)g];
+        if (cnt == 0) continue;
+        if (cnt <= small_max) {
+            any_small = true;
+        } else if (cnt <= block_max) {
+            blk.push_back((int32_t)g);
+        } else {
+            la0.push_back(h_agg[(size_t)g]);
+            lbase.push_back(lbase.back() + cnt);
+        }
+    }
+    Staging sg(c);
+    const uint8_t* d_rows = sg.in(rows, (size_t)total * 57);
+    const int64_t* d_agg = sg.in(agg_off, (size_t)n_agg + 1);
+    int64_t* d_order = sg.out(order, (size_t)total);
+    CK(c, sg.status());
+    if (any_small) {
+        int32_t* d_gid = sg.alloc<int32_t>((size_t)total);
+        CK(c, sg.status());
+        CK(c, timed(c, K_GROUP_IDS, [&] { return launch_group_ids(d_agg, n_agg, total, d_gid, c->ring.num_sms, c->stream); }));
+        CK(c, timed(c, K_CONTENT_ORDER, [&] {
+            return launch_content_order_small(d_agg, d_gid, n_agg, total, d_rows, small_max, d_order, c->ring.num_sms, c->stream);
+        }));
+    }
+    if (!blk.empty()) {
+        const int32_t* d_blk = sg.in(blk.data(), blk.size());
+        CK(c, sg.status());
+        CK(c, timed(c, K_CONTENT_ORDER, [&] {
+            return launch_content_order_block(d_agg, d_blk, (int64_t)blk.size(), n_agg, total, d_rows, d_order, c->stream);
+        }));
+    }
+    if (!la0.empty()) {
+        const int L = (int)la0.size();
+        const int64_t m = lbase.back();
+        size_t temp_bytes = 0;
+        CK(c, content_order_large_scratch(m, &temp_bytes));
+        const int64_t* d_a0 = sg.in(la0.data(), la0.size());
+        const int64_t* d_base = sg.in(lbase.data(), lbase.size());
+        uint64_t* d_keys = sg.alloc<uint64_t>((size_t)(2 * m));
+        int32_t* d_perm = sg.alloc<int32_t>((size_t)(2 * m));
+        uint8_t* d_temp = sg.alloc<uint8_t>(temp_bytes);
+        CK(c, sg.status());
+        CK(c, timed(c, K_CONTENT_ORDER, [&] {
+            return launch_content_order_large(d_rows, total, d_a0, d_base, L, m, d_keys, d_perm, d_temp, temp_bytes, d_order,
+                                              c->ring.num_sms, c->stream);
+        }));
+    }
+    CK(c, sg.finish());
+    return LCB_OK;
+}
+
+int lcb_gather_rows_batch(lcb_ctx* c, const uint8_t* src, int64_t n_src, int64_t row_bytes, const int64_t* index, int64_t n,
+                          uint8_t* dst) {
+    LCB_RANGE();
+    if (!c || n < 0 || n_src < 0 || row_bytes < 1) return LCB_ERR_INVALID;
+    if (int st = within_limit(c, n, "items in one gather call")) return st;
+    if (n == 0) return LCB_OK;
+    if (!index || !dst || (n_src > 0 && !src)) return LCB_ERR_INVALID;
+    if (n_src > INT64_MAX / row_bytes || n > INT64_MAX / row_bytes) return fail(c, LCB_ERR_INVALID, "rows too large");
+    CK(c, cudaSetDevice(c->device));
+    if (int st = check_index(c, index, n, n_src)) return st;
+    Staging sg(c);
+    const uint8_t* d_src = sg.in(src, (size_t)(n_src * row_bytes));
+    const int64_t* d_idx = sg.in(index, (size_t)n);
+    uint8_t* d_dst = sg.out(dst, (size_t)(n * row_bytes));
+    CK(c, sg.status());
+    CK(c, timed(c, K_GATHER_ROWS, [&] {
+        return launch_gather_rows(d_src, n_src, row_bytes, d_idx, n, d_dst, c->ring.num_sms, c->stream);
+    }));
+    CK(c, sg.finish());
+    return LCB_OK;
+}
+
+int lcb_gather_ragged_batch(lcb_ctx* c, const uint8_t* blob, const int64_t* off, int64_t n_src, const int64_t* index, int64_t n,
+                            uint8_t* out, int64_t out_cap, int64_t* out_off) {
+    LCB_RANGE();
+    if (!c || !off || !out_off || n < 0 || n_src < 0 || out_cap < 0) return LCB_ERR_INVALID;
+    if (int st = within_limit(c, n, "items in one gather call")) return st;
+    CK(c, cudaSetDevice(c->device));
+    if (n == 0) return put_offset(c, out_off, 0);
+    if (!index) return LCB_ERR_INVALID;
+    if (int st = check_index(c, index, n, n_src)) return st;
+    Staging sg(c);
+    // a device blob with device offsets is used in place; otherwise the blob's extent off[0] .. off[n_src] is read (and
+    // host offsets are checked) to stage it
+    const uint8_t* d_blob = blob;
+    int64_t shift = 0;
+    if (!(on_device(off) && blob && on_device(blob))) {
+        int64_t first = 0, last = 0;
+        int st = offset_ends(c, off, n_src, &first, &last, "off");
+        if (st != LCB_OK) return st;
+        if ((st = stage_messages(c, sg, blob, first, last, &d_blob, &shift)) != LCB_OK) return st;
+    }
+    const int64_t* d_off = sg.in(off, (size_t)n_src + 1);
+    const int64_t* d_idx = sg.in(index, (size_t)n);
+    const int64_t tiles = ragged_scan_tiles(n);
+    int64_t* d_tile = sg.alloc<int64_t>((size_t)tiles + 1);
+    int64_t* d_out_off = sg.out(out_off, (size_t)n + 1);
+    CK(c, sg.status());
+    CK(c, timed(c, K_GATHER_RAGGED, [&] {
+        return launch_ragged_scan(d_off, n_src, d_idx, n, d_tile, d_out_off, c->ring.num_sms, c->stream);
+    }));
+    // the one synchronisation of this call: the gathered total against out_cap, before anything is written to out
+    int64_t need = 0;
+    CK(c, cudaMemcpyAsync(&need, d_tile + tiles, sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
+    CK(c, cudaStreamSynchronize(c->stream));
+    if (need > out_cap) return fail(c, LCB_ERR_INVALID, "the gathered items need more than out_cap bytes");
+    if (need > 0 && !out) return LCB_ERR_INVALID;
+    uint8_t* d_out = sg.out(out, (size_t)need);
+    CK(c, sg.status());
+    CK(c, timed(c, K_GATHER_RAGGED, [&] {
+        return launch_gather_ragged(d_blob, shift, d_off, n_src, d_idx, n, d_out_off, need, d_out, c->ring.num_sms, c->stream);
     }));
     CK(c, sg.finish());
     return LCB_OK;

@@ -75,7 +75,8 @@ inline int fail_cuda(lcb_ctx* c, cudaError_t e, const char* what) {
 enum KernelId { K_SAMPLER = 0, K_SHAKE, K_NTT_FWD, K_NTT_INV, K_POLY_MUL, K_MATVEC, K_SIGN, K_VERIFY, K_ADDSUB,
                 K_AGG_COEFS, K_AGG_PARTIAL, K_AGG_FINISH, K_AGGV_PARTIAL, K_AGGV_FINISH, K_PACK, K_UNPACK, K_GROUP_IDS,
                 K_AGG_COEFS_SEG, K_AGG_PARTIAL_SEG, K_AGGV_PARTIAL_SEG, K_AGGV_RESIDUES, K_AGGV_LIMITS, K_AGG_FINISH_PACK,
-                K_CONTENT_STR, K_CHALLENGE_INPUTS, K_AGGREGATION_INPUTS, K_COUNT };
+                K_CONTENT_STR, K_CHALLENGE_INPUTS, K_AGGREGATION_INPUTS, K_CONTENT_ORDER, K_GATHER_ROWS, K_GATHER_RAGGED,
+                K_COUNT };
 static_assert(K_COUNT <= 32, "grow lcb_ctx::prof_ms / prof_n");
 
 // Launch wrapper: counts the launch and, when profiling is on, brackets it with CUDA events on the

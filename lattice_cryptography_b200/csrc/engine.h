@@ -225,4 +225,31 @@ cudaError_t launch_aggregation_inputs(const RingCtx& c, const int64_t* agg_off, 
                                       const int32_t* gid, int64_t total, const uint8_t* vk_str, const uint8_t* msg,
                                       int64_t shift, const int64_t* msg_off, int64_t out_len, uint8_t* out, cudaStream_t st);
 
+// per-group stable sort of 57-byte rows and the gathers of the content-mode BKLM route (order.cu).  order int64[total]
+// receives, at agg_off[g] .. agg_off[g+1], the items of group g in row order: groups of at most small_max items from
+// launch_content_order_small (gid from launch_group_ids), the listed groups of at most ORDER_BLOCK_MAX items from
+// launch_content_order_block, and the L largest (items a0[k] .., at positions base[k] .. base[k+1] of their
+// concatenation, m = base[L]) from launch_content_order_large: keys uint64[2m], perm int32[2m], temp of
+// content_order_large_scratch(m) bytes.
+constexpr int ORDER_BLOCK_MAX = 1024;
+cudaError_t launch_content_order_small(const int64_t* agg_off, const int32_t* gid, int64_t n_agg, int64_t total,
+                                       const uint8_t* rows, int small_max, int64_t* order, int num_sms, cudaStream_t st);
+cudaError_t launch_content_order_block(const int64_t* agg_off, const int32_t* groups, int64_t n_groups, int64_t n_agg,
+                                       int64_t total, const uint8_t* rows, int64_t* order, cudaStream_t st);
+cudaError_t content_order_large_scratch(int64_t m, size_t* bytes);
+cudaError_t launch_content_order_large(const uint8_t* rows, int64_t total, const int64_t* a0, const int64_t* base, int L, int64_t m,
+                                       uint64_t* keys, int32_t* perm, void* temp, size_t temp_bytes, int64_t* order,
+                                       int num_sms, cudaStream_t st);
+// dst[k] = src[index[k]] (row_bytes each), zero rows for an index outside [0, n_src)
+cudaError_t launch_gather_rows(const uint8_t* src, int64_t n_src, int64_t row_bytes, const int64_t* index, int64_t n, uint8_t* dst,
+                               int num_sms, cudaStream_t st);
+// out_off[n+1] = exclusive scan of the lengths of items index[k] of (off, n_src) (0 outside [0, n_src)); tile_sum
+// int64[ragged_scan_tiles(n) + 1] of scratch, whose last entry receives the total
+int64_t ragged_scan_tiles(int64_t n);
+cudaError_t launch_ragged_scan(const int64_t* off, int64_t n_src, const int64_t* index, int64_t n, int64_t* tile_sum,
+                               int64_t* out_off, int num_sms, cudaStream_t st);
+// item k of out = blob[off[index[k]] - shift .. off[index[k]+1] - shift) at out_off[k]; never past out_cap
+cudaError_t launch_gather_ragged(const uint8_t* blob, int64_t shift, const int64_t* off, int64_t n_src, const int64_t* index,
+                                 int64_t n, const int64_t* out_off, int64_t out_cap, uint8_t* out, int num_sms, cudaStream_t st);
+
 }  // namespace lcb

@@ -509,6 +509,58 @@ class Engine(object):
                                                         _addr(moff), _addr(out), _addr(out_off)))
         return out, out_off
 
+    # ------------------------------------------------------------------ sorted order of content-mode batches
+    def content_order(self, agg_off, rows, device: bool = False):
+        """-> int64[total]: at agg_off[g] .. agg_off[g+1] the items of group g sorted by their 57-byte rows uint8[total, 57]
+        (unsigned byte order, equal rows in ascending index; include/lcb200.h, lcb_content_order_batch)."""
+        total = int(rows.shape[0]) if len(getattr(rows, 'shape', ())) else 0
+        _want(rows, 'rows', np.uint8, (total, 57))
+        n_agg = self._groups(agg_off, total)
+        order = self._out((total,), np.int64, device)
+        self._ck(self._lib.lcb_content_order_batch(self._ctx, _addr(agg_off), n_agg, _addr(rows), _addr(order)))
+        return order
+
+    def gather_rows(self, src, index, device: bool = False):
+        """src[index] for a uint8 array with a leading item dimension: -> uint8[n, *src.shape[1:]]; an index outside
+        [0, len(src)) gives an all-zero row (device indices; host ones are refused)."""
+        shp = tuple(src.shape) if hasattr(src, 'shape') else ()
+        if len(shp) < 1:
+            raise ValueError('src must have a leading item dimension')
+        _want(src, 'src', np.uint8, shp)
+        _want(index, 'index', np.int64, (None,))
+        n = int(index.shape[0])
+        row = int(np.prod(shp[1:])) if len(shp) > 1 else 1
+        out = self._out((n,) + shp[1:], np.uint8, device)
+        if row == 0:
+            return out
+        self._ck(self._lib.lcb_gather_rows_batch(self._ctx, _addr(src), shp[0], row, _addr(index), n, _addr(out)))
+        return out
+
+    def gather_ragged(self, items, index, device: bool = False):
+        """Items index[k] of ragged items (a list of byte strings or a (blob, offsets) pair) -> (blob, offsets int64[n+1]);
+        an index outside [0, n_src) gives an empty item (device indices; host ones are refused)."""
+        blob, off = self._rag(items)
+        n_src = self._count(off)
+        _want(index, 'index', np.int64, (None,))
+        n = int(index.shape[0])
+        if _is_torch(off) or _is_torch(index):          # size the output: the lengths of the valid indices, summed
+            import torch
+            o = off if _is_torch(off) else torch.from_numpy(np.ascontiguousarray(off))
+            i = index if _is_torch(index) else torch.from_numpy(np.ascontiguousarray(index))
+            i = i.to(o.device)
+            lens = o[1:] - o[:-1]
+            ok = (i >= 0) & (i < n_src)
+            need = int((lens[i.clamp(0, max(n_src - 1, 0))] * ok).sum().item()) if n_src else 0
+        else:
+            lens = np.diff(off)
+            ok = (index >= 0) & (index < n_src)
+            need = int(lens[index[ok]].sum())
+        out = self._out((need,), np.uint8, device)
+        out_off = self._out((n + 1,), np.int64, device)
+        self._ck(self._lib.lcb_gather_ragged_batch(self._ctx, _addr(blob), _addr(off), n_src, _addr(index), n, _addr(out),
+                                                   need, _addr(out_off)))
+        return out, out_off
+
     # ------------------------------------------------------------------ BKLM aggregation
     def agg_coefs(self, sch: LcbScheme, agmsg, first: int, count: int, device: bool = False):
         if isinstance(agmsg, (str, bytes, bytearray)):

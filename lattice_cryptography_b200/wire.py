@@ -42,7 +42,11 @@ module is therefore OPT-IN and does not change what the drop-in API computes:
   key received over the wire identifies its key, and the hash inputs are built on the GPU from packed records and raw
   messages: `content_strs` (the 57-byte repr() of packed keys or statements), `challenge_inputs` (the `chmsgs` of every
   packed sign / verify / adaptor call) and `aggregation_inputs` (the per-group sort order, sorted `chmsgs` and
-  aggregation messages of the packed BKLM calls).  The drop-in `challenge_messages` keeps building them on the host.
+  aggregation messages of the packed BKLM calls; the order is sorted on the GPU over the 57-byte strings).
+  `sorted_aggregation_inputs`, `aggregate_batch_content` and `aggregate_verify_batch_content` take UNSORTED packed keys,
+  raw messages and packed signatures (aggregates) and do the sort and the permutation of the records on the GPU too, so
+  that with device=True a batch never leaves the device (reference ag_mode only).  The drop-in `challenge_messages` and
+  `aggregate_batch` keep building them on the host.
 
 Bit layout (include/lcb200.h): value i of a polynomial at bit offset i*bits, least significant bit first.
 """
@@ -51,6 +55,7 @@ from typing import Any, Dict
 
 import numpy as np
 
+from .engine import Engine, _want, ragged
 from .lattice_algebra import PolynomialVector, engine_for
 from .one_time_keys import SchemeParameters, set_content_str  # noqa: F401
 
@@ -293,8 +298,8 @@ def aggregation_inputs(pp, agg_off, vk_packed, msgs, device: bool = False):
       chmsgs_sorted  (blob, offsets) challenge messages of the sorted items;
       agmsgs         list of the n_agg aggregation messages str(list(zip(sorted keys, sorted messages))).
     Permute the packed signatures / keys by `order` and pass these to `aggregate_batch_packed` /
-    `aggregate_verify_batch_packed`.  Each key is hashed once, on the GPU; the sort runs on the host over the 57-byte
-    strings."""
+    `aggregate_verify_batch_packed`, or use `aggregate_batch_content` / `aggregate_verify_batch_content`, which do all of
+    it on the device.  Each key is hashed once and the order is sorted on the GPU (`Engine.content_order`)."""
     from .lattice_algebra import is_bitstring
     msgs = list(msgs)
     if not all(is_bitstring(m) for m in msgs):
@@ -306,8 +311,7 @@ def aggregation_inputs(pp, agg_off, vk_packed, msgs, device: bool = False):
         raise ValueError(f'agg_off must start at 0, never decrease and end at the number of messages ({total})')
     eng = _engine(pp)
     vk_str = content_strs(pp, vk_packed, 'vk')
-    gid = np.repeat(np.arange(agg_off.shape[0] - 1), np.diff(agg_off))
-    order = np.lexsort((vk_str.view('S57').reshape(-1), gid)).astype(np.int64) if total else np.zeros(0, np.int64)
+    order = eng.content_order(agg_off, vk_str)
     vk_sorted = np.ascontiguousarray(vk_str[order])
     msgs_sorted = [msgs[i] for i in order]
     chmsgs = eng.challenge_inputs(vk_sorted, msgs_sorted, device=device)
@@ -315,6 +319,80 @@ def aggregation_inputs(pp, agg_off, vk_packed, msgs, device: bool = False):
     raw = blob.tobytes()
     agmsgs = [raw[int(off[g]):int(off[g + 1])].decode() for g in range(off.shape[0] - 1)]
     return order, chmsgs, agmsgs
+
+
+def _content_messages(msgs):
+    """Messages of the content-mode BKLM routes as (blob, offsets): a list of bitstrings is checked with the error of
+    `prepare_make_agg_coefs` and packed; a (blob, offsets) pair, host or device, is taken as it is."""
+    from .lattice_algebra import is_bitstring
+    if isinstance(msgs, tuple) and len(msgs) == 2 and not isinstance(msgs[0], str):
+        return Engine._rag(msgs)
+    msgs = list(msgs)
+    if not all(is_bitstring(m) for m in msgs):
+        raise ValueError("Input messages must be bitstrings.")
+    return ragged(msgs)
+
+
+def _sorted_content(pp, agg_off, vk_packed, msgs, device):
+    """-> (order, content strings and messages of the sorted items, aggregation messages (blob, offsets)), on the device
+    when `device`."""
+    if pp.get('ag_mode', 'reference') != 'reference':
+        raise ValueError("the content-mode BKLM routes support ag_mode 'reference' only: in tree mode the commitment of "
+                         "each aggregation message is built on the host")
+    eng = _engine(pp)
+    rag = _content_messages(msgs)
+    vk_str = content_strs(pp, vk_packed, 'vk', device=device)
+    if eng._count(rag[1]) != int(vk_str.shape[0]):
+        raise ValueError(f'{eng._count(rag[1])} messages for {int(vk_str.shape[0])} keys')
+    order = eng.content_order(agg_off, vk_str, device=device)
+    str_sorted = eng.gather_rows(vk_str, order, device=device)
+    msgs_sorted = eng.gather_ragged(rag, order, device=device)
+    agmsgs = eng.aggregation_inputs(agg_off, str_sorted, msgs_sorted, device=device)
+    return order, str_sorted, msgs_sorted, agmsgs
+
+
+def sorted_aggregation_inputs(pp, agg_off, vk_packed, msgs, device: bool = False):
+    """The BKLM inputs of many groups in content mode, sorted on the GPU from unsorted records: packed keys uint8[total, 2,
+    32*key_bits] and messages (a list of bitstrings or a (blob, offsets) pair, items agg_off[g] .. agg_off[g+1] in group
+    g) -> (order, vk_packed_sorted, chmsgs_sorted, agmsgs):
+      order             int64[total], `aggregation_inputs`'s order;
+      vk_packed_sorted  vk_packed[order];
+      chmsgs_sorted     (blob, offsets) challenge messages of the sorted items;
+      agmsgs            (blob, offsets) aggregation messages of the groups.
+    The two message sets go to `Engine.aggregate_packed_batch` / `aggregate_verify_packed_batch` as they are.  With
+    device=True every output is a device tensor and no record leaves the device.  Reference ag_mode only."""
+    eng = _engine(pp)
+    order, str_sorted, msgs_sorted, agmsgs = _sorted_content(pp, agg_off, vk_packed, msgs, device)
+    vk_sorted = eng.gather_rows(vk_packed, order, device=device)
+    chmsgs = eng.challenge_inputs(str_sorted, msgs_sorted, device=device)
+    return order, vk_sorted, chmsgs, agmsgs
+
+
+def aggregate_batch_content(pp, agg_off, vk_packed, msgs, sig_packed, device: bool = False):
+    """Aggregates of many groups in content mode from UNSORTED packed keys, messages and packed signatures
+    uint8[total, l, 32*sig_bits] -> (ag_packed uint8[n_agg, l, 32*sig_bits(pp, 'avf_bd')], in_range uint8[n_agg, l]):
+    exactly `aggregate_batch_packed(pp, agg_off, sig_packed[order], agmsgs)` with `aggregation_inputs`'s order and
+    messages, sorted and gathered on the GPU.  Reference ag_mode only."""
+    from .bklm_one_time_agg_sigs import _ctx
+    eng, sch = _ctx(pp)
+    total = int(vk_packed.shape[0]) if len(getattr(vk_packed, 'shape', ())) else 0
+    _want(sig_packed, 'sig_packed', np.uint8, (total, eng.l, eng.d * sig_bits(pp) // 8))
+    order, _, _, agmsgs = _sorted_content(pp, agg_off, vk_packed, msgs, device)
+    sig_sorted = eng.gather_rows(sig_packed, order, device=device)
+    return eng.aggregate_packed_batch(sch, agg_off, sig_sorted, sig_bits(pp), pp['vf_bd'], agmsgs, sig_bits(pp, 'avf_bd'),
+                                      pp['avf_bd'], device=device, want_range=True)
+
+
+def aggregate_verify_batch_content(pp, agg_off, vk_packed, msgs, ag_packed, device: bool = False):
+    """uint8[n_agg] verdicts of many aggregates in content mode from UNSORTED packed keys and messages and packed
+    aggregates uint8[n_agg, l, 32*sig_bits(pp, 'avf_bd')]: exactly `aggregate_verify_batch_packed` on the inputs of
+    `sorted_aggregation_inputs`, all of them made on the GPU.  Reference ag_mode only."""
+    from .bklm_one_time_agg_sigs import _ctx
+    eng, sch = _ctx(pp)
+    _, vk_sorted, chmsgs, agmsgs = sorted_aggregation_inputs(pp, agg_off, vk_packed, msgs, device=device)
+    return eng.aggregate_verify_packed_batch(sch, agg_off, vk_sorted, key_bits(pp), chmsgs, agmsgs, ag_packed,
+                                             sig_bits(pp, 'avf_bd'), pp['avf_bd'], pp['ag_cap'], pp['avf_bd'], pp['avf_wt'],
+                                             device=device)
 
 
 def key_ch_from_seed(lp, secpar: int, seed: str) -> PolynomialVector:
