@@ -419,8 +419,11 @@ int lcb_ctx_create(lcb_ctx** out, int device, int secpar, int q, int d, int l) {
     if ((e = cudaMalloc(&c->d_tab, sizeof(NttTables))) != cudaSuccess) return bail(e, "cudaMalloc tables");
     if ((e = cudaMemcpy(c->d_tab, &t, sizeof(NttTables), cudaMemcpyHostToDevice)) != cudaSuccess) return bail(e, "cudaMemcpy tables");
     if ((e = cudaMalloc(&c->d_a_hat, (size_t)l * D * sizeof(uint32_t))) != cudaSuccess) return bail(e, "cudaMalloc key_ch");
+    if ((e = cudaMalloc(&c->d_tc_b, verify_tc_matrix_bytes(l))) != cudaSuccess) return bail(e, "cudaMalloc key_ch matrices");
     c->ring.tab = c->d_tab;
     c->ring.a_hat = c->d_a_hat;
+    c->ring.tc_b = c->d_tc_b;
+    c->ring.zeta = t.pw[128];
     c->gen.a_hat = c->d_a_hat;
     c->ring.l = l;
     c->ring.num_sms = prop.multiProcessorCount;
@@ -443,6 +446,7 @@ int lcb_ctx_destroy(lcb_ctx* c) {
     if (c->d_tab) cudaFree(c->d_tab);
     if (c->d_gen_tab) cudaFree(c->d_gen_tab);
     if (c->d_a_hat) cudaFree(c->d_a_hat);
+    if (c->d_tc_b) cudaFree(c->d_tc_b);
     if (c->idx_scratch) cudaFree(c->idx_scratch);
     if (c->d_mod_tab) cudaFree(c->d_mod_tab);
     if (c->il_scratch) cudaFree(c->il_scratch);
@@ -544,6 +548,7 @@ int lcb_set_key_ch(lcb_ctx* c, const int16_t* key_ch_coef) {
         CK(c, cudaStreamSynchronize(c->stream));
         std::vector<uint32_t> h32(h16.begin(), h16.end());
         CK(c, cudaMemcpyAsync(c->d_a_hat, h32.data(), h32.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+        if (!c->generic) CK(c, launch_verify_tc_matrix(c->ring, c->stream));
         CK(c, cudaStreamSynchronize(c->stream));
     }
     c->has_key_ch = true;

@@ -28,6 +28,7 @@ struct lcb_ctx {
     uint32_t* d_gen_tab = nullptr;       // generic twiddle tables: w, ws, iw, iws [d] each, pw [2d]
     lcb::NttTables* d_tab = nullptr;
     uint32_t* d_a_hat = nullptr;
+    uint8_t* d_tc_b = nullptr;           // k_verify_tc's key_ch matrices (ring path)
     bool has_key_ch = false;
     std::string last_error;
     int64_t launches = 0;

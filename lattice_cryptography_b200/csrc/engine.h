@@ -129,6 +129,8 @@ struct RingCtx {
     StageConstF iscf;          // warp-uniform twiddles of the FP32-assisted inverse (ntt_inv_256_fp), index half + j
     const NttTables* tab;      // device
     const uint32_t* a_hat;     // device, uint32[l][256]: NTT(key_ch), slot order
+    uint8_t* tc_b;             // device, verify_tc_matrix_bytes(l): the key_ch matrices of k_verify_tc (ring.cu)
+    uint32_t zeta;             // psi^128
     int l;
     int num_sms;
 };
@@ -143,6 +145,9 @@ cudaError_t launch_matvec(const RingCtx& c, const int16_t* vec_coef, int64_t nve
                           uint16_t* y_ntt, int16_t* y_coef, cudaStream_t st);
 cudaError_t launch_sign(const RingCtx& c, const uint16_t* sk_ntt, const int16_t* ch_pairs, int ch_wt, int64_t n,
                         int16_t* sig, cudaStream_t st);
+// the u8 key_ch matrices B_0 / B_1 of the tensor-core verify, rebuilt from a_hat whenever key_ch changes
+inline size_t verify_tc_matrix_bytes(int l) { return (size_t)l * 4 * 2 * 2 * 256 * 64; }
+cudaError_t launch_verify_tc_matrix(const RingCtx& c, cudaStream_t st);
 // verdict = bounds(vec) && key_ch*vec == [vk_left*c] + [vk_right | rhs0] + [rhs1]
 cudaError_t launch_verify(const RingCtx& c, const int16_t* vec_coef, const uint16_t* vk_ntt,
                           const int16_t* ch_pairs, int ch_wt, const uint16_t* rhs_only, const uint16_t* extra_rhs,

@@ -4,6 +4,7 @@
 //   key_ch * sk / key_ch * wit          lm_one_time_sigs.py:95-96, adaptor_sigs.py:100     -> k_matvec
 //   sk_left ** c + sk_right             lm_one_time_sigs.py:168, adaptor_sigs.py:193       -> k_sign
 //   bounds; key_ch*sig == vk0*c+vk1[+st] lm_one_time_sigs.py:173-191, adaptor_sigs.py:198-266 -> k_verify
+//                                       (k_verify_tc: int16 rows of large batches, on the tensor cores)
 //   sum(sig ** ag)                      bklm_one_time_agg_sigs.py:96                       -> k_agg_partial
 //   sum((vk0*c+vk1)*ag); key_ch*ag_sig == . bklm_one_time_agg_sigs.py:99-116               -> k_aggv_*
 //   the same for many aggregates per call                                                  -> k_agg*_partial_seg
@@ -17,6 +18,7 @@
 #include <cstdlib>
 
 #include "engine.h"
+#include "tc_device.cuh"
 
 namespace lcb {
 
@@ -717,6 +719,291 @@ __global__ void __launch_bounds__(VBS, VERIFY_BLOCKS) k_verify(ModQ m, StageCons
         for (int k = 0; k < EPT; ++k) eq &= divisible_by_q(acc[k] + (uint64_t)(CORR(k) - rhs[k]), m);   // corr = kq18 - bias term
         const unsigned votes = __ballot_sync(0xFFFFFFFFu, eq && !bad);
         if (live && h.lane == 0) verdict[item] = (votes & h.mask) == h.mask ? 1 : 0;
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// k_verify_tc: the same verdict for int16 rows, with key_ch * v as two exact u8 tensor-core GEMMs (DESIGN.md section 3.3).
+// With zeta = psi^128, slot p < 128 of NTT(a) evaluates u0 = a_lo + zeta a_hi and slot p >= 128 evaluates
+// u1 = a_lo - zeta a_hi (a_lo / a_hi: coefficients 0..127 / 128..255) at 128 points, so for block b
+//   sum_k key_hat_k[p] s_hat_k[p] = sum_(k, m) M_b[p][(k, m)] u^b_k[m],   M_b[p][(k, m)] = key_hat_k[p] x_p^m mod q.
+// The CUDA cores form u in [0, q) and split it into two u8 limbs (A = [u & 255 | u >> 8], K = 2 * 128 * l); the context
+// holds B_b = [M_b ; 256 M_b mod q] split into byte columns (N = 2 * 128: slot x (lo, hi)), built by k_verify_tc_matrix.
+// D_b = A B_b^T then gives x[p] = D_lo[p] + 256 D_hi[p] = sum_k key_hat_k[p] s_hat_k[p] (mod q), exactly: every entry is
+// below 255 * 255 * 256 * l < 2^31 for l <= 128 (contexts take l <= 64).
+//
+// One CTA per SM, 128 verifies (= the 128 tensor-memory lanes) per tile, both blocks accumulated at once in all 512
+// columns.  K runs in chunks of 64 bytes per block - (poly k, quarter mq: m in 32 mq .. 32 mq + 31) x (limb 0, limb 1) -
+// through TC_STAGES shared-memory stages.  Roles:
+//   warps 0-3   right-hand sides of the tile (half-warp NTT of the challenge, as k_verify), then the epilogue: thread r
+//               reads tensor-memory lane r (its verify) and tests x - rhs for divisibility by q at every slot;
+//   warp 4      bulk copies of the B chunks (L2-resident, read by every CTA);
+//   warp 5      tensor-memory allocation and the MMA-issuing thread;
+//   warps 6-13  converters: thread (r, h) reads 16 coefficient pairs of verify r per stage from HBM, keeps the running
+//               bound / weight checks, and writes the u limbs of both blocks into the A stage.
+constexpr int TC_ROWS = 128;
+constexpr int TC_STAGES = 3;
+constexpr int TC_A_BLOCK = TC_ROWS * 64;                  // bytes of one block's A chunk (128 rows x 64 K-bytes)
+constexpr int TC_B_BLOCK = 256 * 64;                      // bytes of one block's B chunk (256 columns x 64 K-bytes)
+constexpr int TC_B_CHUNK = 2 * TC_B_BLOCK;                // bytes of B per K chunk (both blocks), one bulk copy
+constexpr int TC_STAGE_BYTES = 2 * TC_A_BLOCK + TC_B_CHUNK;
+constexpr int TC_RHS_PITCH = D / 2 + 1;                   // words per rhs row: the epilogue's 32 rows fall in 32 banks
+constexpr int TC_EPI_WARPS = 4, TC_CONV_WARPS = 8;
+constexpr int TC_MIN_TILES_PER_SM = 1;                   // batches below one tile per SM stay on k_verify
+constexpr int TC_THREADS = 32 * (TC_EPI_WARPS + 2 + TC_CONV_WARPS);
+constexpr size_t tc_smem_bytes() {
+    return (size_t)TC_STAGES * TC_STAGE_BYTES + (size_t)TC_ROWS * TC_RHS_PITCH * 4 + (size_t)TW_BYTES +
+           (size_t)TC_EPI_WARPS * XWARP * 4 + 2 * TC_ROWS + 8 * (2 * TC_STAGES + 2) + 16;
+}
+
+// B_b in the stage layout: K chunk g = 4 k + mq holds [block 0 | block 1], each 4 K-columns of 16 bytes x 256 rows n =
+// 128 hl + p; byte kb = 32 L + (m - 32 mq) of row n is byte hl of 256^L key_hat_k[P] x_P^m mod q, P = 128 b + p.
+__global__ void k_verify_tc_matrix(ModQ m, const NttTables* __restrict__ tab, const uint32_t* __restrict__ a_hat, int l,
+                                   uint8_t* __restrict__ out) {
+    const int64_t total = (int64_t)l * 4 * TC_B_CHUNK;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const int g = (int)(i / TC_B_CHUNK), rem = (int)(i % TC_B_CHUNK);
+        const int b = rem / TC_B_BLOCK, off = rem % TC_B_BLOCK;
+        const int kb = (off >> 12) * 16 + (off & 15), n = (off >> 4) & 255;
+        const int L = kb >> 5, mm = 32 * (g & 3) + (kb & 31), k = g >> 2;
+        const int P = 128 * b + (n & 127);
+        uint64_t v = (uint64_t)a_hat[k * D + P] * tab->pw[((uint32_t)tab->oddexp[P] * (uint32_t)mm) & 511] % m.q;
+        if (L) v = v * 256 % m.q;
+        out[i] = (uint8_t)((n >> 7) ? v >> 8 : v & 255);
+    }
+}
+
+template <bool CHECK_WT>
+__global__ void __launch_bounds__(TC_THREADS, 1) k_verify_tc(ModQ m, StageConstF scf, const NttTables* __restrict__ tab,
+                                                   const uint8_t* __restrict__ bmat, int l,
+                                                   const int16_t* __restrict__ vec_coef, const uint16_t* __restrict__ vk_ntt,
+                                                   const int16_t* __restrict__ ch_pairs, int ch_wt,
+                                                   const uint16_t* __restrict__ rhs_only,
+                                                   const uint16_t* __restrict__ extra_rhs, int64_t n, int bd, int wt,
+                                                   uint32_t zeta, uint32_t kz0, uint32_t kz1, uint8_t* __restrict__ verdict) {
+    extern __shared__ __align__(128) unsigned char tc_smem[];
+    unsigned char* stages = tc_smem;
+    uint32_t* rhs_buf = reinterpret_cast<uint32_t*>(stages + TC_STAGES * TC_STAGE_BYTES);
+    uint4* twtab = reinterpret_cast<uint4*>(rhs_buf + TC_ROWS * TC_RHS_PITCH);
+    uint32_t* xbuf = reinterpret_cast<uint32_t*>(reinterpret_cast<unsigned char*>(twtab) + TW_BYTES);
+    uint8_t* badbuf = reinterpret_cast<uint8_t*>(xbuf + TC_EPI_WARPS * XWARP);     // [2][128], by tile parity
+    uint64_t* full = reinterpret_cast<uint64_t*>(badbuf + 2 * TC_ROWS);
+    uint64_t* empty = full + TC_STAGES;
+    uint64_t* acc_full = empty + TC_STAGES;
+    uint64_t* acc_empty = acc_full + 1;
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 1);
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < TC_STAGES; ++s) {
+            mbar_init(&full[s], TC_CONV_WARPS + 1);     // converter warps + the B copy (arrive.expect_tx)
+            mbar_init(&empty[s], 1);                    // MMA commit
+        }
+        mbar_init(acc_full, 2);                         // MMA commit + the MMA thread (orders the bound flags)
+        mbar_init(acc_empty, TC_EPI_WARPS * 32);
+        mbar_init_fence();
+    }
+    if (warp == TC_EPI_WARPS + 1) {
+        tmem_alloc(tmem_slot, 512);
+        tc_fence_before();
+    }
+    fill_tw_shared(twtab, tab);                         // ends in __syncthreads
+    tc_fence_after();
+    const uint32_t tmem = *tmem_slot;
+
+    const uint32_t n32 = (uint32_t)n;
+    const uint32_t tiles = (n32 + TC_ROWS - 1) / TC_ROWS;
+    const int chunks = 4 * l;                           // K chunks per tile
+
+    if (warp < TC_EPI_WARPS) {
+        // ---- right-hand sides, then the epilogue
+        const HalfWarp h = half_warp(xbuf);
+        const LaneTwFShared twf{twtab + h.lane * TW_ROW};
+        const int r = threadIdx.x;
+        int t = 0;
+        for (uint32_t tile = blockIdx.x; tile < tiles; tile += gridDim.x, ++t) {
+            asm volatile("bar.sync 1, %0;" ::"n"(TC_EPI_WARPS * 32) : "memory");    // rhs_buf of the last tile is read
+            for (int row = h.slot; row < TC_ROWS; row += 2 * TC_EPI_WARPS) {
+                const uint32_t raw = tile * TC_ROWS + row;
+                const int64_t item = raw < n32 ? raw : n32 - 1;
+                uint32_t rhs[EPT];
+                if (vk_ntt) {
+                    uint32_t c[EPT], vl[EPT];
+                    int cx[EPT];
+                    load_pairs_raw(cx, ch_pairs + item * ch_wt * 2, ch_wt, h.xb, h.lane);
+                    ntt_fwd_256_fp(cx, c, m, scf, twf, h.xb, h.lane);
+                    load_u16x16(vl, vk_ntt + item * 2 * D + 16 * h.lane);
+                    load_u16x16(rhs, vk_ntt + item * 2 * D + D + 16 * h.lane);
+#pragma unroll
+                    for (int k = 0; k < EPT; ++k) rhs[k] += mulmod_full(barrett_full(c[k] - FP_BIAS, m), vl[k], m);
+                } else {
+                    load_u16x16(rhs, rhs_only + item * D + 16 * h.lane);
+                }
+                if (extra_rhs) {
+                    uint32_t ex[EPT];
+                    load_u16x16(ex, extra_rhs + item * D + 16 * h.lane);
+#pragma unroll
+                    for (int k = 0; k < EPT; ++k) rhs[k] += ex[k];
+                }
+                uint32_t* dst = rhs_buf + row * TC_RHS_PITCH + 8 * h.lane;
+#pragma unroll
+                for (int k = 0; k < EPT; k += 2) dst[k / 2] = barrett_full(rhs[k], m) | (barrett_full(rhs[k + 1], m) << 16);
+            }
+            asm volatile("bar.sync 1, %0;" ::"n"(TC_EPI_WARPS * 32) : "memory");    // every rhs row of this tile written
+            mbar_wait(acc_full, t & 1);
+            tc_fence_after();
+            bool eq = true;
+            const uint32_t* my = rhs_buf + r * TC_RHS_PITCH;
+            const uint32_t lane_base = tmem + ((uint32_t)(32 * warp) << 16);
+#pragma unroll 1
+            for (int col = 0; col < 2 * 128; col += 16) {           // col = 128 b + p0
+                const int b = col >> 7, p0 = col & 127;
+                uint32_t lo[16], hi[16];
+                tmem_ld16(lane_base + 256 * b + p0, lo);
+                tmem_ld16(lane_base + 256 * b + 128 + p0, hi);
+                tmem_ld_wait();
+#pragma unroll
+                for (int j = 0; j < 16; j += 2) {
+                    const uint32_t w = my[(col + j) >> 1];
+                    eq &= divisible_by_q((uint64_t)lo[j] + ((uint64_t)hi[j] << 8) + (m.q - (w & 0xFFFFu)), m);
+                    eq &= divisible_by_q((uint64_t)lo[j + 1] + ((uint64_t)hi[j + 1] << 8) + (m.q - (w >> 16)), m);
+                }
+            }
+            tc_fence_before();
+            mbar_arrive(acc_empty);
+            const uint32_t raw = tile * TC_ROWS + r;
+            if (raw < n32) verdict[raw] = (eq && !badbuf[(t & 1) * TC_ROWS + r]) ? 1 : 0;
+        }
+    } else if (warp == TC_EPI_WARPS) {
+        // ---- B chunks
+        if (lane == 0) {
+            uint32_t s = 0;
+            for (uint32_t tile = blockIdx.x; tile < tiles; tile += gridDim.x)
+                for (int g = 0; g < chunks; ++g, ++s) {
+                    const uint32_t slot = s % TC_STAGES, round = s / TC_STAGES;
+                    if (round > 0) mbar_wait(&empty[slot], (round - 1) & 1);
+                    mbar_arrive_tx(&full[slot], TC_B_CHUNK);
+                    bulk_g2s(stages + slot * TC_STAGE_BYTES + 2 * TC_A_BLOCK, bmat + (size_t)g * TC_B_CHUNK, TC_B_CHUNK,
+                             &full[slot]);
+                }
+        }
+    } else if (warp == TC_EPI_WARPS + 1) {
+        // ---- MMA issue
+        if (lane == 0) {
+            constexpr uint32_t idesc = umma_idesc_u8(TC_ROWS, 256);
+            uint32_t s = 0;
+            int t = 0;
+            for (uint32_t tile = blockIdx.x; tile < tiles; tile += gridDim.x, ++t) {
+                if (t > 0) {
+                    mbar_wait(acc_empty, (t - 1) & 1);
+                    tc_fence_after();
+                }
+                for (int g = 0; g < chunks; ++g, ++s) {
+                    const uint32_t slot = s % TC_STAGES, round = s / TC_STAGES;
+                    mbar_wait(&full[slot], round & 1);
+                    tc_fence_after();
+                    const uint32_t a0 = smem_addr(stages + slot * TC_STAGE_BYTES), b0 = a0 + 2 * TC_A_BLOCK;
+#pragma unroll
+                    for (int b = 0; b < 2; ++b)
+#pragma unroll
+                        for (int L = 0; L < 2; ++L)
+                            umma_u8(tmem + 256 * b, umma_desc(a0 + b * TC_A_BLOCK + L * 2 * (16 * TC_ROWS), 16 * TC_ROWS, 128),
+                                    umma_desc(b0 + b * TC_B_BLOCK + L * 2 * (16 * 256), 16 * 256, 128), idesc, g > 0 || L > 0);
+                    umma_commit(&empty[slot]);
+                }
+                umma_commit(acc_full);
+                mbar_arrive(acc_full);
+            }
+        }
+    } else {
+        // ---- converters: thread (r, hh) owns coefficient pairs m in 32 mq + 16 hh + [0, 16) of verify r in every chunk
+        const int ct = threadIdx.x - 32 * (TC_EPI_WARPS + 2);
+        const int r = ct >> 1, hh = ct & 1;
+        const uint32_t zn = m.q - zeta;
+        const int lim_hi = 32768 + bd, lim_lo = 32768 - bd;     // on the biased values a + 32768
+        uint32_t s = 0;
+        int t = 0;
+        // one chunk ahead in registers: 16 low and 16 high coefficients
+        uint4 nx[4];
+        auto load = [&](uint32_t tile, int g) {
+            const uint32_t raw = tile * TC_ROWS + r;
+            const int64_t item = raw < n32 ? raw : n32 - 1;
+            const int16_t* row = vec_coef + (item * l + (g >> 2)) * D + 32 * (g & 3) + 16 * hh;
+            LCB_CHECK(row >= vec_coef && row + D / 2 + 16 <= vec_coef + n * l * D);
+            const uint4* p = reinterpret_cast<const uint4*>(row);
+            const uint4* q = reinterpret_cast<const uint4*>(row + D / 2);
+            nx[0] = __ldg(p);
+            nx[1] = __ldg(p + 1);
+            nx[2] = __ldg(q);
+            nx[3] = __ldg(q + 1);
+        };
+        if (blockIdx.x < tiles) load(blockIdx.x, 0);
+        for (uint32_t tile = blockIdx.x; tile < tiles; tile += gridDim.x, ++t) {
+            uint32_t mx = 0, mn = 0xFFFFFFFFu;                  // running max / min of the biased halves
+            bool heavy = false;
+            int nz = 0;
+            for (int g = 0; g < chunks; ++g, ++s) {
+                const uint4 cur[4] = {nx[0], nx[1], nx[2], nx[3]};
+                if (g + 1 < chunks) load(tile, g + 1);
+                else if (tile + gridDim.x < tiles) load(tile + gridDim.x, 0);
+                const uint32_t wl[8] = {cur[0].x, cur[0].y, cur[0].z, cur[0].w, cur[1].x, cur[1].y, cur[1].z, cur[1].w};
+                const uint32_t wh[8] = {cur[2].x, cur[2].y, cur[2].z, cur[2].w, cur[3].x, cur[3].y, cur[3].z, cur[3].w};
+                uint32_t o[2][2][4];                            // [block][limb][word]
+#pragma unroll
+                for (int w4 = 0; w4 < 4; ++w4) {
+                    uint32_t u[2][4];
+#pragma unroll
+                    for (int w = 0; w < 2; ++w) {
+                        const uint32_t bl = wl[2 * w4 + w] ^ 0x80008000u, bh = wh[2 * w4 + w] ^ 0x80008000u;
+                        mx = __vmaxu2(mx, __vmaxu2(bl, bh));
+                        mn = __vminu2(mn, __vminu2(bl, bh));
+                        if (CHECK_WT)
+                            nz += ((bl & 0xFFFFu) != 0x8000u) + ((bl >> 16) != 0x8000u) + ((bh & 0xFFFFu) != 0x8000u) +
+                                  ((bh >> 16) != 0x8000u);
+#pragma unroll
+                        for (int e = 0; e < 2; ++e) {
+                            const uint32_t lo = e ? bl >> 16 : bl & 0xFFFFu, hi = e ? bh >> 16 : bh & 0xFFFFu;
+                            u[0][2 * w + e] = barrett_full(hi * zeta + (lo + kz0), m);
+                            u[1][2 * w + e] = barrett_full(hi * zn + (lo + kz1), m);
+                        }
+                    }
+#pragma unroll
+                    for (int b = 0; b < 2; ++b) {
+                        const uint32_t p01 = __byte_perm(u[b][0], u[b][1], 0x5410), p23 = __byte_perm(u[b][2], u[b][3], 0x5410);
+                        o[b][0][w4] = __byte_perm(p01, p23, 0x6420);
+                        o[b][1][w4] = __byte_perm(p01, p23, 0x7531);
+                    }
+                }
+                if (CHECK_WT && (g & 3) == 3) {                 // the row (poly g / 4) is complete over the pair
+                    heavy |= nz + __shfl_xor_sync(0xFFFFFFFFu, nz, 1) > wt;
+                    nz = 0;
+                }
+                const uint32_t slot = s % TC_STAGES, round = s / TC_STAGES;
+                if (g + 1 == chunks) {                          // bound flags of the tile, before its last chunk is signalled
+                    const uint32_t MX = max(mx & 0xFFFFu, mx >> 16), MN = min(mn & 0xFFFFu, mn >> 16);
+                    bool bad = heavy || (int)MX > lim_hi || (int)MN < lim_lo;
+                    bad |= __shfl_xor_sync(0xFFFFFFFFu, (int)bad, 1) != 0;
+                    if (hh == 0) badbuf[(t & 1) * TC_ROWS + r] = bad ? 1 : 0;
+                }
+                if (round > 0) mbar_wait(&empty[slot], (round - 1) & 1);
+                unsigned char* a = stages + slot * TC_STAGE_BYTES + 16 * r;
+#pragma unroll
+                for (int b = 0; b < 2; ++b)
+#pragma unroll
+                    for (int L = 0; L < 2; ++L)
+                        *reinterpret_cast<uint4*>(a + b * TC_A_BLOCK + (2 * L + hh) * (16 * TC_ROWS)) =
+                            make_uint4(o[b][L][0], o[b][L][1], o[b][L][2], o[b][L][3]);
+                fence_async_smem();
+                __syncwarp();
+                if (lane == 0) mbar_arrive(&full[slot]);
+            }
+        }
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == TC_EPI_WARPS + 1) {
+        tc_fence_after();
+        tmem_free(tmem, 512);
     }
 }
 
@@ -1448,7 +1735,32 @@ cudaError_t launch_verify_t(const RingCtx& c, const void* vec, const void* vk, c
 cudaError_t launch_verify(const RingCtx& c, const int16_t* vec_coef, const uint16_t* vk_ntt, const int16_t* ch_pairs,
                           int ch_wt, const uint16_t* rhs_only, const uint16_t* extra_rhs, int64_t n, int bd, int wt,
                           uint8_t* verdict, cudaStream_t st) {
-    return launch_verify_t<0, 0>(c, vec_coef, vk_ntt, ch_pairs, ch_wt, rhs_only, extra_rhs, n, bd, wt, 0, verdict, st);
+    if (n <= 0) return cudaSuccess;
+    if (n > ((int64_t)1 << 30)) return cudaErrorInvalidValue;      // 32-bit item indices inside the kernel
+    // k_verify_tc walks the 4 l chunks of a 128-verify tile one after the other: about 70 us for any batch up to one
+    // tile per SM.  k_verify takes 27 us for one verify and grows by a trip of 32 verifies per SM: 66 us at 14,208
+    // verifies, 82 us at 18,944, where k_verify_tc takes 72 us (B200, secpar 128).  Smaller batches, the single drop-in
+    // verify among them, keep k_verify.
+    if (n < (int64_t)TC_MIN_TILES_PER_SM * TC_ROWS * c.num_sms)
+        return launch_verify_t<0, 0>(c, vec_coef, vk_ntt, ch_pairs, ch_wt, rhs_only, extra_rhs, n, bd, wt, 0, verdict, st);
+    const size_t smem = tc_smem_bytes();
+    auto kern = wt < D ? k_verify_tc<true> : k_verify_tc<false>;
+    cudaError_t e = allow_smem(kern, smem);
+    if (e != cudaSuccess) return e;
+    const uint32_t q = c.m.q, zn = q - c.zeta;
+    const uint64_t b15 = 32768 % q;                                // -> kz = -(32768 + 32768 z) mod q
+    const uint32_t kz0 = (uint32_t)((2 * (uint64_t)q - b15 - b15 * c.zeta % q) % q);
+    const uint32_t kz1 = (uint32_t)((2 * (uint64_t)q - b15 - b15 * zn % q) % q);
+    const int64_t tiles = (n + TC_ROWS - 1) / TC_ROWS;
+    const unsigned grid = (unsigned)(tiles < c.num_sms ? tiles : c.num_sms);
+    kern<<<grid, TC_THREADS, smem, st>>>(c.m, c.scf, c.tab, c.tc_b, c.l, vec_coef, vk_ntt, ch_pairs, ch_wt, rhs_only,
+                                          extra_rhs, n, bd, wt, c.zeta, kz0, kz1, verdict);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_verify_tc_matrix(const RingCtx& c, cudaStream_t st) {
+    k_verify_tc_matrix<<<c.num_sms * 4, 256, 0, st>>>(c.m, c.tab, c.a_hat, c.l, c.tc_b);
+    return cudaGetLastError();
 }
 
 // The two shipped packings are expanded inside the kernel; anything else is reported as unsupported and the
