@@ -727,8 +727,9 @@ __global__ void __launch_bounds__(VBS, VERIFY_BLOCKS) k_verify(ModQ m, StageCons
 // With zeta = psi^128, slot p < 128 of NTT(a) evaluates u0 = a_lo + zeta a_hi and slot p >= 128 evaluates
 // u1 = a_lo - zeta a_hi (a_lo / a_hi: coefficients 0..127 / 128..255) at 128 points, so for block b
 //   sum_k key_hat_k[p] s_hat_k[p] = sum_(k, m) M_b[p][(k, m)] u^b_k[m],   M_b[p][(k, m)] = key_hat_k[p] x_p^m mod q.
-// The CUDA cores form u in [0, q) and split it into two u8 limbs (A = [u & 255 | u >> 8], K = 2 * 128 * l); the context
-// holds B_b = [M_b ; 256 M_b mod q] split into byte columns (N = 2 * 128: slot x (lo, hi)), built by k_verify_tc_matrix.
+// The CUDA cores form u < 2^16 congruent to it mod q (tc_limbs_reduce) and split it into two u8 limbs (A = [u & 255 |
+// u >> 8], K = 2 * 128 * l); the context holds B_b = [M_b ; 256 M_b mod q] split into byte columns (N = 2 * 128:
+// slot x (lo, hi)), built by k_verify_tc_matrix.
 // D_b = A B_b^T then gives x[p] = D_lo[p] + 256 D_hi[p] = sum_k key_hat_k[p] s_hat_k[p] (mod q), exactly: every entry is
 // below 255 * 255 * 256 * l < 2^31 for l <= 128 (contexts take l <= 64).
 //
@@ -773,7 +774,15 @@ __global__ void k_verify_tc_matrix(ModQ m, const NttTables* __restrict__ tab, co
     }
 }
 
-template <bool CHECK_WT>
+// u only has to be congruent to a_lo +- zeta a_hi mod q and below 2^16 (two u8 limbs): D_lo + 256 D_hi is then congruent
+// to the key_ch product, which is all the epilogue tests, and every D entry keeps its bound.  barrett_lazy lands in
+// [0, 2q), so for q <= 32768 (LAZY) it is reduced enough; larger q take one conditional subtraction.
+template <bool LAZY>
+__device__ __forceinline__ uint32_t tc_limbs_reduce(uint32_t x, const ModQ& m) {
+    return LAZY ? barrett_lazy(x, m) : csub(barrett_lazy(x, m), m.q);
+}
+
+template <bool CHECK_WT, bool LAZY>
 __global__ void __launch_bounds__(TC_THREADS, 1) k_verify_tc(ModQ m, StageConstF scf, const NttTables* __restrict__ tab,
                                                    const uint8_t* __restrict__ bmat, int l,
                                                    const int16_t* __restrict__ vec_coef, const uint16_t* __restrict__ vk_ntt,
@@ -963,8 +972,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_verify_tc(ModQ m, StageConstF
 #pragma unroll
                         for (int e = 0; e < 2; ++e) {
                             const uint32_t lo = e ? bl >> 16 : bl & 0xFFFFu, hi = e ? bh >> 16 : bh & 0xFFFFu;
-                            u[0][2 * w + e] = barrett_full(hi * zeta + (lo + kz0), m);
-                            u[1][2 * w + e] = barrett_full(hi * zn + (lo + kz1), m);
+                            u[0][2 * w + e] = tc_limbs_reduce<LAZY>(hi * zeta + (lo + kz0), m);
+                            u[1][2 * w + e] = tc_limbs_reduce<LAZY>(hi * zn + (lo + kz1), m);
                         }
                     }
 #pragma unroll
@@ -1744,7 +1753,9 @@ cudaError_t launch_verify(const RingCtx& c, const int16_t* vec_coef, const uint1
     if (n < (int64_t)TC_MIN_TILES_PER_SM * TC_ROWS * c.num_sms)
         return launch_verify_t<0, 0>(c, vec_coef, vk_ntt, ch_pairs, ch_wt, rhs_only, extra_rhs, n, bd, wt, 0, verdict, st);
     const size_t smem = tc_smem_bytes();
-    auto kern = wt < D ? k_verify_tc<true> : k_verify_tc<false>;
+    const bool lazy = c.m.q <= 32768;
+    auto kern = wt < D ? (lazy ? k_verify_tc<true, true> : k_verify_tc<true, false>)
+                       : (lazy ? k_verify_tc<false, true> : k_verify_tc<false, false>);
     cudaError_t e = allow_smem(kern, smem);
     if (e != cudaSuccess) return e;
     const uint32_t q = c.m.q, zn = q - c.zeta;
