@@ -150,7 +150,9 @@ __device__ __forceinline__ uint32_t shoup_mul(uint32_t a, uint32_t w, uint32_t w
 }
 
 __device__ __forceinline__ uint32_t barrett_lazy(uint32_t x, const ModQ& m) {
-    // x any 32-bit value -> x mod q in [0, 2q)
+    // x any 32-bit value -> x mod q in [0, 2q): with 2^32 - 1 = barrett q + s (s < q) and x = Q q + R, the estimate is
+    // short by two only if R barrett + 2^32 < Q (1 + s), and Q (1 + s) < 2^32 (1 + s) / q <= 2^32
+    // (tests/test_verify_tc_limbs_cpu.py checks the inputs of k_verify_tc's limb reduction exhaustively)
     uint32_t hi = __umulhi(x, m.barrett);
     return x + hi * m.negq;
 }
@@ -158,7 +160,7 @@ __device__ __forceinline__ uint32_t barrett_lazy(uint32_t x, const ModQ& m) {
 __device__ __forceinline__ uint32_t csub(uint32_t x, uint32_t q) { return x >= q ? x - q : x; }
 
 __device__ __forceinline__ uint32_t barrett_full(uint32_t x, const ModQ& m) {
-    // floor((2^32-1)/q) underestimates the quotient by at most 2
+    // floor((2^32-1)/q) underestimates the quotient by at most 1 (barrett_lazy); the second subtraction never fires
     return csub(csub(barrett_lazy(x, m), m.q), m.q);
 }
 
